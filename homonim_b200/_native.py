@@ -18,7 +18,7 @@ from homonim_b200.errors import NativeLibraryError
 HB_U8, HB_U16, HB_F32, HB_I16 = 0, 1, 2, 3
 HB_MODEL_GAIN, HB_MODEL_GAIN_BLK_OFFSET, HB_MODEL_GAIN_OFFSET = 0, 1, 2
 HB_UP_CUBIC_SPLINE, HB_UP_NEAREST = 0, 1
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 _PKG_DIR = pathlib.Path(__file__).resolve().parent
 LIB_PATH = _PKG_DIR / 'libhomonim_b200.so'
@@ -75,6 +75,7 @@ SIGNATURES = {
     'hb_fuse_refspace_host': (c_int, [c_void_p, c_int, c_long, c_long, c_int, c_double, c_void_p, c_long, c_long,
                                       c_int, c_double, c_double, c_double, c_double, c_double, c_int, c_int, c_int,
                                       c_int, c_int, c_double, c_int, c_int, c_double, c_void_p, c_void_p, c_void_p]),
+    'hb_build_overviews': (c_int, [c_void_p, c_int, c_long, c_long, c_long, c_int, c_double, c_int, c_void_p, c_void_p]),
 }
 
 

@@ -126,9 +126,10 @@ class FilePair:
                                  'minisblack'))
 
     def write_corrected(self, corr_ra: RasterArray, corr_filename, proc_crs, out_profile: Dict, overwrite: bool = False,
-                        **kwargs) -> pathlib.Path:
+                        overviews=None, **kwargs) -> pathlib.Path:
         """ The corrected image, in the source's grid and CRS, with the reference bands' wavelength metadata and
-        descriptions copied to the bands they corrected (fuse.py:217-238). """
+        descriptions copied to the bands they corrected (fuse.py:217-238), and its internal ``overviews`` (levels of
+        factor 2, 4, ...; a band stream carries its own). """
         keep = ('center_wavelength', 'name', 'description', 'offset', 'scale')
         band_tags = [{k: v for k, v in tags.items() if k in keep} for tags in self.ref_band_tags]
         nodata = out_profile.get('nodata')
@@ -136,13 +137,13 @@ class FilePair:
             logger.debug('nodata=None: no internal mask is written; invalid pixels hold 0')
         return write_geotiff(corr_filename, corr_ra.array, corr_ra.transform, crs=corr_ra.crs, nodata=nodata,
                              descriptions=self.ref_descriptions, tags=self._meta(proc_crs, **kwargs),
-                             band_tags=band_tags, geokeys=self.src_geokeys, overwrite=overwrite,
+                             band_tags=band_tags, geokeys=self.src_geokeys, overwrite=overwrite, overviews=overviews,
                              **self._creation(out_profile))
 
     def write_params(self, param_ra: RasterArray, param_filename, proc_crs, out_profile: Dict, overwrite: bool = False,
-                     **kwargs) -> pathlib.Path:
+                     overviews=None, **kwargs) -> pathlib.Path:
         """ The parameter image (float32, NaN nodata; gains, then offsets, then R2, one of each per band,
-        fuse.py:186-201, 240-262). """
+        fuse.py:186-201, 240-262), with its internal ``overviews`` (interleaved as the image). """
         n_bands = len(self.src_bands)
         descriptions: List[Optional[str]] = [None] * param_ra.count
         band_tags: List[Dict] = [dict() for _ in range(param_ra.count)]
@@ -157,7 +158,7 @@ class FilePair:
         creation['photometric'] = 'minisblack'
         return write_geotiff(param_filename, param_ra.array, param_ra.transform, crs=param_ra.crs,
                              nodata=float('nan'), descriptions=descriptions, tags=self._meta(proc_crs, **kwargs),
-                             band_tags=band_tags, geokeys=geokeys, overwrite=overwrite, **creation)
+                             band_tags=band_tags, geokeys=geokeys, overwrite=overwrite, overviews=overviews, **creation)
 
 
 def create_out_postfix(proc_crs, model, kernel_shape: Tuple[int, int], driver: str = 'GTiff') -> str:

@@ -1,5 +1,5 @@
 """
-RasterFuse for B200: the caller of the kernel-model path, for in-memory rasters.
+RasterFuse for B200: the caller of the kernel-model path, for in-memory rasters and GeoTIFF files.
 
 Mirrors the user-facing surface of ``homonim.RasterFuse`` that reaches the hot path
 (/root/reference/homonim/fuse.py:44-149 config factories, :295-408 ``_process_block`` / ``process``;
@@ -7,11 +7,13 @@ raster_pair.py:194-225 ``proc_crs`` resolution, :280-296 processing windows): sa
 signatures, config dictionaries, model selection (``SrcSpaceModel if proc_crs == src else RefSpaceModel``,
 fuse.py:376-377) and per-band fit -> apply flow (fuse.py:304-307).
 
-Out of scope (SURVEY.md section 2 / 8): GeoTIFF file I/O, overviews, metadata, band matching by wavelength.  Sources
-and references are therefore :class:`~homonim_b200.raster_array.RasterArray` objects (host numpy or CUDA tensors)
-and ``process`` RETURNS the corrected (and optionally parameter) rasters instead of writing files.  The reference's
-block grid exists to bound host memory (raster_pair.py:227-269); on a 180 GB B200 a whole band is one block, which is
-also the reference's own result for ``max_block_mem`` large enough (SURVEY.md 7.4-5).
+Sources and references are :class:`~homonim_b200.raster_array.RasterArray` objects (host numpy or CUDA tensors), for
+which ``process`` RETURNS the corrected (and optionally parameter) rasters, or GeoTIFF file names, for which it also
+writes the corrected / parameter files as the reference does (band matching by wavelength, metadata, and -- with
+``build_ovw=True``, the default -- internal average overviews built on the GPU from the planes as written; see
+:mod:`homonim_b200.overviews`).  The reference's block grid exists to bound host memory (raster_pair.py:227-269); on a
+180 GB B200 a whole band is one block, which is also the reference's own result for ``max_block_mem`` large enough
+(SURVEY.md 7.4-5).
 """
 import pathlib
 import threading
@@ -27,6 +29,7 @@ from homonim_b200.files import FilePair, is_path
 from homonim_b200.geometry import Affine
 from homonim_b200.kernel_model import (KernelModel, RefSpaceModel, SrcSpaceModel, current_stream, on_stream,
                                        overlap_for_kernel)
+from homonim_b200.overviews import OVERVIEW_DTYPES, build_overviews, level_shape, overview_factors
 from homonim_b200.raster_array import RasterArray, is_tensor
 
 try:
@@ -289,9 +292,6 @@ class RasterFuse:
             with torch.cuda.device(self._src.array.device):        # the native calls launch on the current device
                 return self.process(corr_filename, model, kernel_shape, param_filename, build_ovw, overwrite,
                                     model_config, out_profile, block_config, corr_out)
-        if self._files is not None and is_path(corr_filename) and build_ovw:
-            warnings.warn('`build_ovw` is ignored: overviews are not built by this path (use gdaladdo on the output).',
-                          category=ConfigWarning)
         model_config = RasterFuse.create_model_config(**(model_config or {}))
         block_config = RasterFuse.create_block_config(**(block_config or {}))
         out_profile = RasterFuse.create_out_profile(**(out_profile or {}))
@@ -328,6 +328,22 @@ class RasterFuse:
         # a float32 plane and a separate conversion
         fused_out = out_dtype in ('float32', 'uint8', 'uint16', 'int16')
 
+        # Internal overviews of the written files (reference fuse.py:151-165): every band's levels are built on the GPU from
+        # its device plane as written (output dtype and nodata), on the band's stream, and copied to host buffers with the
+        # band -- so that the writer encodes them band by band like the image's own tiles.
+        write_files = self._files is not None and is_path(corr_filename)
+        corr_levels = 0
+        if write_files and build_ovw:
+            if out_dtype in OVERVIEW_DTYPES:
+                corr_levels = len(overview_factors((hs, ws)))
+            else:
+                warnings.warn(f'`build_ovw`: overviews are built for {", ".join(OVERVIEW_DTYPES)} outputs; the {out_dtype} '
+                              f'output is written without them (use gdaladdo on it).', category=ConfigWarning)
+        param_ovw = write_files and build_ovw and is_path(param_filename)
+        corr_ovw = [torch.empty(level_shape((n_bands, hs, ws), 2 ** k), dtype=getattr(torch, out_dtype))
+                    for k in range(1, corr_levels + 1)]
+        param_ovw_planes = [None] * n_bands
+
         # File -> file (SURVEY.md 8f-4): the corrected image is encoded and written band by band WHILE the GPU works on the
         # later bands -- the writer waits on a band stream that a small completion thread feeds as every band's device ->
         # host copy lands.  (The reference's writer likewise runs inside its thread pool, fuse.py:254-293, 396-408.)
@@ -340,7 +356,7 @@ class RasterFuse:
             import queue
             import types
             from homonim_b200.geotiff import BandStream
-            band_stream = BandStream(corr_all.numpy())
+            band_stream = BandStream(corr_all.numpy(), overviews=[o.numpy() for o in corr_ovw])
             done_queue = queue.Queue()
 
             def _complete():
@@ -377,10 +393,18 @@ class RasterFuse:
                                                        out_nodata=out_nodata)
                 if to_host:
                     corr_all[band_i].copy_(plane, non_blocking=True)
+                if corr_levels:
+                    for host, level in zip(corr_ovw, build_overviews(plane, out_nodata, corr_levels)):
+                        host[band_i].copy_(level, non_blocking=True)
             else:
                 corr_ra, param_ra = self._process_band(band_i, kernel_model, out=None, stage=True, want_params=want)
                 plane = _convert_dtype(corr_ra, out_dtype, out_nodata)
                 corr_all[band_i].copy_(plane, non_blocking=True)
+            if param_ra is not None and param_ovw:
+                levels = build_overviews(param_ra.array.contiguous(), float('nan'),
+                                         len(overview_factors(param_ra.array.shape)))
+                param_ovw_planes[band_i] = [torch.empty(lv.shape, dtype=lv.dtype).copy_(lv, non_blocking=True)
+                                            for lv in levels]
             if param_ra is not None:
                 param_planes[band_i] = param_ra if (src_on_device or param_filename is None) else param_ra.to_host()
             if streaming:
@@ -401,7 +425,7 @@ class RasterFuse:
                 done_queue.put(None)
                 writer.join(timeout=60)
             raise
-        if to_host:
+        if to_host or corr_ovw or param_ovw:
             current_stream().synchronize()  # the host copies have landed
         if streaming:
             done_queue.put(None)
@@ -419,14 +443,19 @@ class RasterFuse:
             planes = [param_planes[b].array[p] for p in range(n_params) for b in range(n_bands)]
             stack = torch.stack if is_tensor(planes[0]) else np.stack
             params = RasterArray(stack(planes), param_planes[0].crs, param_planes[0].transform, nodata=float('nan'))
+        param_levels = None
+        if param_ovw and param_ovw_planes[0]:                 # (None without parameters, [] under 512 px)
+            n_params = param_ovw_planes[0][0].shape[0]       # interleaved band-major, as the parameter image itself
+            param_levels = [torch.stack([param_ovw_planes[b][k][p] for p in range(n_params) for b in range(n_bands)])
+                            for k in range(len(param_ovw_planes[0]))]
         if self._files is not None and is_path(corr_filename):
             # a pair opened from files: write the outputs with the reference's metadata (fuse.py:264-293)
             if not streaming:
                 self._files.write_corrected(corr.to_host(), corr_filename, self.proc_crs, out_profile,
-                                            overwrite=overwrite, **meta)
+                                            overwrite=overwrite, overviews=corr_ovw, **meta)
             if params is not None and is_path(param_filename):
                 self._files.write_params(params.to_host(), param_filename, self.proc_crs, out_profile,
-                                         overwrite=overwrite, **meta)
+                                         overwrite=overwrite, overviews=param_levels, **meta)
         return corr, params
 
     @staticmethod

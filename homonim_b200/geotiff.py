@@ -96,16 +96,24 @@ class GeoTiffReader:
     Read access to one GeoTIFF file.  Attribute names follow the rasterio dataset attributes the reference uses
     (``width``, ``height``, ``count``, ``dtypes``, ``nodata``, ``transform``, ``crs``, ``descriptions``, ``colorinterp``,
     ``tags()``, ``profile``), so that the pair / band-matching logic reads like the reference's.
+
+    ``overview_level`` (rasterio's open option of that name): open internal overview ``overview_level`` instead of the
+    full-resolution image, counted from 0 for the first (factor 2) overview.  Its pixels, size, blocks and transform are
+    the overview's; CRS, nodata, metadata and descriptions are the image's.
     """
 
-    def __init__(self, filename):
+    def __init__(self, filename, overview_level: Optional[int] = None):
         self.name = str(filename)
         self._fh = open(filename, 'rb')
         self._closed = False
-        self._parse_header()
+        try:
+            self._parse_header(overview_level)
+        except BaseException:
+            self.close()
+            raise
 
     # ---- header -----------------------------------------------------------------------------------------------------
-    def _parse_header(self):
+    def _parse_header(self, overview_level: Optional[int] = None):
         fh = self._fh
         head = fh.read(16)
         if head[:2] not in (b'II', b'MM'):
@@ -127,17 +135,27 @@ class GeoTiffReader:
         # them through dataset_mask (raster_array.py:170-197).  They are not decoded here, and reading such a file as
         # "fully valid" would let invalid pixels into the fit, so refuse it.
         self.has_internal_mask = False
+        self._overview_ifds: List[Dict[int, tuple]] = []          # reduced-resolution IFDs (NewSubfileType bit 0)
         next_off, seen = self._next_ifd, 0
         while next_off and seen < 64:
             sub = self._read_ifd(next_off)
             next_off, seen = self._next_ifd, seen + 1
             if 254 in sub and (int(sub[254][0]) & 4):
                 self.has_internal_mask = True
+            elif 254 in sub and (int(sub[254][0]) & 1):
+                self._overview_ifds.append(sub)
         if os.path.exists(self.name + '.msk'):
             self.has_internal_mask = True
         if self.has_internal_mask:
             raise NotImplementedError(f'{self.name}: internal / side-car mask bands are not supported (give the image '
                                       f'a nodata value instead)')
+        self._full_shape = (int(tags[257][0]), int(tags[256][0]))
+        self.overview_level = overview_level
+        if overview_level is not None:
+            if not 0 <= int(overview_level) < len(self._overview_ifds):
+                raise ValueError(f'{self.name}: overview level {overview_level} does not exist (the file has '
+                                 f'{len(self._overview_ifds)})')
+            tags = self._overview_ifds[int(overview_level)]     # the pixels' layout; the metadata stay IFD 0's
         self.width, self.height = int(tags[256][0]), int(tags[257][0])
         self.count = int(tags.get(277, (1,))[0])
         bits = tags.get(258, (1,))
@@ -168,6 +186,9 @@ class GeoTiffReader:
             raise ValueError(f'{self.name}: inconsistent block table')
         if 254 in tags and (tags[254][0] & 4):
             raise NotImplementedError(f'{self.name}: the first IFD is a mask')
+        tags = self._raw_tags
+        if overview_level is not None and int(tags.get(277, (1,))[0]) != self.count:
+            raise ValueError(f'{self.name}: overview {overview_level} has a different band count')
         # geo-referencing
         if 33550 in tags and 33922 in tags:
             scale, tie = tags[33550], tags[33922]
@@ -184,6 +205,9 @@ class GeoTiffReader:
             self.crs.raw_geokeys = self._geo
             if _raster_type(self._geo[0]) == 2:                 # RasterPixelIsPoint: the tie point is a pixel centre
                 self.transform = self.transform * Affine.translation(-0.5, -0.5)
+        if overview_level is not None:                          # rasterio: the full transform scaled to the overview
+            full_h, full_w = self._full_shape
+            self.transform = self.transform * Affine.scale(full_w / self.width, full_h / self.height)
         nodata = tags.get(42113)
         self.nodata = None
         if nodata is not None:
@@ -299,6 +323,13 @@ class GeoTiffReader:
                     blockxsize=self.block_shape[1], blockysize=self.block_shape[0], tiled=self.tiled,
                     compress='deflate' if self.compression in _DEFLATE else None,
                     interleave='band' if self.planar == 2 else 'pixel')
+
+    def overviews(self, bidx: int) -> List[int]:
+        """ Decimation factors of the internal overviews of 1-based band ``bidx`` (rasterio ``DatasetReader.overviews``:
+        ``round(width / overview width)``; every band has the same overviews here). """
+        if not 1 <= bidx <= self.count:
+            raise IndexError(f'{self.name}: band index out of range')
+        return [int(round(self._full_shape[1] / int(sub[256][0]))) for sub in self._overview_ifds]
 
     def tags(self, bidx: Optional[int] = None) -> Dict[str, str]:
         """ Dataset metadata items, or those of 1-based band ``bidx`` (rasterio ``DatasetReader.tags``). """
@@ -423,12 +454,15 @@ class BandStream:
     A ``[bands, H, W]`` array whose bands become available one after the other -- what :func:`write_geotiff` takes to
     encode band ``b`` while the GPU is still producing band ``b + 1`` (SURVEY.md 8f-4).  ``array`` is the (host) buffer
     the producer fills; the producer calls ``set_ready(b)`` once band ``b`` is complete in it, or ``fail(exc)``.
+    ``overviews``: optional ``[bands, h_k, w_k]`` host buffers of the image's overview levels (factors 2, 4, ...), whose
+    band ``b`` the producer also fills before ``set_ready(b)``.
     """
 
-    def __init__(self, array: np.ndarray):
+    def __init__(self, array: np.ndarray, overviews: Optional[Sequence[np.ndarray]] = None):
         if array.ndim != 3:
             raise ValueError('BandStream needs a [bands, H, W] buffer')
         self.array = array
+        self.overviews = list(overviews) if overviews else None
         self.shape, self.dtype, self.ndim = array.shape, array.dtype, 3
         self._ready = [threading.Event() for _ in range(array.shape[0])]
         self._error: Optional[BaseException] = None
@@ -454,16 +488,41 @@ class BandStream:
         return self.array
 
 
+def _check_overviews(overviews, shape, dtype) -> list:
+    """ The overview arrays as [bands, h_k, w_k] numpy arrays; level k (0-based) must have decimation factor 2^(k+1). """
+    levels = []
+    count, height, width = shape
+    for k, level in enumerate(overviews or ()):
+        if torch is not None and isinstance(level, torch.Tensor):
+            level = level.detach().cpu().numpy()
+        level = np.asarray(level)
+        if level.ndim == 2:
+            level = level[None]
+        f = 2 ** (k + 1)
+        expect = (count, -(-height // f), -(-width // f))
+        if level.shape != expect:
+            raise ValueError(f'overview {k} (factor {f}) must be {list(expect)}, not {list(level.shape)}')
+        if np.dtype(level.dtype).newbyteorder('=') != dtype:
+            raise ValueError(f'overview {k} has dtype {level.dtype}, the image {dtype}')
+        levels.append(level)
+    return levels
+
+
 def write_geotiff(filename, array, transform, crs=None, nodata=None, descriptions=None, tags=None, band_tags=None,
                   geokeys=None, compress: Optional[str] = 'deflate', blocksize: int = 512, interleave: str = 'band',
                   photometric: Optional[str] = None, bigtiff: Optional[bool] = None, overwrite: bool = False,
-                  level: int = 6):
+                  level: int = 6, overviews: Optional[Sequence] = None):
     """
     Write ``array`` ([bands, H, W] or [H, W]; numpy or CPU torch tensor) as a tiled GeoTIFF -- what
     ``RasterArray.to_rio_dataset`` + the creation profile do in the reference (raster_array.py:424-524,
     fuse.py:167-215).  ``geokeys`` = (GeoKeyDirectory, GeoDoubleParams, GeoAsciiParams) as read by
     :class:`GeoTiffReader` is written through unchanged (the path never re-projects, so the output CRS is the source's).
     BigTIFF is chosen automatically when the pixels would not fit a classic TIFF.
+
+    ``overviews``: internal overviews (what ``gdaladdo`` / the reference's ``_build_overviews`` add), a list of
+    ``[bands, ceil(H / f), ceil(W / f)]`` arrays of the image's dtype for f = 2, 4, 8, ...  They are written as
+    reduced-resolution IFDs (NewSubfileType = 1) chained after the image's, with its layout, compression and tile size.
+    A :class:`BandStream` ``array`` carries its overviews itself.
     """
     path = pathlib.Path(filename)
     if path.exists() and not overwrite:
@@ -475,6 +534,10 @@ def write_geotiff(filename, array, transform, crs=None, nodata=None, description
         array = np.asarray(array)
         if array.ndim == 2:
             array = array[None]
+    elif overviews:
+        raise ValueError('a BandStream carries its own overviews')
+    else:
+        overviews = stream.overviews
     if array.ndim != 3:
         raise ValueError('`array` must be [bands, H, W] or [H, W]')
     dtype = np.dtype(array.dtype).newbyteorder('=')
@@ -485,35 +548,47 @@ def write_geotiff(filename, array, transform, crs=None, nodata=None, description
         raise NotImplementedError(f'compression {compress!r} is not supported (deflate or None)')
     deflate = compress == 'deflate'
     count, height, width = array.shape
+    levels = _check_overviews(overviews, array.shape, dtype)
     blocksize = max(16, (int(blocksize) + 15) // 16 * 16)                 # TIFF: tile sides are multiples of 16
     th, tw = blocksize, blocksize
-    down, across = -(-height // th), -(-width // tw)
+    # per IFD (the image, then each overview): (height, width, tiles down, tiles across)
+    grids = [(h, w, -(-h // th), -(-w // tw)) for h, w in [(height, width)] + [lv.shape[1:] for lv in levels]]
     planar = 2 if (interleave == 'band' and count > 1) else 1
-    raw_bytes = count * height * width * dtype.itemsize
+    raw_bytes = sum(count * h * w for h, w, _, _ in grids) * dtype.itemsize
     big = bool(bigtiff) if bigtiff is not None else raw_bytes > 3_900_000_000
     t = Affine.coerce(transform)
     if not t.is_rectilinear:
         raise NotImplementedError('rotated geo-transforms cannot be written')
 
+    def source(ifd, plane):
+        """ [bands or 1, h, w] pixels of IFD `ifd`: one band (planar 2) or all of them; a band stream blocks until the
+        producer has finished them. """
+        if stream is not None:
+            stream.wait_band(plane) if planar == 2 else stream.wait_all()
+        full = array if ifd == 0 else levels[ifd - 1]
+        if stream is not None and ifd == 0:
+            full = stream.array
+        return full[plane:plane + 1] if planar == 2 else full
+
     def encode(job):
-        plane, by, bx = job
+        ifd, plane, by, bx = job
+        h, w = grids[ifd][:2]
         tile = np.zeros((th, tw, 1 if planar == 2 else count), dtype=dtype)
-        ys, xs = slice(by * th, min((by + 1) * th, height)), slice(bx * tw, min((bx + 1) * tw, width))
-        if planar == 2:
-            # (a band stream: blocks until the producer has finished this band)
-            part = (stream.wait_band(plane) if stream is not None else array[plane])[ys, xs]
-            tile[:part.shape[0], :part.shape[1], 0] = part
-        else:
-            part = (stream.wait_all() if stream is not None else array)[:, ys, xs]
-            tile[:part.shape[1], :part.shape[2], :] = np.moveaxis(part, 0, 2)
+        ys, xs = slice(by * th, min((by + 1) * th, h)), slice(bx * tw, min((bx + 1) * tw, w))
+        part = source(ifd, plane)[:, ys, xs]
+        tile[:part.shape[1], :part.shape[2], :] = np.moveaxis(part, 0, 2)
         data = tile.tobytes()
         return zlib.compress(data, level) if deflate else data
 
-    jobs = [(p, by, bx) for p in range(count if planar == 2 else 1) for by in range(down) for bx in range(across)]
+    # file order: band by band (planar 2), each band's image tiles followed by its overview tiles -- so that a band
+    # stream's overview tiles are encoded as soon as their band is ready
+    jobs = [(i, p, by, bx) for p in range(count if planar == 2 else 1) for i, (_, _, down, across) in enumerate(grids)
+            for by in range(down) for bx in range(across)]
     bo = '<'
     off_fmt, off_type = ('Q', 16) if big else ('I', 4)
     tmp = path.with_name(path.name + '.part')
-    offsets, counts = [], []
+    offsets = [[0] * (down * across * (count if planar == 2 else 1)) for _, _, down, across in grids]
+    counts = [list(o) for o in offsets]
     try:
         with open(tmp, 'wb') as fh:
             fh.write(b'II' + (struct.pack('<HHHQ', 43, 8, 0, 0) if big else struct.pack('<HI', 42, 0)))
@@ -522,93 +597,106 @@ def write_geotiff(filename, array, transform, crs=None, nodata=None, description
             own_pool = concurrent.futures.ThreadPoolExecutor(max_workers=max(2, os.cpu_count() or 2)) if stream is not None \
                 else None
             try:
-                for data in (own_pool if own_pool is not None else _codec_pool()).map(encode, jobs):
-                    offsets.append(fh.tell())
-                    counts.append(len(data))
+                for (ifd, plane, by, bx), data in zip(jobs, (own_pool if own_pool is not None else _codec_pool()).map(
+                        encode, jobs)):
+                    down, across = grids[ifd][2:]
+                    index = (plane * down + by) * across + bx
+                    offsets[ifd][index] = fh.tell()
+                    counts[ifd][index] = len(data)
                     fh.write(data)
                     if fh.tell() % 2:
                         fh.write(b'\x00')
             finally:
                 if own_pool is not None:
                     own_pool.shutdown(wait=True, cancel_futures=True)
-            # ---- IFD ----
-            entries = []                                            # (tag, type, count, packed value bytes)
-
-            def add(tag, typ, values):
-                if typ == 2:
-                    data = str(values).encode('latin1', 'replace') + b'\x00'
-                    entries.append((tag, 2, len(data), data))
-                else:
-                    fmt = _FIELD[typ][0]
-                    values = list(values)
-                    entries.append((tag, typ, len(values), struct.pack(bo + fmt * len(values), *values)))
-
             if photometric is None:
                 photometric = 'rgb' if (count == 3 and dtype.kind == 'u' and dtype.itemsize == 1) else 'minisblack'
             base = 3 if photometric == 'rgb' else 1
-            add(256, 3 if width < 65536 else 4, [width])
-            add(257, 3 if height < 65536 else 4, [height])
-            add(258, 3, [sample[1]] * count)
-            add(259, 3, [8 if deflate else 1])
-            add(262, 3, [2 if photometric == 'rgb' else 1])
-            add(277, 3, [count])
-            add(284, 3, [planar])
-            add(322, 3, [tw])
-            add(323, 3, [th])
-            add(324, off_type, offsets)
-            add(325, off_type, counts)
-            if count > base:
-                add(338, 3, [0] * (count - base))
-            add(339, 3, [sample[0]] * count)
-            add(33550, 12, [abs(t.a), abs(t.e), 0.0])
-            add(33922, 12, [0.0, 0.0, 0.0, t.c, t.f, 0.0])
-            if geokeys is None:
-                geokeys = getattr(crs, 'raw_geokeys', None)         # a CRS read by GeoTiffReader carries its raw keys
-            if geokeys and geokeys[0]:
-                geokeys = _geokeys_pixel_is_area(geokeys)           # the tie point below is a pixel corner
-                add(34735, 3, geokeys[0])
-                if geokeys[1]:
-                    add(34736, 12, geokeys[1])
-                if geokeys[2]:
-                    add(34737, 2, geokeys[2])
-            xml = _gdal_metadata_xml(tags, band_tags, descriptions)
-            if xml:
-                add(42112, 2, xml)
-            if nodata is not None:
-                add(42113, 2, 'nan' if (isinstance(nodata, float) and math.isnan(nodata)) else repr(
-                    int(nodata) if float(nodata).is_integer() else float(nodata)))
-            entries.sort(key=lambda e: e[0])
-            if fh.tell() % 2:
-                fh.write(b'\x00')
-            # out-of-line values first, then the directory
-            inline = 8 if big else 4
-            placed = []
-            for tag, typ, cnt, data in entries:
-                if len(data) <= inline:
-                    placed.append((tag, typ, cnt, data.ljust(inline, b'\x00')))
+            next_field = 8 if big else 4                            # where the first IFD's offset goes
+            for ifd, (h, w, _, _) in enumerate(grids):
+                # ---- IFD ----
+                entries = []                                        # (tag, type, count, packed value bytes)
+
+                def add(tag, typ, values):
+                    if typ == 2:
+                        data = str(values).encode('latin1', 'replace') + b'\x00'
+                        entries.append((tag, 2, len(data), data))
+                    else:
+                        fmt = _FIELD[typ][0]
+                        values = list(values)
+                        entries.append((tag, typ, len(values), struct.pack(bo + fmt * len(values), *values)))
+
+                if ifd > 0:
+                    add(254, 4, [1])                                # NewSubfileType: reduced-resolution image
+                add(256, 3 if w < 65536 else 4, [w])
+                add(257, 3 if h < 65536 else 4, [h])
+                add(258, 3, [sample[1]] * count)
+                add(259, 3, [8 if deflate else 1])
+                add(262, 3, [2 if photometric == 'rgb' else 1])
+                add(277, 3, [count])
+                add(284, 3, [planar])
+                add(322, 3, [tw])
+                add(323, 3, [th])
+                add(324, off_type, offsets[ifd])
+                add(325, off_type, counts[ifd])
+                if count > base:
+                    add(338, 3, [0] * (count - base))
+                add(339, 3, [sample[0]] * count)
+                if ifd == 0:
+                    add(33550, 12, [abs(t.a), abs(t.e), 0.0])
+                    add(33922, 12, [0.0, 0.0, 0.0, t.c, t.f, 0.0])
+                    if geokeys is None:
+                        geokeys = getattr(crs, 'raw_geokeys', None)  # a CRS read by GeoTiffReader carries its raw keys
+                    if geokeys and geokeys[0]:
+                        geokeys = _geokeys_pixel_is_area(geokeys)    # the tie point below is a pixel corner
+                        add(34735, 3, geokeys[0])
+                        if geokeys[1]:
+                            add(34736, 12, geokeys[1])
+                        if geokeys[2]:
+                            add(34737, 2, geokeys[2])
+                    xml = _gdal_metadata_xml(tags, band_tags, descriptions)
+                    if xml:
+                        add(42112, 2, xml)
+                if nodata is not None:
+                    add(42113, 2, 'nan' if (isinstance(nodata, float) and math.isnan(nodata)) else repr(
+                        int(nodata) if float(nodata).is_integer() else float(nodata)))
+                entries.sort(key=lambda e: e[0])
+                if fh.tell() % 2:
+                    fh.write(b'\x00')
+                # out-of-line values first, then the directory
+                inline = 8 if big else 4
+                placed = []
+                for tag, typ, cnt, data in entries:
+                    if len(data) <= inline:
+                        placed.append((tag, typ, cnt, data.ljust(inline, b'\x00')))
+                    else:
+                        pos = fh.tell()
+                        fh.write(data)
+                        if fh.tell() % 2:
+                            fh.write(b'\x00')
+                        placed.append((tag, typ, cnt, struct.pack(bo + off_fmt, pos)))
+                ifd_pos = fh.tell()
+                if big:
+                    fh.write(struct.pack('<Q', len(placed)))
+                    for tag, typ, cnt, value in placed:
+                        fh.write(struct.pack('<HHQ', tag, typ, cnt) + value)
+                    fh.write(struct.pack('<Q', 0))
+                    end = fh.tell()
+                    fh.seek(next_field)
+                    fh.write(struct.pack('<Q', ifd_pos))
+                    next_field = end - 8
                 else:
-                    pos = fh.tell()
-                    fh.write(data)
-                    if fh.tell() % 2:
-                        fh.write(b'\x00')
-                    placed.append((tag, typ, cnt, struct.pack(bo + off_fmt, pos)))
-            ifd_pos = fh.tell()
-            if big:
-                fh.write(struct.pack('<Q', len(placed)))
-                for tag, typ, cnt, value in placed:
-                    fh.write(struct.pack('<HHQ', tag, typ, cnt) + value)
-                fh.write(struct.pack('<Q', 0))
-                fh.seek(8)
-                fh.write(struct.pack('<Q', ifd_pos))
-            else:
-                if ifd_pos >= 2 ** 32:
-                    raise ValueError('the image does not fit a classic TIFF: pass bigtiff=True')
-                fh.write(struct.pack('<H', len(placed)))
-                for tag, typ, cnt, value in placed:
-                    fh.write(struct.pack('<HHI', tag, typ, cnt) + value)
-                fh.write(struct.pack('<I', 0))
-                fh.seek(4)
-                fh.write(struct.pack('<I', ifd_pos))
+                    if ifd_pos >= 2 ** 32:
+                        raise ValueError('the image does not fit a classic TIFF: pass bigtiff=True')
+                    fh.write(struct.pack('<H', len(placed)))
+                    for tag, typ, cnt, value in placed:
+                        fh.write(struct.pack('<HHI', tag, typ, cnt) + value)
+                    fh.write(struct.pack('<I', 0))
+                    end = fh.tell()
+                    fh.seek(next_field)
+                    fh.write(struct.pack('<I', ifd_pos))
+                    next_field = end - 4
+                fh.seek(end)
     except BaseException:
         # (a failed write -- e.g. a band stream whose producer failed -- leaves no partial file behind)
         try:

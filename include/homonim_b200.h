@@ -35,10 +35,11 @@
 extern "C" {
 #endif
 
-#define HB_ABI_VERSION 7
+#define HB_ABI_VERSION 8
 
 /* storage dtype of a source raster plane */
-enum { HB_U8 = 0, HB_U16 = 1, HB_F32 = 2, HB_I16 = 3 };   /* HB_I16: output dtypes only (out_dtype, hb_convert_dtype) */
+enum { HB_U8 = 0, HB_U16 = 1, HB_F32 = 2, HB_I16 = 3 };   /* HB_I16: output dtypes only (out_dtype, hb_convert_dtype,
+                                                             hb_build_overviews) */
 /* homonim.enums.Model (homonim/enums.py:22-42) */
 enum { HB_MODEL_GAIN = 0, HB_MODEL_GAIN_BLK_OFFSET = 1, HB_MODEL_GAIN_OFFSET = 2 };
 /* up-sampling methods of hb_resample_up */
@@ -244,6 +245,22 @@ int hb_fuse_refspace_host(const void *src_host, int src_dtype, long hs, long ws,
                           double ref_nodata, double sx, double ox, double sy, double oy, int model, int kh, int kw,
                           int want_r2, int do_inpaint, double r2_thresh, int out_dtype, int out_has_nodata,
                           double out_nodata, void *corr_host, float *params_host, void *stream);
+
+/* ---------------------------------------------------------------------------------------------------------------
+ * Overview pyramid of written planes: RasterFuse._build_overviews (homonim/fuse.py:151-165, Resampling.average) on the
+ * corrected / parameter planes as they are stored in the output file.
+ *   src        [nb][h][w] of `dtype` (HB_U8, HB_U16, HB_I16 or HB_F32), the written values (output dtype and nodata).
+ *   levels_dev HOST array of n_levels (1..8) DEVICE pointers; level k (1-based) is [nb][ceil(h / 2^k)][ceil(w / 2^k)] of
+ *              the same dtype.
+ * Level k is computed from level k - 1 as stored (level 0 = src): pixel (i, j) averages the valid pixels among rows 2i,
+ * 2i+1 and columns 2j, 2j+1 of level k - 1 (rows / columns past an odd edge are absent).  Valid = not equal to nodata
+ * (when has_nodata) and, for HB_F32, not NaN; a window without valid pixels gets nodata (NaN for HB_F32 without one).
+ * Integer types: floor((2s + n) / 2n) of the exact sum s of the n valid pixels (round half up).  HB_F32: the valid
+ * values summed in double in the order top-left, top-right, bottom-left, bottom-right, divided by n in double, rounded
+ * once to float.  Two kernel launches at most (levels 1-6 from one read of the plane, then levels 7-8).
+ * --------------------------------------------------------------------------------------------------------------- */
+int hb_build_overviews(const void *src_dev, int dtype, long nb, long h, long w, int has_nodata, double nodata,
+                       int n_levels, void *const *levels_dev, void *stream);
 
 #ifdef __cplusplus
 }
