@@ -360,6 +360,15 @@ upsample_prep_kernel(const float *__restrict__ coarse, long hp, long wp, float2 
 // =====================================================================================================================
 struct __align__(16) RowEntry { float wy[4]; };            // the row's B-spline y-weights (taps ky-1 .. ky+2)
 
+// upsample_poly_kernel's row table: everything a destination row needs in one 32-byte entry (one LDS.128 + one LDS.64)
+struct __align__(32) PolyRow {
+    float wy[4];    // the row's B-spline y-weights (taps ky-1 .. ky+2)
+    int ky;         // first tap row + 1, clamped to [-4, hp + 4] (non-decreasing: sy > 0); INT_MAX past the CTA's rows
+    float sy;       // sum of the y-weights: exactly 1.0f unless taps were dropped
+    int pad[2];
+};
+constexpr int kPolyRowTableBytes = (kMaxRows + kRb - 1) * (int)sizeof(PolyRow);   // (+ pad entries of a partial stage)
+
 #ifndef HB_POLY_MIN_CTAS
 #define HB_POLY_MIN_CTAS 2
 #endif
@@ -384,27 +393,29 @@ upsample_poly_kernel(const T *__restrict__ src, NoData nd, const void *__restric
     const int nrows = (int)min((long)rows_per_cta, g.hs - Y0);
     const float qnan = __int_as_float(0x7fc00000);
 
-    // per-CTA row table: y-weights and first tap row (+1) of the CTA's destination rows
-    RowEntry *s_rows = reinterpret_cast<RowEntry *>(smem_raw);
-    int *s_ky = reinterpret_cast<int *>(smem_raw + kMaxRows * sizeof(RowEntry));
-    float *s_sy = reinterpret_cast<float *>(smem_raw + kMaxRows * (sizeof(RowEntry) + sizeof(int)));
-    if ((int)threadIdx.x < nrows) {
-        double wy[4];
-        long ky;
-        up_axis_weights(g.sy, g.oy, Y0 + threadIdx.x, g.hp, wy, ky);
-        RowEntry e;
+    // per-CTA row table of the CTA's destination rows, padded to whole stages (rows are processed a stage at a time)
+    PolyRow *s_rows = reinterpret_cast<PolyRow *>(smem_raw);
+    if ((int)threadIdx.x < nrows + kRb - 1) {
+        PolyRow e = {{0.f, 0.f, 0.f, 0.f}, INT_MAX, 0.f, {0, 0}};
+        if ((int)threadIdx.x < nrows) {
+            double wy[4];
+            long ky;
+            up_axis_weights(g.sy, g.oy, Y0 + threadIdx.x, g.hp, wy, ky);
 #pragma unroll
-        for (int j = 0; j < 4; j++) e.wy[j] = (float)wy[j];
+            for (int j = 0; j < 4; j++) e.wy[j] = (float)wy[j];
+            e.ky = (int)min(max(ky, -4L), g.hp + 4);
+            e.sy = (float)(((wy[0] + wy[1]) + wy[2]) + wy[3]);
+        }
         s_rows[threadIdx.x] = e;
-        s_ky[threadIdx.x] = (int)min(max(ky, -4L), g.hp + 4);
-        s_sy[threadIdx.x] = (float)(((wy[0] + wy[1]) + wy[2]) + wy[3]);      // exactly 1.0f unless taps were dropped
     }
     __syncthreads();                                        // the only CTA barrier
 
     const long X0 = ((long)blockIdx.x * kWarps + warp) * kWarpW + (long)lane * kPpt;
     if (X0 - lane * kPpt >= g.ws) return;                   // the whole warp is beyond the raster
-    const bool lane_in = X0 < g.ws;                         // (ws % 4 == 0: a lane is wholly inside or outside)
-    unsigned char *warp_base = smem_raw + kRowTableBytes + warp * (kWBytes + kRingBytes);
+    int lane_in_i = X0 < g.ws;                              // (ws % 4 == 0: a lane is wholly inside or outside)
+    asm("" : "+r"(lane_in_i));                              // (kept in a register, not re-derived at every stage)
+    const bool lane_in = lane_in_i != 0;
+    unsigned char *warp_base = smem_raw + kPolyRowTableBytes + warp * (kWBytes + kRingBytes);
     float4 *s_w = reinterpret_cast<float4 *>(warp_base) + lane;            // s_w[i * 32]: tap i of the lane's 4 pixels
     const uint32_t ring_sa = (uint32_t)__cvta_generic_to_shared(warp_base + kWBytes + lane * kLaneBytes);
 
@@ -421,7 +432,8 @@ upsample_poly_kernel(const T *__restrict__ src, NoData nd, const void *__restric
                     cp_async_lane<kLaneBytes>(pf_dst + rr * kRowBytes, pf);
                     pf += pitch_b;
                 }
-            } else {
+            } else {                                        // (the CTA's last, partial stage)
+#pragma unroll 1
                 for (int rr = 0; rr < pf_left; rr++) {
                     cp_async_lane<kLaneBytes>(pf_dst + rr * kRowBytes, pf);
                     pf += pitch_b;
@@ -468,10 +480,16 @@ upsample_poly_kernel(const T *__restrict__ src, NoData nd, const void *__restric
     // cells outside the flag table hold no pixel with an in-range centre: DEAD
     auto cell_flags = [&](int ky, int cell) -> unsigned {
         if (ky < -1 || ky > hp || cell < 0 || cell >= fw) return 6u;
-        return flags[(long)(ky + 1) * fw + cell];
+        return flags[(ky + 1) * fw + cell];
     };
+    // the lane's tap columns; taps outside the raster have weight 0 (x-weights / row table): read the clamped position
+    int coff[5];
+#pragma unroll
+    for (int i = 0; i < 5; i++) coff[i] = min(max(col0 + i, 0), wp - 1);
+    const bool five = (cellB != cellA);                     // some pixel's window starts one column in: 5th column is used
 
-    const typename SrcQuad<T>::Key nd_key = SrcQuad<T>::key(nd);
+    typename SrcQuad<T>::Key nd_key = SrcQuad<T>::key(nd);
+    if constexpr (sizeof(nd_key) == 4) asm("" : "+r"(nd_key));   // (kept in a register, not re-derived at every row)
     // x-interpolated tap rows per pixel PAIR and band.  CLEAN lanes: the interpolated values; DEAD lanes: NaN (so that
     // the row arithmetic produces nodata by itself); DIRTY lanes / lanes beyond the raster: stale, never stored.
     //
@@ -479,138 +497,118 @@ upsample_poly_kernel(const T *__restrict__ src, NoData nd, const void *__restric
     //     sum_i w_i t_i  =  base * sum_i w_i  +  sum_i w_i (t_i - base)
     // The parameter planes are smooth, so the second term is small and its float32 rounding errors vanish against the
     // result, while the first is exact (sum_i w_i == 1.0f wherever no tap was dropped) -- the float32 parameter the
-    // reference gets from GDAL's double-precision accumulation comes out correctly rounded in all but near-tie cases,
-    // and gain * src + offset is then formed with numpy's two float32 roundings (kernel_model.py:461).
+    // reference gets from GDAL's double-precision accumulation comes out correctly rounded in all but near-tie cases.
     float2 q[2][NB][4];
     float base[NB];
+    float2 base2[NB];                                       // (base, base): an operand of every row's packed FMA
 #pragma unroll
-    for (int b = 0; b < NB; b++) base[b] = 0.f;
+    for (int b = 0; b < NB; b++) base[b] = 0.f, base2[b] = splat(0.f);
     const float4 sx4 = s_w[5 * 32];
     int q_ky = INT_MIN;
     bool do_store = false;
-    long opix = Y0 * g.ws + X0;                             // pixel index of the lane's 4 pixels in the output plane
-    const long out_pitch = g.ws;
-    uint32_t ring_rd = ring_sa;                             // this lane's pixels of the current row in the ring
-    // the row table entry of row r + 1 is fetched while row r is computed (the loop is a chain of short dependent
-    // steps with only a few warps per scheduler to hide shared-memory latency behind)
-    int ky_next = s_ky[0];
-    RowEntry ri_next = s_rows[0];
-    float sy_next = s_sy[0];
-#pragma unroll 1
-    for (int r = 0; r < nrows; r++, opix += out_pitch) {
-        if (APPLY && (r & (kRb - 1)) == 0) {                // (warp-uniform) a new stage: keep the ring full, wait for it
-            prefetch();
-            cp_async_wait<kStages - 1>();
+
+    // ---- new tap rows `ky` (once per cell row): re-classify the lane, re-interpolate its pixel columns -----------------
+    auto reinterpolate = [&](int ky) {
+        q_ky = ky;
+        const unsigned fa = cell_flags(ky, cellA), fb = cell_flags(ky, cellB);
+        if (lane_in) {
+            // next cell row's flags -> L1 (the flag load heads the dependency chain of every re-interpolation)
+            const int nf = min(max(ky + 2, 0), hp + 1) * fw;
+            asm volatile("prefetch.global.L1 [%0];" ::"l"(flags + nf + min(max(cellA, 0), fw - 1)));
+            asm volatile("prefetch.global.L1 [%0];" ::"l"(flags + nf + min(max(cellB, 0), fw - 1)));
         }
-        const int ky = ky_next;
-        const RowEntry ri = ri_next;
-        const float sy = sy_next;
-        {
-            const int rn = min(r + 1, nrows - 1);
-            ky_next = s_ky[rn];
-            ri_next = s_rows[rn];
-            sy_next = s_sy[rn];
+        // 0: CLEAN, 1: SKIP (DIRTY: left to the fix-up kernel; or a lane beyond the raster), 2: DEAD.
+        // A CLEAN cell next to an OUT cell: the OUT cell's pixel columns carry NaN x-weights.
+        const bool clean2 = ((fa | fb) & 1u) && (fa & 5u) && (fb & 5u);
+        const int state = !lane_in ? 1 : (clean2 ? 0 : ((fa & fb & 2u) ? 2 : 1));
+        do_store = (state != 1);
+        if (state == 2) {
+#pragma unroll
+            for (int p = 0; p < 2; p++)
+#pragma unroll
+                for (int b = 0; b < NB; b++)
+#pragma unroll
+                    for (int j = 0; j < 4; j++) q[p][b][j] = splat(qnan);
         }
-        if (ky != q_ky) {                                   // (warp-uniform) new tap rows: re-classify, re-interpolate
-            q_ky = ky;
-            const unsigned fa = cell_flags(ky, cellA), fb = cell_flags(ky, cellB);
-            if (lane_in) {
-                // next cell row's flags -> L1 (the flag load heads the dependency chain of every re-interpolation)
-                const long nf = (long)min(max(ky + 2, 0), hp + 1) * fw;
-                asm volatile("prefetch.global.L1 [%0];" ::"l"(flags + nf + min(max(cellA, 0), fw - 1)));
-                asm volatile("prefetch.global.L1 [%0];" ::"l"(flags + nf + min(max(cellB, 0), fw - 1)));
+        if (lane_in) {
+            // the NEXT cell row re-uses 3 of these tap rows (L1 hits by then); pull its one new row into L1 now, so
+            // that the whole CTA does not stall on L2 at its next (simultaneous) re-interpolation
+            const int nrow = min(max(ky + 3, 0), hp - 1) * wp + coff[0];
+            const char *np = reinterpret_cast<const char *>(coarse_v) + (long)nrow * (NB == 2 ? 8 : 4);
+            asm volatile("prefetch.global.L1 [%0];" ::"l"(np));
+            asm volatile("prefetch.global.L1 [%0];" ::"l"(np + (NB == 2 ? 32 : 16)));
+        }
+        if (state == 0) {
+            float2 wp01[5], wp23[5];
+#pragma unroll
+            for (int i = 0; i < 5; i++) {
+                const float4 w = s_w[i * 32];
+                wp01[i] = make_float2(w.x, w.y);
+                wp23[i] = make_float2(w.z, w.w);
             }
-            // 0: CLEAN, 1: SKIP (DIRTY: left to the fix-up kernel; or a lane beyond the raster), 2: DEAD.
-            // A CLEAN cell next to an OUT cell: the OUT cell's pixel columns carry NaN x-weights.
-            const bool clean2 = ((fa | fb) & 1u) && (fa & 5u) && (fb & 5u);
-            const int state = !lane_in ? 1 : (clean2 ? 0 : ((fa & fb & 2u) ? 2 : 1));
-            do_store = (state != 1);
-            if (state == 2) {
-#pragma unroll
-                for (int p = 0; p < 2; p++)
-#pragma unroll
-                    for (int b = 0; b < NB; b++)
-#pragma unroll
-                        for (int j = 0; j < 4; j++) q[p][b][j] = splat(qnan);
-            }
-            if (lane_in) {
-                // the NEXT cell row re-uses 3 of these tap rows (L1 hits by then); pull its one new row into L1 now, so
-                // that the whole CTA does not stall on L2 at its next (simultaneous) re-interpolation
-                const long nrow = (long)min(max(ky + 3, 0), hp - 1) * wp + min(max(col0, 0), wp - 1);
-                const char *np = reinterpret_cast<const char *>(coarse_v) + nrow * (NB == 2 ? 8 : 4);
-                asm volatile("prefetch.global.L1 [%0];" ::"l"(np));
-                asm volatile("prefetch.global.L1 [%0];" ::"l"(np + (NB == 2 ? 32 : 16)));
-            }
-            if (state == 0) {
-                const bool five = (cellB != cellA);         // some pixel's window starts one column in: 5th column is used
-                // taps outside the raster have weight 0 (x-weights / row table): read the clamped position
-                int coff[5];
-#pragma unroll
-                for (int i = 0; i < 5; i++) coff[i] = min(max(col0 + i, 0), wp - 1);
-                float2 wp01[5], wp23[5];
-#pragma unroll
-                for (int i = 0; i < 5; i++) {
-                    const float4 w = s_w[i * 32];
-                    wp01[i] = make_float2(w.x, w.y);
-                    wp23[i] = make_float2(w.z, w.w);
-                }
-                {
-                    // base: the coarse pixel at tap row 1, tap column 1 of the lane's window (inside the raster, hence
-                    // usable in a CLEAN cell)
-                    const long boff = (long)min(max(ky, 0), hp - 1) * wp + coff[1];
-                    if (NB == 2) {
-                        const float2 v = __ldg(reinterpret_cast<const float2 *>(coarse_v) + boff);
-                        base[0] = v.x;
-                        base[NB - 1] = v.y;
-                    } else {
-                        base[0] = __ldg(reinterpret_cast<const float *>(coarse_v) + boff);
-                    }
+            {
+                // base: the coarse pixel at tap row 1, tap column 1 of the lane's window (inside the raster, hence
+                // usable in a CLEAN cell)
+                const int boff = min(max(ky, 0), hp - 1) * wp + coff[1];
+                if (NB == 2) {
+                    const float2 v = __ldg(reinterpret_cast<const float2 *>(coarse_v) + boff);
+                    base[0] = v.x;
+                    base[NB - 1] = v.y;
+                } else {
+                    base[0] = __ldg(reinterpret_cast<const float *>(coarse_v) + boff);
                 }
 #pragma unroll
-                for (int j = 0; j < 4; j++) {
-                    const long row_off = (long)min(max(ky - 1 + j, 0), hp - 1) * wp;
-                    float t[NB][5];
-                    if (NB == 2) {
-                        const float2 *p = reinterpret_cast<const float2 *>(coarse_v) + row_off;
+                for (int b = 0; b < NB; b++) base2[b] = splat(base[b]);
+            }
 #pragma unroll
-                        for (int i = 0; i < 5; i++) {
-                            // (the 5th column has weight 0 when unused, but may be NaN: skip it)
-                            const float2 v = (i < 4 || five) ? __ldg(p + coff[i]) : make_float2(base[0], base[NB - 1]);
-                            t[0][i] = __fsub_rn(v.x, base[0]);
-                            t[NB - 1][i] = __fsub_rn(v.y, base[NB - 1]);
-                        }
-                    } else {
-                        const float *p = reinterpret_cast<const float *>(coarse_v) + row_off;
+            for (int j = 0; j < 4; j++) {
+                const int row_off = min(max(ky - 1 + j, 0), hp - 1) * wp;     // (hp * wp < 2^31: launch_poly)
+                float t[NB][5];
+                if (NB == 2) {
+                    const float2 *p = reinterpret_cast<const float2 *>(coarse_v);
 #pragma unroll
-                        for (int i = 0; i < 5; i++) t[0][i] = __fsub_rn((i < 4 || five) ? __ldg(p + coff[i]) : base[0], base[0]);
+                    for (int i = 0; i < 5; i++) {
+                        // (the 5th column has weight 0 when unused, but may be NaN: skip it)
+                        const float2 v = (i < 4 || five) ? __ldg(p + (row_off + coff[i])) : make_float2(base[0], base[NB - 1]);
+                        t[0][i] = __fsub_rn(v.x, base[0]);
+                        t[NB - 1][i] = __fsub_rn(v.y, base[NB - 1]);
                     }
+                } else {
+                    const float *p = reinterpret_cast<const float *>(coarse_v);
 #pragma unroll
-                    for (int b = 0; b < NB; b++) {          // x-interpolation of tap row j at the lane's 4 pixel columns
-                        float2 r0 = fmul2(wp01[0], splat(t[b][0])), r1 = fmul2(wp23[0], splat(t[b][0]));
+                    for (int i = 0; i < 5; i++)
+                        t[0][i] = __fsub_rn((i < 4 || five) ? __ldg(p + (row_off + coff[i])) : base[0], base[0]);
+                }
 #pragma unroll
-                        for (int i = 1; i < 5; i++) {
-                            r0 = ffma2(wp01[i], splat(t[b][i]), r0);
-                            r1 = ffma2(wp23[i], splat(t[b][i]), r1);
-                        }
-                        q[0][b][j] = r0;
-                        q[1][b][j] = r1;
+                for (int b = 0; b < NB; b++) {              // x-interpolation of tap row j at the lane's 4 pixel columns
+                    float2 r0 = fmul2(wp01[0], splat(t[b][0])), r1 = fmul2(wp23[0], splat(t[b][0]));
+#pragma unroll
+                    for (int i = 1; i < 5; i++) {
+                        r0 = ffma2(wp01[i], splat(t[b][i]), r0);
+                        r1 = ffma2(wp23[i], splat(t[b][i]), r1);
                     }
+                    q[0][b][j] = r0;
+                    q[1][b][j] = r1;
                 }
             }
         }
-        // ---- one destination row: 4 multiply-adds per pixel pair and band with the row's y-weights, fused apply ------------
-        const float2 w0 = splat(ri.wy[0]), w1 = splat(ri.wy[1]), w2 = splat(ri.wy[2]), w3 = splat(ri.wy[3]);
+    };
+
+    // ---- one destination row: 4 multiply-adds per pixel pair and band with the row's y-weights, fused apply ------------
+    // `rd`: the lane's source pixels of the row in the ring; `pix`: pixel index of the lane's 4 pixels in the output plane
+    auto dest_row = [&](const PolyRow &e, uint32_t rd, long pix) {
+        const float2 w0 = splat(e.wy[0]), w1 = splat(e.wy[1]), w2 = splat(e.wy[2]), w3 = splat(e.wy[3]);
         float2 gv[2], ov[2];
 #pragma unroll
         for (int p = 0; p < 2; p++) {
             // weight sum of the pixel = (sum of its x-weights) * (sum of the row's y-weights): 1.0f away from the edges
-            const float2 wsum = fmul2(p == 0 ? make_float2(sx4.x, sx4.y) : make_float2(sx4.z, sx4.w), splat(sy));
+            const float2 wsum = fmul2(p == 0 ? make_float2(sx4.x, sx4.y) : make_float2(sx4.z, sx4.w), splat(e.sy));
             const float2 dg = ffma2(q[p][0][3], w3, ffma2(q[p][0][2], w2, ffma2(q[p][0][1], w1, fmul2(q[p][0][0], w0))));
-            gv[p] = ffma2(splat(base[0]), wsum, dg);
+            gv[p] = ffma2(base2[0], wsum, dg);
             if (NB > 1) {
                 const float2 dof = ffma2(q[p][NB - 1][3], w3, ffma2(q[p][NB - 1][2], w2, ffma2(q[p][NB - 1][1], w1,
                                          fmul2(q[p][NB - 1][0], w0))));
-                ov[p] = ffma2(splat(base[NB - 1]), wsum, dof);
+                ov[p] = ffma2(base2[NB - 1], wsum, dof);
             } else {
                 ov[p] = splat(0.f);
             }
@@ -619,19 +617,44 @@ upsample_poly_kernel(const T *__restrict__ src, NoData nd, const void *__restric
         if constexpr (APPLY) {
             float2 s[2];
             bool ok[4];
-            SrcQuad<T>::get_shared(ring_rd, nd_key, s, ok);
-            ring_rd = (ring_rd + kRowBytes == ring_sa + kRingBytes) ? ring_sa : ring_rd + kRowBytes;
-            // corr = gain * src + offset with numpy's two float32 roundings (kernel_model.py:461)
-            const float2 c0 = fadd2(fmul2(gv[0], s[0]), ov[0]), c1 = fadd2(fmul2(gv[1], s[1]), ov[1]);
+            SrcQuad<T>::get_shared(rd, nd_key, s, ok);
+            // corr = gain * src + offset as ONE fused multiply-add, rounded once (DESIGN.md 4.5)
+            const float2 c0 = ffma2(gv[0], s[0], ov[0]), c1 = ffma2(gv[1], s[1], ov[1]);
             res[0] = make_float4(ok[0] ? c0.x : qnan, ok[1] ? c0.y : qnan, ok[2] ? c1.x : qnan, ok[3] ? c1.y : qnan);
         } else {
             res[0] = make_float4(gv[0].x, gv[0].y, gv[1].x, gv[1].y);
             if constexpr (NOUT == 2) res[1] = make_float4(ov[0].x, ov[0].y, ov[1].x, ov[1].y);
         }
         if (do_store) {                                     // (DIRTY lanes are written by the fix-up kernel)
-            if constexpr (APPLY && CONVERT) hb_store4_out(out, opix, res[0], g.ospec);   // output dtype conversion in the store
-            else hb_stg_stream16(out + opix, res[0]);
-            if constexpr (NOUT == 2) hb_stg_stream16(out + g.hs * g.ws + opix, res[1]);
+            if constexpr (APPLY && CONVERT) hb_store4_out(out, pix, res[0], g.ospec);   // output dtype conversion in the store
+            else hb_stg_stream16(out + pix, res[0]);
+            if constexpr (NOUT == 2) hb_stg_stream16(out + g.hs * g.ws + pix, res[1]);
+        }
+    };
+
+    // ---- the rows, one ring stage (kRb rows) per iteration ----------------------------------------------------------------
+    long opix = Y0 * g.ws + X0;
+    const long out_pitch = g.ws;
+#pragma unroll 1
+    for (int r = 0; r < nrows; r += kRb, opix += kRb * out_pitch) {
+        if (APPLY) {                                        // keep the ring full, wait for this stage
+            prefetch();
+            cp_async_wait<kStages - 1>();
+        }
+        const uint32_t rd = ring_sa + (uint32_t)(r & (kStages * kRb - 1)) * kRowBytes;
+        // (warp-uniform) the tap rows are non-decreasing in the row and q_ky is the previous row's: if the stage's last
+        // row still has them, so does every row of the stage
+        if (s_rows[r + kRb - 1].ky == q_ky) {
+#pragma unroll
+            for (int h = 0; h < kRb; h++) dest_row(s_rows[r + h], rd + h * kRowBytes, opix + h * out_pitch);
+        } else {                                            // new tap rows in this stage, or the CTA's partial last stage
+            const int n = min(kRb, nrows - r);
+#pragma unroll 1
+            for (int h = 0; h < n; h++) {
+                const PolyRow e = s_rows[r + h];
+                if (e.ky != q_ky) reinterpolate(e.ky);
+                dest_row(e, rd + h * kRowBytes, opix + h * out_pitch);
+            }
         }
     }
 }
@@ -830,9 +853,9 @@ upsample_yfirst_kernel(const T *__restrict__ src, NoData nd, const void *__restr
             bool ok[4];
             SrcQuad<T>::get_shared(ring_rd, nd_key, s, ok);
             ring_rd = (ring_rd + kRowBytes == ring_sa + kRingBytes) ? ring_sa : ring_rd + kRowBytes;
-            // corr = gain * src + offset with numpy's two float32 roundings (kernel_model.py:461)
-            const pk2 c0 = pk_add(pk_mul(o[0][0], pk(s[0].x, s[0].y)), o[NB - 1][0]);
-            const pk2 c1 = pk_add(pk_mul(o[0][1], pk(s[1].x, s[1].y)), o[NB - 1][1]);
+            // corr = gain * src + offset as ONE fused multiply-add, rounded once (DESIGN.md 4.5)
+            const pk2 c0 = pk_fma(o[0][0], pk(s[0].x, s[0].y), o[NB - 1][0]);
+            const pk2 c1 = pk_fma(o[0][1], pk(s[1].x, s[1].y), o[NB - 1][1]);
             res[0] = make_float4(ok[0] ? pk_lo(c0) : qnan, ok[1] ? pk_hi(c0) : qnan, ok[2] ? pk_lo(c1) : qnan,
                                  ok[3] ? pk_hi(c1) : qnan);
         } else {
@@ -1240,7 +1263,8 @@ int launch_poly(const void *src, NoData nd, const float *coarse, const UpPolyGeo
         // a lane spanning 3 coarse cells (fewer than ~3.4 destination pixels per coarse pixel): the "y first" kernel
         const bool yfirst = (g.sx > 0.3);
         const size_t ring = APPLY ? (size_t)kStages * kRb * 32 * kPpt * sizeof(T) : 0;
-        const size_t smem = kRowTableBytes + ((yfirst ? kYfCols : 6) * 32 * sizeof(float4) + ring) * kWarps;
+        const size_t smem = (yfirst ? kRowTableBytes : kPolyRowTableBytes) +
+                            ((yfirst ? kYfCols : 6) * 32 * sizeof(float4) + ring) * kWarps;
         const long cta_w = (long)kWarpW * kWarps;
         const long gx = (g.ws + cta_w - 1) / cta_w;
         // (CONVERT: an output dtype / nodata other than plain float32 -- its own instantiation, so that the float32 path's
