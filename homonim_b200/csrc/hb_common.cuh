@@ -219,12 +219,6 @@ template <class F> static inline int hb_once_per_device(HbOncePerDevice &once, F
     return rc;
 }
 
-// high-priority side stream with a fork / join event pair (defined in upsample_poly.cu); nullptr when none could be made.
-// The caller holds `mu` from the fork record to the join wait (a few host-side enqueues): the events of a slot are
-// re-recorded by every user, so two host threads must not interleave on one slot.
-struct SideStream { cudaStream_t s; cudaEvent_t fork, join; bool ok; std::mutex mu; };
-SideStream *hb_side_stream();
-
 static inline int hb_sm_count()
 {
     static int sms = 0;
@@ -235,4 +229,14 @@ static inline int hb_sm_count()
             sms = 148;
     }
     return sms;
+}
+
+// blocks of a grid-stride launch over n items: one item per thread, at most `per_sm` blocks per SM
+static inline unsigned hb_grid_for(long n, int threads, int per_sm = 8)
+{
+    long blocks = (n + threads - 1) / threads;
+    const long cap = (long)hb_sm_count() * per_sm;
+    if (blocks > cap) blocks = cap;
+    if (blocks < 1) blocks = 1;
+    return (unsigned)blocks;
 }

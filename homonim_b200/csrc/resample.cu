@@ -1,21 +1,16 @@
-// resample.cu -- grid-changing kernels of the kernel-model path (sm_100a):
+// resample.cu -- down-sampling and element-wise kernels of the kernel-model path (sm_100a):
 //   * hb_downsample_average : RasterArray.reproject(resampling=average)     (reference raster_array.py:526-578,
 //                             kernel_model.py:480)                            [HBM-bound: reads every hi-res pixel]
-//   * hb_upsample_apply     : RefSpaceModel.apply = cubic-spline up-sampling of (gain, offset) fused with
-//                             corr = gain*src + offset                        (kernel_model.py:484-503, 442-463)
-//   * hb_resample_up        : plain cubic-spline / nearest up-sampling        (kernel_model.py:491, 497, 520)
 //   * hb_apply_same_grid, hb_valid_mask, hb_full_coverage_mask                (kernel_model.py:375-409, 442-463)
+//   * hb_convert_dtype      : output dtype conversion                         (raster_array.py:353-387)
+// Up-sampling (hb_upsample_apply, hb_resample_up) lives in upsample.cu.
 //
 // The GDAL algorithms restated here are specified in oracle/gdal_restate.c (GDAL itself is not in this image).
-#include <limits.h>
 #include <type_traits>
 
 #include "hb_common.cuh"
-#include "upsample_poly.cuh"
 
 namespace {
-
-constexpr int kThreads = 256;
 
 // =====================================================================================================================
 // 1. average down-sampling
@@ -62,7 +57,6 @@ template <> struct Raw8<float> {
     }
 };
 
-template <typename T> constexpr int hb_dtype_code() { return sizeof(T) == 1 ? HB_U8 : (sizeof(T) == 2 ? HB_U16 : HB_F32); }
 template <typename T> struct IsInt { static constexpr bool value = true; };
 template <> struct IsInt<float> { static constexpr bool value = false; };
 
@@ -489,453 +483,7 @@ int launch_downsample(const void *src, long hs, long ws, NoData nd, float *dst, 
 }
 
 // =====================================================================================================================
-// 2. cubic-spline up-sampling, optionally fused with the apply step
-// =====================================================================================================================
-// GDAL GRA_CubicSpline (4x4 cubic B-spline taps, invalid / out-of-range taps dropped and the rest renormalised; spec in
-// oracle/gdal_restate.c).  After a one-off per-CTA table of the rows' y-geometry, every WARP is autonomous (no further
-// CTA barrier): it owns a 128-pixel-wide column strip (4 pixels per lane, vector stores) and walks down it row by row.
-// Source pixels arrive through a 4-deep cp.async ring (each lane copies, and later reads, only its own bytes).
-//
-//   (Destinations >= ~3.4x finer than the coarse grid take the polynomial fast path of upsample_poly.cu instead; this
-//   kernel handles small ratios, unaligned rasters and the coverage mask of mask_partial.)
-//   Per destination row:
-//     A. lane <-> coarse column: combine the column's 4 tap rows (register cache, invalid taps zeroed + validity mask)
-//        with the row's y-weights into warp-private shared memory (values, weight sums, flags);
-//     C. lane <-> 4 pixels: sum the 4 column combinations with the pixel's x-weights, apply GDAL's centre-pixel and
-//        renormalisation rules.
-// In APPLY mode the up-sampled parameters never exist in memory.
-struct __align__(16) Pair { double g, o; };          // band 0 (gain) and band 1 (offset)
-struct __align__(16) RowInfo {
-    double dy;        // fractional row position inside the cell row
-    int ky;           // first tap row + 1
-    int jc;           // tap row hosting the centre pixel (1 or 2; 0 when clamped), -1: centre row out of range
-    int cy;           // coarse row of the centre pixel
-    int pad;
-};
-
-#ifndef HB_UP_MIN_CTAS
-#define HB_UP_MIN_CTAS 2
-#endif
-constexpr int kUpPpt = 4;                             // destination pixels per lane
-constexpr int kUpWarpW = 32 * kUpPpt;                 // destination columns per warp
-constexpr int kUpWarps = kThreads / 32;
-constexpr int kUpRb = 4;                              // rows per cp.async stage
-constexpr int kUpStages = 4;                          // stages of source rows in flight per warp
-constexpr int kUpMaxRows = 64;                        // destination rows per CTA (upper bound)
-
-__device__ __forceinline__ void bspline_weights(double d, double (&w)[4])   // taps -1, 0, 1, 2: B(tap - d)
-{
-    const double u = 1.0 - d, d2 = d * d, u2 = u * u;
-    w[0] = u2 * u * (1.0 / 6.0);
-    w[1] = (4.0 + d2 * (3.0 * d - 6.0)) * (1.0 / 6.0);
-    w[2] = (4.0 + u2 * (3.0 * u - 6.0)) * (1.0 / 6.0);
-    w[3] = d2 * d * (1.0 / 6.0);
-}
-
-// asynchronous global -> shared copy of one lane's 4 source pixels (LDGSTS; completion via wait_group)
-template <int BYTES> __device__ __forceinline__ void cp_async_lane(uint32_t smem_dst, const void *gmem_src)
-{
-    if (BYTES == 16) asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_dst), "l"(gmem_src) : "memory");
-    else asm volatile("cp.async.ca.shared.global [%0], [%1], %2;" ::"r"(smem_dst), "l"(gmem_src), "n"(BYTES) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-
-// 4 source pixels of storage type T -> float32, plus their validity against the nodata value
-template <typename T> struct Src4;
-template <> struct Src4<uint16_t> {
-    static constexpr int kBytes = 8;
-    static __device__ __forceinline__ void get(const void *p, const NoData &nd, float (&v)[4], bool (&ok)[4])
-    {
-        const uint2 w = *reinterpret_cast<const uint2 *>(p);
-        const uint32_t r[4] = {w.x & 0xFFFFu, w.x >> 16, w.y & 0xFFFFu, w.y >> 16};
-#pragma unroll
-        for (int k = 0; k < 4; k++) {
-            v[k] = __uint_as_float(0x4B000000u | r[k]) - 8388608.0f;      // exact, no I2F
-            ok[k] = (int)r[k] != nd.ivalue;                                // ivalue = -1 when no integer nodata
-        }
-    }
-};
-template <> struct Src4<uint8_t> {
-    static constexpr int kBytes = 4;
-    static __device__ __forceinline__ void get(const void *p, const NoData &nd, float (&v)[4], bool (&ok)[4])
-    {
-        const uint32_t w = *reinterpret_cast<const uint32_t *>(p);
-#pragma unroll
-        for (int k = 0; k < 4; k++) {
-            const uint32_t r = (w >> (8 * k)) & 0xFFu;
-            v[k] = __uint_as_float(0x4B000000u | r) - 8388608.0f;
-            ok[k] = (int)r != nd.ivalue;
-        }
-    }
-};
-template <> struct Src4<float> {
-    static constexpr int kBytes = 16;
-    static __device__ __forceinline__ void get(const void *p, const NoData &nd, float (&v)[4], bool (&ok)[4])
-    {
-        const float4 w = *reinterpret_cast<const float4 *>(p);
-        v[0] = w.x; v[1] = w.y; v[2] = w.z; v[3] = w.w;
-#pragma unroll
-        for (int k = 0; k < 4; k++) ok[k] = hb_valid(v[k], nd);
-    }
-};
-
-struct UpGeom {
-    long hs, ws;          // destination (fine) grid
-    long hp, wp;          // coarse grid
-    double sx, ox, sy, oy;
-    int ncols;            // coarse columns staged per warp (cells + 3)
-    int rows_per_cta;
-    OutSpec ospec;        // output dtype / nodata of the corrected plane (APPLY); plain float32 otherwise
-};
-
-// T: storage type of the source plane (APPLY); NB: coarse bands (1 or 2); APPLY: fuse gain*src+offset;
-// MC: coarse columns per lane (ncols <= 32 * MC).
-template <typename T, int NB, bool APPLY, bool ALIGNED, int MC>
-__global__ void __launch_bounds__(kThreads, HB_UP_MIN_CTAS)
-upsample_kernel(const T *__restrict__ src, NoData nd, const float *__restrict__ coarse, UpGeom g,
-                const uint8_t *__restrict__ cover, float *__restrict__ out)
-{
-    constexpr int PPT = kUpPpt;
-    constexpr int NOUT = (NB == 2 && !APPLY) ? 2 : 1;
-    constexpr int kLaneBytes = APPLY ? Src4<T>::kBytes : 0;
-    constexpr int kRowBytes = 32 * kLaneBytes;                            // one staged source row of the warp
-    constexpr int kRingBytes = kUpStages * kUpRb * kRowBytes;
-    constexpr unsigned kFullMask = (NB == 2) ? 0xFFu : 0x0Fu;
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int ncols = g.ncols;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const float qnan = __int_as_float(0x7fc00000);
-
-    auto row_info = [&](long Y) {
-        const double srcy = g.sy * ((double)Y + 0.5) + g.oy;
-        const long ky = (long)floor(srcy - 0.5);
-        long cy = (long)floor(srcy + 1e-10);
-        if (cy == g.hp) cy--;
-        const bool cy_ok = (srcy >= 0.0) && cy >= 0 && cy < g.hp;
-        RowInfo ri;
-        ri.dy = srcy - 0.5 - (double)ky;
-        ri.ky = (int)ky;
-        ri.jc = cy_ok ? (int)(cy - (ky - 1)) : -1;          // 1 or 2 (0 when clamped at the bottom edge)
-        ri.cy = (int)cy;
-        ri.pad = 0;
-        return ri;
-    };
-
-    // ---- per-CTA row table: y-geometry of the CTA's destination rows ---------------------------------------------------
-    RowInfo *s_rows = reinterpret_cast<RowInfo *>(smem_raw);
-    const long Y0 = (long)blockIdx.y * g.rows_per_cta;
-    const long Y1 = min(Y0 + (long)g.rows_per_cta, g.hs);
-    const long strip = (long)blockIdx.x * kUpWarps + warp;
-    if ((long)threadIdx.x < Y1 - Y0) s_rows[threadIdx.x] = row_info(Y0 + threadIdx.x);
-    __syncthreads();                                        // the only CTA barrier
-
-    // warp-private shared memory: values [ncols], weights [ncols], column flags [ncols] of ONE row, source ring
-    const int comb_bytes = ((ncols * (2 * (int)sizeof(Pair) + 1)) + 15) / 16 * 16;
-    unsigned char *base = smem_raw + kUpMaxRows * sizeof(RowInfo) + warp * (comb_bytes + kRingBytes);
-    Pair *s_val = reinterpret_cast<Pair *>(base);
-    Pair *s_wgt = s_val + ncols;
-    uint8_t *s_colf = reinterpret_cast<uint8_t *>(s_wgt + ncols);          // bit0: a tap missing, bit1: centre usable
-    const unsigned char *s_ring = base + comb_bytes + lane * kLaneBytes;   // this lane's slot in a staged row
-    const uint32_t ring_sa = (uint32_t)__cvta_generic_to_shared(s_ring);
-
-    const long Xw0 = strip * kUpWarpW;                      // first destination column of the warp
-    if (Xw0 >= g.ws) return;
-    const long X0 = Xw0 + (long)lane * PPT;
-    const long plane = g.hp * g.wp;
-
-    // coarse column window of the warp: the taps of its first pixel start at column kx - 1
-    const double srcx_w0 = g.sx * ((double)Xw0 + 0.5) + g.ox;
-    const long col_base = (long)floor(srcx_w0 - 0.5) - 1;
-
-    // ---- per-pixel, row-invariant geometry (recomputed on demand: keeps it out of the hot loop's registers) ------------
-    auto px_geom = [&](int k, double &dxk, int &clk, int &ctk) {
-        const double srcx = g.sx * ((double)(X0 + k) + 0.5) + g.ox;
-        const long kx = (long)floor(srcx - 0.5);
-        dxk = srcx - 0.5 - (double)kx;                      // fractional column position inside the cell
-        long c = kx - 1 - col_base;                         // first tap column, relative to col_base
-        long cx = (long)floor(srcx + 1e-10);
-        if (cx == g.wp) cx--;
-        const bool okx = (srcx >= 0.0) && (cx >= 0) && (cx < g.wp);
-        int ct = -1;                                        // tap column hosting the centre (0..3), -1: none usable
-        if (c < 0 || c + 3 >= ncols) c = 0;                 // only for X >= ws (never stored)
-        else if (okx) ct = (int)(cx - (kx - 1));            // 1 or 2 (0 when clamped at the right edge)
-        clk = (int)c;
-        ctk = (ct >= 0 && ct < 4) ? ct : -1;
-    };
-    const bool full_vec = (X0 + PPT <= g.ws);
-    const bool use_async = APPLY && ALIGNED && full_vec;   // pixels come through the cp.async ring
-    double wxr[PPT][4];                                     // x-weights, first tap column, centre tap column per pixel
-    int clr[PPT], ctr[PPT];
-#pragma unroll
-    for (int k = 0; k < PPT; k++) {
-        double dxk;
-        px_geom(k, dxk, clr[k], ctr[k]);
-        bspline_weights(dxk, wxr[k]);
-    }
-
-    // ---- tap rows cached per lane column ---------------------------------------------------------------------------
-    float tv[MC][NB][4];
-    unsigned tmask[MC];
-#pragma unroll
-    for (int m = 0; m < MC; m++) tmask[m] = 0;
-    int a_ky = INT_MIN;
-
-    auto prefetch = [&](long Yp, int stage) {
-        if (use_async) {
-#pragma unroll
-            for (int rr = 0; rr < kUpRb; rr++)
-                if (Yp + rr < Y1)
-                    cp_async_lane<kLaneBytes>(ring_sa + (stage * kUpRb + rr) * kRowBytes, src + (Yp + rr) * g.ws + X0);
-        }
-        cp_async_commit();
-    };
-    if (APPLY) {
-#pragma unroll
-        for (int st = 0; st < kUpStages - 1; st++) prefetch(Y0 + (long)st * kUpRb, st);
-    }
-
-    // (APPLY: the corrected plane's output dtype conversion is fused into the store; `opix` = pixel index of the lane's
-    //  first pixel in the output plane)
-    auto store_row = [&](long opix, const float (&res)[NOUT][PPT]) {
-        if (ALIGNED && full_vec) {
-            if constexpr (APPLY) hb_store4_out(out, opix, make_float4(res[0][0], res[0][1], res[0][2], res[0][3]), g.ospec);
-            else hb_stg_stream16(out + opix, make_float4(res[0][0], res[0][1], res[0][2], res[0][3]));
-            if constexpr (NOUT == 2)
-                hb_stg_stream16(out + g.hs * g.ws + opix, make_float4(res[1][0], res[1][1], res[1][2], res[1][3]));
-        } else {
-#pragma unroll
-            for (int k = 0; k < PPT; k++) {
-                if ((X0 + k) < g.ws) {
-                    if constexpr (APPLY) hb_store1_out(out, opix + k, res[0][k], g.ospec);
-                    else out[opix + k] = res[0][k];
-                    if constexpr (NOUT == 2) out[g.hs * g.ws + opix + k] = res[1][k];
-                }
-            }
-        }
-    };
-    auto load_src = [&](long Y, const unsigned char *ring_row, float (&s)[PPT], bool (&ok)[PPT]) {
-        if constexpr (APPLY) {
-            if (use_async) {
-                Src4<T>::get(ring_row, nd, s, ok);
-            } else {
-                const T *row = src + Y * g.ws;
-#pragma unroll
-                for (int k = 0; k < PPT; k++) {
-                    const bool in_row = (X0 + k) < g.ws;
-                    s[k] = in_row ? hb_to_f32<T>(row[X0 + k]) : 0.f;
-                    ok[k] = in_row && hb_valid(s[k], nd);
-                }
-            }
-        } else {
-#pragma unroll
-            for (int k = 0; k < PPT; k++) { s[k] = 0.f; ok[k] = (X0 + k) < g.ws; }
-        }
-    };
-
-    int batch = 0;
-    for (long Yb = Y0; Yb < Y1; Yb += kUpRb, batch++) {
-        const int nrows = (int)min((long)kUpRb, Y1 - Yb);
-        if (APPLY) {
-            prefetch(Yb + (long)(kUpStages - 1) * kUpRb, (batch + kUpStages - 1) % kUpStages);
-            cp_async_wait<kUpStages - 1>();                 // this stage's source rows have landed
-        }
-        const unsigned char *ring_b = s_ring + ((batch % kUpStages) * kUpRb) * kRowBytes;
-
-        for (int rr = 0; rr < nrows; rr++) {
-            const long orow = (Yb + rr) * g.ws + X0;
-            const long Y = Yb + rr;
-            const RowInfo ri = s_rows[Y - Y0];
-
-            float s[PPT];
-            bool ok[PPT];
-            float res[NOUT][PPT];
-
-            // ---- GENERAL row, phase A: column combinations ------------------------------------------------------------
-            double wy[4];
-            bspline_weights(ri.dy, wy);
-            if (ri.ky != a_ky) {                            // (warp-uniform) fetch / shift the tap rows
-                const bool shift1 = (ri.ky - a_ky) == 1;
-#pragma unroll
-                for (int m = 0; m < MC; m++) {
-                    const long col = col_base + lane + 32 * m;
-                    const bool col_in = (lane + 32 * m < ncols) && col >= 0 && col < g.wp;
-                    unsigned mask = shift1 ? ((tmask[m] >> 1) & 0x77u) : 0u;
-#pragma unroll
-                    for (int j = 0; j < 4; j++) {
-                        const long row = (long)ri.ky - 1 + j;
-                        const bool inside = col_in && row >= 0 && row < g.hp;
-#pragma unroll
-                        for (int b = 0; b < NB; b++) {
-                            if (shift1 && j < 3) {
-                                tv[m][b][j] = tv[m][b][j + 1];
-                            } else {
-                                const float v = inside ? __ldg(coarse + b * plane + row * g.wp + col) : qnan;
-                                const bool okv = !isnan(v);
-                                tv[m][b][j] = okv ? v : 0.f;
-                                if (okv) mask |= 1u << (b * 4 + j);
-                            }
-                        }
-                    }
-                    tmask[m] = mask;
-                }
-                a_ky = ri.ky;
-            }
-#pragma unroll
-            for (int m = 0; m < MC; m++) {
-                const int c = lane + 32 * m;
-                if (c < ncols) {
-                    Pair val;                               // invalid taps are stored as 0: no predication needed
-                    val.g = fma(wy[3], (double)tv[m][0][3], fma(wy[2], (double)tv[m][0][2],
-                            fma(wy[1], (double)tv[m][0][1], wy[0] * (double)tv[m][0][0])));
-                    val.o = 0.0;
-                    if (NB > 1)
-                        val.o = fma(wy[3], (double)tv[m][1][3], fma(wy[2], (double)tv[m][1][2],
-                                fma(wy[1], (double)tv[m][1][1], wy[0] * (double)tv[m][1][0])));
-                    s_val[c] = val;
-                    const unsigned mask = tmask[m];
-                    const bool all_ok = (mask == kFullMask);
-                    // centre pixel: its coarse pixel must be in range and valid in any band (+ the coverage mask)
-                    bool c_ok = (ri.jc >= 0) && (((mask | (mask >> 4)) >> ri.jc) & 1u);
-                    if (c_ok && cover != nullptr) c_ok = cover[(long)ri.cy * g.wp + col_base + c] != 0;
-                    // a band's tap counts iff that band is valid there (band-valid implies "any band" validity)
-                    Pair wgt = {0.0, 0.0};
-#pragma unroll
-                    for (int j = 0; j < 4; j++) {
-                        if ((mask >> j) & 1u) wgt.g += wy[j];
-                        if (NB > 1 && ((mask >> (4 + j)) & 1u)) wgt.o += wy[j];
-                    }
-                    s_wgt[c] = wgt;
-                    s_colf[c] = (uint8_t)((all_ok ? 0 : 1) | (c_ok ? 2 : 0));
-                }
-            }
-            __syncwarp();
-
-            // ---- GENERAL row, phase C: destination pixels -------------------------------------------------------------
-            if (X0 < g.ws) {
-                load_src(Y, ring_b + rr * kRowBytes, s, ok);
-#pragma unroll
-                for (int k = 0; k < PPT; k++) {
-                    const double (&wx)[4] = wxr[k];
-                    const int clk = clr[k], ctk = ctr[k];
-                    const Pair *v = s_val + clk;
-                    const Pair a0 = v[0], a1 = v[1], a2 = v[2], a3 = v[3];
-                    double gv = fma(wx[3], a3.g, fma(wx[2], a2.g, fma(wx[1], a1.g, wx[0] * a0.g)));
-                    double ov = 0.0;
-                    if (NB > 1) ov = fma(wx[3], a3.o, fma(wx[2], a2.o, fma(wx[1], a1.o, wx[0] * a0.o)));
-                    const unsigned f0 = s_colf[clk], f1 = s_colf[clk + 1], f2 = s_colf[clk + 2], f3 = s_colf[clk + 3];
-                    const unsigned fc = (ctk == 0) ? f0 : (ctk == 1) ? f1 : (ctk == 2) ? f2 : (ctk == 3) ? f3 : 0u;
-                    bool g_ok = ok[k] && (fc & 2u), o_ok = g_ok;
-                    if ((f0 | f1 | f2 | f3) & 1u) {
-                        // GDAL GWKResample: drop if sum(w) < 1e-6, divide unless sum(w) is within 1e-5 of 1
-                        const Pair *w = s_wgt + clk;
-                        const Pair m0 = w[0], m1 = w[1], m2 = w[2], m3 = w[3];
-                        const double wg = fma(wx[3], m3.g, fma(wx[2], m2.g, fma(wx[1], m1.g, wx[0] * m0.g)));
-                        if (wg < 0.000001) g_ok = false;
-                        else if (wg < 0.99999 || wg > 1.00001) gv /= wg;
-                        if (NB > 1) {
-                            const double wo = fma(wx[3], m3.o, fma(wx[2], m2.o, fma(wx[1], m1.o, wx[0] * m0.o)));
-                            if (wo < 0.000001) o_ok = false;
-                            else if (wo < 0.99999 || wo > 1.00001) ov /= wo;
-                        }
-                    }
-                    const float gf = g_ok ? (float)gv : qnan;
-                    const float of = o_ok ? (float)ov : qnan;
-                    if (APPLY) {
-                        res[0][k] = __fadd_rn(__fmul_rn(gf, s[k]), of);
-                    } else {
-                        res[0][k] = gf;
-                        if constexpr (NOUT == 2) res[1][k] = of;
-                    }
-                }
-                store_row(orow, res);
-            }
-            __syncwarp();
-        }
-    }
-}
-
-template <typename T, int NB, bool APPLY>
-int launch_upsample(const void *src, NoData nd, const float *coarse, long hs, long ws, long hp, long wp, double sx,
-                    double ox, double sy, double oy, const uint8_t *cover, float *out, cudaStream_t stream,
-                    OutSpec ospec = hb_make_outspec(HB_F32, 0, 0.0))
-{
-    HB_REQUIRE(sx > 0 && sy > 0 && sx <= 1.0 + 1e-9 && sy <= 1.0 + 1e-9,
-               "cubic-spline up-sampling needs a destination grid at least as fine as the source (scale %.4f, %.4f)",
-               sx, sy);
-    HB_REQUIRE(hp < 2147483000L && wp < 2147483000L, "coarse raster too large");
-    UpGeom g;
-    g.hs = hs; g.ws = ws; g.hp = hp; g.wp = wp; g.sx = sx; g.ox = ox; g.sy = sy; g.oy = oy;
-    g.ospec = ospec;
-    g.ncols = (int)ceil((double)kUpWarpW * sx) + 5;
-    // rows per CTA: a couple of coarse rows' worth, so that the per-cell-row work is amortised
-    long rpc = (long)ceil(2.0 / sy);
-    rpc = ((rpc + kUpRb - 1) / kUpRb) * kUpRb;
-    if (rpc < 16) rpc = 16;
-    if (rpc > kUpMaxRows) rpc = kUpMaxRows;
-    g.rows_per_cta = (int)rpc;
-    const size_t ring = APPLY ? (size_t)kUpStages * kUpRb * 32 * kUpPpt * sizeof(T) : 0;
-    const size_t per_warp = ((size_t)g.ncols * (2 * sizeof(Pair) + 1) + 15) / 16 * 16 + ring;
-    const size_t smem = kUpMaxRows * sizeof(RowInfo) + per_warp * kUpWarps;
-    const long cta_w = (long)kUpWarpW * kUpWarps;
-    dim3 grid((unsigned)((ws + cta_w - 1) / cta_w), (unsigned)((hs + rpc - 1) / rpc));
-    HB_REQUIRE(grid.y <= 65535u, "up-sampling destination has too many rows (%ld)", hs);
-    const size_t align = APPLY ? sizeof(T) * kUpPpt : 16;
-    const bool aligned = (!APPLY || (((ws * (long)sizeof(T)) % (long)align == 0) && (((uintptr_t)src) % align == 0))) &&
-                         (ws % 4 == 0) && (((uintptr_t)out) % (4 * hb_out_size(ospec.dtype)) == 0);
-    NoData ndk = nd;
-    if (!ndk.int_ok) ndk.ivalue = -1;                       // integer sources: no pixel can equal it
-    // ---- fast paths (upsample_poly.cu): aligned rasters, >= ~1.6 destination pixels per coarse pixel, no coverage mask
-    if (aligned && cover == nullptr) {
-        UpPolyGeom pg;
-        pg.hs = hs; pg.ws = ws; pg.hp = hp; pg.wp = wp; pg.sx = sx; pg.ox = ox; pg.sy = sy; pg.oy = oy;
-        pg.ospec = ospec;
-        if (hb_up_poly_eligible(pg)) {
-            if (APPLY) return hb_up_poly_apply(src, hb_dtype_code<T>(), ndk, coarse, pg, out, stream);
-            if (NB == 1) return hb_up_poly_resample(coarse, 1, pg, out, stream);   // (double precision: feeds a fit)
-        }
-    }
-#define HB_UP_LAUNCH(AL_, MC_)                                                                                        \
-    do {                                                                                                              \
-        auto kern = upsample_kernel<T, NB, APPLY, AL_, MC_>;                                                          \
-        if (smem > 48 * 1024)                                                                                         \
-            HB_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));          \
-        kern<<<grid, kThreads, smem, stream>>>((const T *)src, ndk, coarse, g, cover, out);                          \
-    } while (0)
-    if (g.ncols <= 32) { if (aligned) HB_UP_LAUNCH(true, 1); else HB_UP_LAUNCH(false, 1); }
-    else if (g.ncols <= 96) { if (aligned) HB_UP_LAUNCH(true, 3); else HB_UP_LAUNCH(false, 3); }
-    else { if (aligned) HB_UP_LAUNCH(true, 5); else HB_UP_LAUNCH(false, 5); }
-#undef HB_UP_LAUNCH
-    HB_LAUNCH_OK("upsample_kernel");
-    return 0;
-}
-
-// nearest-neighbour up-sampling of float planes (kernel_model.py:497 semantics for float data)
-__global__ void nearest_kernel(const float *__restrict__ src, long nb, long hs, long ws, NoData nd,
-                               float *__restrict__ dst, long hd, long wd, double sx, double ox, double sy, double oy)
-{
-    const long n = hd * wd;
-    const float qnan = __int_as_float(0x7fc00000);
-    for (long idx = (long)blockIdx.x * blockDim.x + threadIdx.x; idx < n; idx += (long)gridDim.x * blockDim.x) {
-        const long i = idx / wd, j = idx - i * wd;
-        const double srcy = sy * ((double)i + 0.5) + oy, srcx = sx * ((double)j + 0.5) + ox;
-        long cy = (long)floor(srcy + 1e-10), cx = (long)floor(srcx + 1e-10);
-        if (cy == hs) cy--;
-        if (cx == ws) cx--;
-        const bool ok = srcy >= 0.0 && srcx >= 0.0 && cy >= 0 && cy < hs && cx >= 0 && cx < ws;
-        for (long b = 0; b < nb; b++) {
-            float v = qnan;
-            if (ok) {
-                const float s = src[b * hs * ws + cy * ws + cx];
-                if (hb_valid(s, nd)) v = s;
-            }
-            dst[b * n + idx] = v;
-        }
-    }
-}
-
-// =====================================================================================================================
-// 3. element-wise kernels
+// 2. element-wise kernels
 // =====================================================================================================================
 template <typename T>
 __global__ void apply_same_grid_kernel(const T *__restrict__ src, NoData nd, int mask_src,
@@ -1040,15 +588,6 @@ __global__ void erode_kernel(const uint8_t *__restrict__ in, long h, long w, int
     }
 }
 
-inline unsigned grid_for(long n, int threads, int per_sm = 8)
-{
-    long blocks = (n + threads - 1) / threads;
-    const long cap = (long)hb_sm_count() * per_sm;
-    if (blocks > cap) blocks = cap;
-    if (blocks < 1) blocks = 1;
-    return (unsigned)blocks;
-}
-
 }  // namespace
 
 // =====================================================================================================================
@@ -1070,57 +609,6 @@ extern "C" int hb_downsample_average(const void *src_dev, int src_dtype, long hs
     HB_REQUIRE(false, "hb_downsample_average: unknown dtype %d", src_dtype);
 }
 
-extern "C" int hb_upsample_apply(const void *src_dev, int src_dtype, long hs, long ws, int has_nodata, double nodata,
-                                 const float *params_dev, long hp, long wp, double sx, double ox, double sy, double oy,
-                                 const uint8_t *cover_dev, int out_dtype, int out_has_nodata, double out_nodata,
-                                 void *corr_dev, void *stream)
-{
-    HB_REQUIRE(src_dev && params_dev && corr_dev && hs > 0 && ws > 0 && hp > 0 && wp > 0,
-               "hb_upsample_apply: bad arguments");
-    HB_REQUIRE(hb_outspec_error(out_dtype, out_has_nodata, out_nodata) == nullptr, "hb_upsample_apply: %s",
-               hb_outspec_error(out_dtype, out_has_nodata, out_nodata));
-    const NoData nd = hb_make_nodata(has_nodata, nodata);
-    const OutSpec os = hb_make_outspec(out_dtype, out_has_nodata, out_nodata);
-    cudaStream_t st = (cudaStream_t)stream;
-    float *out = (float *)corr_dev;                          // (typed by `os`; the kernels index it in pixels)
-    switch (src_dtype) {
-        case HB_U8:
-            return launch_upsample<uint8_t, 2, true>(src_dev, nd, params_dev, hs, ws, hp, wp, sx, ox, sy, oy, cover_dev,
-                                                     out, st, os);
-        case HB_U16:
-            return launch_upsample<uint16_t, 2, true>(src_dev, nd, params_dev, hs, ws, hp, wp, sx, ox, sy, oy,
-                                                      cover_dev, out, st, os);
-        case HB_F32:
-            return launch_upsample<float, 2, true>(src_dev, nd, params_dev, hs, ws, hp, wp, sx, ox, sy, oy, cover_dev,
-                                                   out, st, os);
-    }
-    HB_REQUIRE(false, "hb_upsample_apply: unknown dtype %d", src_dtype);
-}
-
-extern "C" int hb_resample_up(const float *src_dev, long nb, long hs, long ws, int has_nodata, double nodata,
-                              float *dst_dev, long hd, long wd, double sx, double ox, double sy, double oy, int method,
-                              void *stream)
-{
-    HB_REQUIRE(src_dev && dst_dev && nb >= 1 && hs > 0 && ws > 0 && hd > 0 && wd > 0, "hb_resample_up: bad arguments");
-    cudaStream_t st = (cudaStream_t)stream;
-    const NoData nd = hb_make_nodata(has_nodata, nodata);
-    if (method == HB_UP_NEAREST) {
-        nearest_kernel<<<grid_for(hd * wd, 256), 256, 0, st>>>(src_dev, nb, hs, ws, nd, dst_dev, hd, wd, sx, ox, sy,
-                                                               oy);
-        HB_LAUNCH_OK("nearest_kernel");
-        return 0;
-    }
-    HB_REQUIRE(method == HB_UP_CUBIC_SPLINE, "hb_resample_up: unknown method %d", method);
-    HB_REQUIRE(has_nodata && isnan(nodata), "hb_resample_up: cubic-spline input must use NaN as nodata");
-    HB_REQUIRE(nb <= 2, "hb_resample_up: cubic-spline supports 1 or 2 bands per call (got %ld)", nb);
-    const NoData none = hb_make_nodata(0, 0.0);
-    if (nb == 1)
-        return launch_upsample<float, 1, false>(nullptr, none, src_dev, hd, wd, hs, ws, sx, ox, sy, oy, nullptr,
-                                                dst_dev, st);
-    return launch_upsample<float, 2, false>(nullptr, none, src_dev, hd, wd, hs, ws, sx, ox, sy, oy, nullptr, dst_dev,
-                                            st);
-}
-
 extern "C" int hb_apply_same_grid(const void *src_dev, int src_dtype, int has_nodata, double nodata, int mask_src,
                                   const float *params_dev, long h, long w, int out_dtype, int out_has_nodata,
                                   double out_nodata, void *corr_dev, void *stream)
@@ -1132,7 +620,7 @@ extern "C" int hb_apply_same_grid(const void *src_dev, int src_dtype, int has_no
     const OutSpec os = hb_make_outspec(out_dtype, out_has_nodata, out_nodata);
     cudaStream_t st = (cudaStream_t)stream;
     const long n = h * w;
-    const unsigned grid = grid_for(n, 256, 16);
+    const unsigned grid = hb_grid_for(n, 256, 16);
     switch (src_dtype) {
         case HB_U8:
             apply_same_grid_kernel<uint8_t><<<grid, 256, 0, st>>>((const uint8_t *)src_dev, nd, mask_src, params_dev, n,
@@ -1158,7 +646,7 @@ extern "C" int hb_convert_dtype(const float *src_dev, long n, int out_dtype, int
     HB_REQUIRE(src_dev && dst_dev && n > 0, "hb_convert_dtype: bad arguments");
     cudaStream_t st = (cudaStream_t)stream;
     const float nd = has_nodata ? (float)nodata : 0.f;
-    const unsigned grid = grid_for((n + 3) / 4, 256, 16);
+    const unsigned grid = hb_grid_for((n + 3) / 4, 256, 16);
     switch (out_dtype) {
         case HB_U8:
             HB_REQUIRE(!has_nodata || (nodata >= 0 && nodata <= 255 && nodata == floor(nodata)),
@@ -1191,7 +679,7 @@ extern "C" int hb_valid_mask(const void *src_dev, int src_dtype, long n, int has
     HB_REQUIRE(src_dev && mask_dev && n > 0, "hb_valid_mask: bad arguments");
     const NoData nd = hb_make_nodata(has_nodata, nodata);
     cudaStream_t st = (cudaStream_t)stream;
-    const unsigned grid = grid_for(n, 256, 16);
+    const unsigned grid = hb_grid_for(n, 256, 16);
     switch (src_dtype) {
         case HB_U8: valid_mask_kernel<uint8_t><<<grid, 256, 0, st>>>((const uint8_t *)src_dev, n, nd, mask_dev); break;
         case HB_U16:
@@ -1212,10 +700,10 @@ extern "C" int hb_full_coverage_mask(const uint8_t *in_mask_dev, long hi, long w
                "hb_full_coverage_mask: bad arguments");
     cudaStream_t st = (cudaStream_t)stream;
     uint8_t *covered = (uint8_t *)workspace_dev;
-    coverage_kernel<<<grid_for(hp * wp, 256), 256, 0, st>>>(in_mask_dev, hi, wi, params_dev, hp, wp, sx, ox, sy, oy,
-                                                            covered);
+    coverage_kernel<<<hb_grid_for(hp * wp, 256), 256, 0, st>>>(in_mask_dev, hi, wi, params_dev, hp, wp, sx, ox, sy, oy,
+                                                               covered);
     HB_LAUNCH_OK("coverage_kernel");
-    erode_kernel<<<grid_for(hp * wp, 256), 256, 0, st>>>(covered, hp, wp, kh + 2, kw + 2, out_dev);
+    erode_kernel<<<hb_grid_for(hp * wp, 256), 256, 0, st>>>(covered, hp, wp, kh + 2, kw + 2, out_dev);
     HB_LAUNCH_OK("erode_kernel");
     return 0;
 }

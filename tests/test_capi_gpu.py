@@ -294,7 +294,7 @@ def test_full_size_same_grid_properties():
     assert float(((a - b).abs()[fin] / a.abs()[fin].clamp_min(1e-3)).max()) <= RTOL
 
 
-# ---- the polynomial fast path of the up-sampler (csrc/upsample_poly.cu): destination >= ~3.4x finer, width % 4 == 0 ----
+# ---- the polynomial fast path of the up-sampler (csrc/upsample.cu): destination >= ~3.4x finer, width % 4 == 0 ---------
 _POLY_CASES = [
     # dtype, nodata, ratio, shift (source-grid pixels), extra destination pixels beyond the coarse raster, pattern
     ('uint16', 0, 20, (0, 0), 0, 'holes'),

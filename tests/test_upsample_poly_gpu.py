@@ -1,5 +1,5 @@
 """
-GPU tier: upsample_poly_kernel (csrc/upsample_poly.cu) on the geometries its row loop distinguishes -- rasters several
+GPU tier: upsample_poly_kernel (csrc/upsample.cu) on the geometries its row loop distinguishes -- rasters several
 CTAs wide with a partial last CTA, widths that are not a multiple of 8, CTAs whose row count is not a multiple of the
 rows handled per loop iteration, cell rows that start in the middle of an iteration, and the output conversion to
 uint8 / uint16 -- against RefSpaceModel.apply of the oracle.
