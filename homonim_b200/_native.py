@@ -17,8 +17,8 @@ from homonim_b200.errors import NativeLibraryError
 
 HB_U8, HB_U16, HB_F32, HB_I16 = 0, 1, 2, 3
 HB_MODEL_GAIN, HB_MODEL_GAIN_BLK_OFFSET, HB_MODEL_GAIN_OFFSET = 0, 1, 2
-HB_UP_CUBIC_SPLINE, HB_UP_NEAREST = 0, 1
-ABI_VERSION = 8
+HB_UP_CUBIC_SPLINE, HB_UP_NEAREST, HB_UP_BILINEAR, HB_UP_CUBIC, HB_UP_LANCZOS = 0, 1, 2, 3, 4
+ABI_VERSION = 9
 
 _PKG_DIR = pathlib.Path(__file__).resolve().parent
 LIB_PATH = _PKG_DIR / 'libhomonim_b200.so'
@@ -59,7 +59,8 @@ SIGNATURES = {
     'hb_apply_same_grid': (c_int, [c_void_p, c_int, c_int, c_double, c_int, c_void_p, c_long, c_long, c_int, c_int,
                                    c_double, c_void_p, c_void_p]),
     'hb_upsample_apply': (c_int, [c_void_p, c_int, c_long, c_long, c_int, c_double, c_void_p, c_long, c_long, c_double,
-                                  c_double, c_double, c_double, c_void_p, c_int, c_int, c_double, c_void_p, c_void_p]),
+                                  c_double, c_double, c_double, c_void_p, c_int, c_int, c_double, c_void_p, c_int,
+                                  c_void_p]),
     'hb_resample_up': (c_int, [c_void_p, c_long, c_long, c_long, c_int, c_double, c_void_p, c_long, c_long, c_double,
                                c_double, c_double, c_double, c_int, c_void_p]),
     'hb_full_coverage_mask': (c_int, [c_void_p, c_long, c_long, c_void_p, c_long, c_long, c_double, c_double, c_double,

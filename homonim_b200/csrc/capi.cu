@@ -100,7 +100,8 @@ static int fuse_refspace_direct(const void *src_dev, int src_dtype, long hs, lon
     }
     // source grid -> reference (param) grid is the inverse of the reference -> source map
     return hb_upsample_apply(src_dev, src_dtype, hs, ws, src_has_nodata, src_nodata, params, hr, wr, 1.0 / sx, -ox / sx,
-                             1.0 / sy, -oy / sy, nullptr, out_dtype, out_has_nodata, out_nodata, corr_dev, stream);
+                             1.0 / sy, -oy / sy, nullptr, out_dtype, out_has_nodata, out_nodata, corr_dev,
+                             HB_UP_CUBIC_SPLINE, stream);
 }
 
 // No CUDA-graph cache here: replaying a captured band step (8 kernels + stream-ordered allocations) saved 0.18 ms of host

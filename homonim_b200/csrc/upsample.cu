@@ -156,6 +156,51 @@ __device__ __forceinline__ void bspline_weights(double d, double (&w)[4])   // t
     w[3] = d2 * d * (1.0 / 6.0);
 }
 
+// ---- the other up-sampling methods of the general kernel (spec: oracle/interp_up_restate.c) ----------------------
+// Taps per axis: 6 for lanczos (k-2 .. k+3), 4 otherwise (k-1 .. k+2; bilinear uses the inner two).
+__host__ __device__ constexpr int up_taps(int method) { return method == HB_UP_LANCZOS ? 6 : 4; }
+
+// Weights of the up_taps(METHOD) taps at fractional position d in [0, 1): bilinear (0, 1-d, d, 0); cubic: Keys, a = -0.5;
+// lanczos: L(i - d), i = -2 .. 3, L(t) = sin(pi t) sin(pi t / 3) / (pi^2 t^2 / 3), L(0) = 1.
+template <int METHOD> __device__ __forceinline__ void up_weights(double d, double (&w)[up_taps(METHOD)])
+{
+    if constexpr (METHOD == HB_UP_BILINEAR) {
+        w[0] = 0.0; w[1] = 1.0 - d; w[2] = d; w[3] = 0.0;
+    } else if constexpr (METHOD == HB_UP_CUBIC) {
+        w[0] = 0.5 * d * (-1.0 + d * (2.0 - d));
+        w[1] = 1.0 + 0.5 * d * d * (-5.0 + 3.0 * d);
+        w[2] = 0.5 * d * (1.0 + d * (4.0 - 3.0 * d));
+        w[3] = 0.5 * d * d * (-1.0 + d);
+    } else {
+        // (sinpi: |t| < 4 needs no general argument reduction, and sin(pi t) of the six taps is +-sin(pi d))
+        const double pi = 3.14159265358979323846;
+        const double s = sinpi(d);
+#pragma unroll
+        for (int i = 0; i < 6; i++) {
+            const double t = (double)(i - 2) - d;
+            double l = 0.0;
+            if (t == 0.0) l = 1.0;
+            else if (fabs(t) < 3.0) l = ((i & 1) ? s : -s) * sinpi(t / 3.0) / (pi * pi * t * t / 3.0);
+            w[i] = l;
+        }
+    }
+}
+
+// GDAL's normalisation of a weighted sum `v` by its weight sum `w`; false: the pixel is nodata.  Bilinear / cubic's
+// bilinear fallback (GWKBilinearResample4Sample): nodata below 1e-5, divide unless exactly 1.  Lanczos (GWKResample):
+// nodata below 1e-6, divide unless within 1e-5 of 1.
+template <int METHOD> __device__ __forceinline__ bool up_normalise(double &v, double w)
+{
+    if constexpr (METHOD == HB_UP_LANCZOS) {
+        if (w < 0.000001) return false;
+        if (w < 0.99999 || w > 1.00001) v /= w;
+    } else {
+        if (w < 0.00001) return false;
+        if (w != 1.0) v /= w;
+    }
+    return true;
+}
+
 // B-spline weights of one destination index along one axis with GDAL's edge rules folded in: taps outside [0, n) get
 // weight 0 and the remaining weights are divided by their sum unless it is within 1e-5 of 1 (GWKResample's rule,
 // applied per axis -- GDAL applies it to the product of the two axis sums; the two differ by <= 2e-5 relative, and
@@ -1246,12 +1291,21 @@ struct UpGeom {
 };
 
 // T: storage type of the source plane (APPLY); NB: coarse bands (1 or 2); APPLY: fuse gain*src+offset;
-// MC: coarse columns per lane (ncols <= 32 * MC).
-template <typename T, int NB, bool APPLY, bool ALIGNED, int MC>
+// MC: coarse columns per lane (ncols <= 32 * MC); METHOD: HB_UP_CUBIC_SPLINE, HB_UP_BILINEAR, HB_UP_CUBIC or
+// HB_UP_LANCZOS.
+//   The other methods share the geometry, the centre / cover rules and the stores.  They differ in phase A: no tap-row
+//   register cache (the taps are re-read through L1 every row: nothing persists across rows, so even MC = 5 stays
+//   clear of spills with 6 taps), per-band "tap missing" flags (bit0 gain, bit2 offset), and for cubic a second
+//   column combination of the two inner taps with its own weight sum (its bilinear fallback, s_val2 / s_wgt).
+template <typename T, int NB, bool APPLY, bool ALIGNED, int MC, int METHOD>
 __global__ void __launch_bounds__(kThreads, kMinCtas)
 upsample_kernel(const T *__restrict__ src, NoData nd, const float *__restrict__ coarse, UpGeom g,
                 const uint8_t *__restrict__ cover, float *__restrict__ out)
 {
+    constexpr bool kSpline = (METHOD == HB_UP_CUBIC_SPLINE);
+    constexpr int NT = up_taps(METHOD);                                   // taps per axis
+    constexpr int kLo = NT / 2 - 1;                                       // taps before the cell's first row / column
+    constexpr int kPairs = (METHOD == HB_UP_CUBIC) ? 3 : 2;               // Pairs per staged column
     constexpr int NOUT = (NB == 2 && !APPLY) ? 2 : 1;
     constexpr int kLaneBytes = APPLY ? Src4<T>::kBytes : 0;
     constexpr int kRowBytes = 32 * kLaneBytes;                            // one staged source row of the warp
@@ -1271,7 +1325,7 @@ upsample_kernel(const T *__restrict__ src, NoData nd, const float *__restrict__ 
         RowInfo ri;
         ri.dy = srcy - 0.5 - (double)ky;
         ri.ky = (int)ky;
-        ri.jc = cy_ok ? (int)(cy - (ky - 1)) : -1;          // 1 or 2 (0 when clamped at the bottom edge)
+        ri.jc = cy_ok ? (int)(cy - (ky - kLo)) : -1;        // kLo or kLo + 1 (kLo - 1 when clamped at the bottom edge)
         ri.cy = (int)cy;
         ri.pad = 0;
         return ri;
@@ -1286,11 +1340,12 @@ upsample_kernel(const T *__restrict__ src, NoData nd, const float *__restrict__ 
     __syncthreads();                                        // the only CTA barrier
 
     // warp-private shared memory: values [ncols], weights [ncols], column flags [ncols] of ONE row, source ring
-    const int comb_bytes = ((ncols * (2 * (int)sizeof(Pair) + 1)) + 15) / 16 * 16;
+    const int comb_bytes = ((ncols * (kPairs * (int)sizeof(Pair) + 1)) + 15) / 16 * 16;
     unsigned char *base = smem_raw + kUpMaxRows * sizeof(RowInfo) + warp * (comb_bytes + kRingBytes);
     Pair *s_val = reinterpret_cast<Pair *>(base);
     Pair *s_wgt = s_val + ncols;
-    uint8_t *s_colf = reinterpret_cast<uint8_t *>(s_wgt + ncols);          // bit0: a tap missing, bit1: centre usable
+    Pair *s_val2 = s_wgt + ncols;                                          // (cubic only)
+    uint8_t *s_colf = reinterpret_cast<uint8_t *>(s_wgt + (kPairs - 1) * ncols);   // bit0: a tap missing, bit1: centre usable
     const unsigned char *s_ring = base + comb_bytes + lane * kLaneBytes;   // this lane's slot in a staged row
     const uint32_t ring_sa = (uint32_t)__cvta_generic_to_shared(s_ring);
 
@@ -1301,32 +1356,38 @@ upsample_kernel(const T *__restrict__ src, NoData nd, const float *__restrict__ 
 
     // coarse column window of the warp: the taps of its first pixel start at column kx - 1
     const double srcx_w0 = g.sx * ((double)Xw0 + 0.5) + g.ox;
-    const long col_base = (long)floor(srcx_w0 - 0.5) - 1;
+    const long col_base = (long)floor(srcx_w0 - 0.5) - kLo;
 
     // ---- per-pixel, row-invariant geometry (recomputed on demand: keeps it out of the hot loop's registers) ------------
     auto px_geom = [&](int k, double &dxk, int &clk, int &ctk) {
         const double srcx = g.sx * ((double)(X0 + k) + 0.5) + g.ox;
         const long kx = (long)floor(srcx - 0.5);
         dxk = srcx - 0.5 - (double)kx;                      // fractional column position inside the cell
-        long c = kx - 1 - col_base;                         // first tap column, relative to col_base
+        long c = kx - kLo - col_base;                       // first tap column, relative to col_base
         long cx = (long)floor(srcx + 1e-10);
         if (cx == g.wp) cx--;
         const bool okx = (srcx >= 0.0) && (cx >= 0) && (cx < g.wp);
-        int ct = -1;                                        // tap column hosting the centre (0..3), -1: none usable
-        if (c < 0 || c + 3 >= ncols) c = 0;                 // only for X >= ws (never stored)
-        else if (okx) ct = (int)(cx - (kx - 1));            // 1 or 2 (0 when clamped at the right edge)
+        int ct = -1;                                        // tap column hosting the centre (0..NT-1), -1: none usable
+        if (c < 0 || c + (NT - 1) >= ncols) c = 0;          // only for X >= ws (never stored)
+        else if (okx) ct = (int)(cx - (kx - kLo));          // kLo or kLo + 1 (kLo - 1 when clamped at the right edge)
         clk = (int)c;
-        ctk = (ct >= 0 && ct < 4) ? ct : -1;
+        ctk = (ct >= 0 && ct < NT) ? ct : -1;
     };
     const bool full_vec = (X0 + kPpt <= g.ws);
     const bool use_async = APPLY && ALIGNED && full_vec;   // pixels come through the cp.async ring
-    double wxr[kPpt][4];                                    // x-weights, first tap column, centre tap column per pixel
+    double wxr[kPpt][NT];                                   // x-weights, first tap column, centre tap column per pixel
+    double dxr[kPpt];                                       // (cubic: the bilinear fallback's fractional column)
     int clr[kPpt], ctr[kPpt];
 #pragma unroll
     for (int k = 0; k < kPpt; k++) {
         double dxk;
         px_geom(k, dxk, clr[k], ctr[k]);
-        bspline_weights(dxk, wxr[k]);
+        if constexpr (kSpline) {
+            bspline_weights(dxk, wxr[k]);
+        } else {
+            up_weights<METHOD>(dxk, wxr[k]);
+            dxr[k] = dxk;
+        }
     }
 
     // ---- tap rows cached per lane column ---------------------------------------------------------------------------
@@ -1407,6 +1468,7 @@ upsample_kernel(const T *__restrict__ src, NoData nd, const float *__restrict__ 
             float res[NOUT][kPpt];
 
             // ---- GENERAL row, phase A: column combinations ------------------------------------------------------------
+            if constexpr (kSpline) {
             double wy[4];
             bspline_weights(ri.dy, wy);
             if (ri.ky != a_ky) {                            // (warp-uniform) fetch / shift the tap rows
@@ -1464,6 +1526,61 @@ upsample_kernel(const T *__restrict__ src, NoData nd, const float *__restrict__ 
                     s_colf[c] = (uint8_t)((all_ok ? 0 : 1) | (c_ok ? 2 : 0));
                 }
             }
+            } else {
+            double wy[NT];
+            up_weights<METHOD>(ri.dy, wy);
+            const double by[2] = {1.0 - ri.dy, ri.dy};      // (cubic: the bilinear fallback's y-weights)
+#pragma unroll 1
+            for (int m = 0; m < MC; m++) {
+                const int c = lane + 32 * m;
+                if (c < ncols) {
+                    const long col = col_base + c;
+                    const bool col_in = col >= 0 && col < g.wp;
+                    double acc[NB], wsum[NB], acc2[NB], wsum2[NB];
+#pragma unroll
+                    for (int b = 0; b < NB; b++) acc[b] = wsum[b] = acc2[b] = wsum2[b] = 0.0;
+                    unsigned miss = 0;
+                    bool c_any = false;
+#pragma unroll
+                    for (int j = 0; j < NT; j++) {
+                        // bilinear weighs only the inner two rows; an outer row is read only when it hosts the centre
+                        const bool weighed = METHOD != HB_UP_BILINEAR || (j == 1 || j == 2);
+                        const long row = (long)ri.ky - kLo + j;
+                        const bool inside = (weighed || j == ri.jc) && col_in && row >= 0 && row < g.hp;
+                        bool any = false;
+#pragma unroll
+                        for (int b = 0; b < NB; b++) {
+                            const float v = inside ? __ldg(coarse + b * plane + row * g.wp + col) : qnan;
+                            const bool okv = !isnan(v);
+                            any |= okv;
+                            if (!weighed) continue;
+                            if (okv) {
+                                acc[b] = fma(wy[j], (double)v, acc[b]);
+                                wsum[b] += wy[j];
+                                if (METHOD == HB_UP_CUBIC && (j == 1 || j == 2)) {
+                                    acc2[b] = fma(by[j - 1], (double)v, acc2[b]);
+                                    wsum2[b] += by[j - 1];
+                                }
+                            } else {
+                                miss |= 1u << (2 * b);
+                            }
+                        }
+                        if (j == ri.jc) c_any = any;
+                    }
+                    // centre pixel: its coarse pixel must be in range and valid in any band (+ the coverage mask)
+                    bool c_ok = (ri.jc >= 0) && c_any;
+                    if (c_ok && cover != nullptr) c_ok = cover[(long)ri.cy * g.wp + col] != 0;
+                    s_val[c] = Pair{acc[0], NB > 1 ? acc[NB - 1] : 0.0};
+                    if constexpr (METHOD == HB_UP_CUBIC) {
+                        s_val2[c] = Pair{acc2[0], NB > 1 ? acc2[NB - 1] : 0.0};
+                        s_wgt[c] = Pair{wsum2[0], NB > 1 ? wsum2[NB - 1] : 0.0};
+                    } else {
+                        s_wgt[c] = Pair{wsum[0], NB > 1 ? wsum[NB - 1] : 0.0};
+                    }
+                    s_colf[c] = (uint8_t)(miss | (c_ok ? 2u : 0u));
+                }
+            }
+            }
             __syncwarp();
 
             // ---- GENERAL row, phase C: destination pixels -------------------------------------------------------------
@@ -1471,6 +1588,56 @@ upsample_kernel(const T *__restrict__ src, NoData nd, const float *__restrict__ 
                 load_src(Y, ring_b + rr * kRowBytes, s, ok);
 #pragma unroll
                 for (int k = 0; k < kPpt; k++) {
+                    if constexpr (!kSpline) {
+                    const double (&wx)[NT] = wxr[k];
+                    const int clk = clr[k], ctk = ctr[k];
+                    const Pair *v = s_val + clk;
+                    double gv = 0.0, ov = 0.0;
+                    unsigned fm = 0;                        // per-band "tap missing" over the footprint's columns
+#pragma unroll
+                    for (int i = 0; i < NT; i++) {
+                        if (METHOD == HB_UP_BILINEAR && (i == 0 || i == 3)) continue;
+                        const Pair a = v[i];
+                        gv = fma(wx[i], a.g, gv);
+                        if (NB > 1) ov = fma(wx[i], a.o, ov);
+                        fm |= s_colf[clk + i];
+                    }
+                    const unsigned fc = (ctk >= 0) ? s_colf[clk + ctk] : 0u;
+                    bool g_ok = ok[k] && (fc & 2u), o_ok = g_ok;
+                    const Pair *w = s_wgt + clk;
+                    if constexpr (METHOD == HB_UP_CUBIC) {
+                        // the 4x4 Keys sum where every tap of the band is valid and in range, else the bilinear result
+                        const double bx0 = 1.0 - dxr[k], bx1 = dxr[k];
+                        const Pair *v2 = s_val2 + clk;
+                        if (fm & 1u) {
+                            gv = fma(bx1, v2[2].g, bx0 * v2[1].g);
+                            g_ok = g_ok && up_normalise<METHOD>(gv, fma(bx1, w[2].g, bx0 * w[1].g));
+                        }
+                        if (NB > 1 && (fm & 4u)) {
+                            ov = fma(bx1, v2[2].o, bx0 * v2[1].o);
+                            o_ok = o_ok && up_normalise<METHOD>(ov, fma(bx1, w[2].o, bx0 * w[1].o));
+                        }
+                    } else if (METHOD == HB_UP_LANCZOS || (fm & 5u)) {
+                        // lanczos: its weights do not sum to 1, so every pixel is normalised
+                        double wg = 0.0, wo = 0.0;
+#pragma unroll
+                        for (int i = 0; i < NT; i++) {
+                            if (METHOD == HB_UP_BILINEAR && (i == 0 || i == 3)) continue;
+                            wg = fma(wx[i], w[i].g, wg);
+                            if (NB > 1) wo = fma(wx[i], w[i].o, wo);
+                        }
+                        g_ok = g_ok && up_normalise<METHOD>(gv, wg);
+                        if (NB > 1) o_ok = o_ok && up_normalise<METHOD>(ov, wo);
+                    }
+                    const float gf = g_ok ? (float)gv : qnan;
+                    const float of = o_ok ? (float)ov : qnan;
+                    if (APPLY) {
+                        res[0][k] = __fadd_rn(__fmul_rn(gf, s[k]), of);
+                    } else {
+                        res[0][k] = gf;
+                        if constexpr (NOUT == 2) res[1][k] = of;
+                    }
+                    } else {
                     const double (&wx)[4] = wxr[k];
                     const int clk = clr[k], ctk = ctr[k];
                     const Pair *v = s_val + clk;
@@ -1501,6 +1668,7 @@ upsample_kernel(const T *__restrict__ src, NoData nd, const float *__restrict__ 
                     } else {
                         res[0][k] = gf;
                         if constexpr (NOUT == 2) res[1][k] = of;
+                    }
                     }
                 }
                 store_row(orow, res);
@@ -1650,19 +1818,44 @@ int launch_yfirst_f64(const float *coarse, const UpPolyGeom &g, float *out, cuda
     return 0;
 }
 
+// the general kernel for one method: coarse columns per lane (MC) and alignment picked from the geometry
+template <typename T, int NB, bool APPLY, int METHOD>
+int launch_general(const void *src, NoData ndk, const float *coarse, const UpGeom &g, bool aligned, dim3 grid,
+                   size_t smem, const uint8_t *cover, float *out, cudaStream_t stream)
+{
+#define HB_UP_LAUNCH(AL_, MC_)                                                                                        \
+    do {                                                                                                              \
+        auto kern = upsample_kernel<T, NB, APPLY, AL_, MC_, METHOD>;                                                  \
+        if (smem > 48 * 1024)                                                                                         \
+            HB_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));          \
+        kern<<<grid, kThreads, smem, stream>>>((const T *)src, ndk, coarse, g, cover, out);                          \
+    } while (0)
+    if constexpr (METHOD == HB_UP_CUBIC_SPLINE) {
+        if (g.ncols <= 32) { if (aligned) HB_UP_LAUNCH(true, 1); else HB_UP_LAUNCH(false, 1); }
+        else if (g.ncols <= 96) { if (aligned) HB_UP_LAUNCH(true, 3); else HB_UP_LAUNCH(false, 3); }
+        else { if (aligned) HB_UP_LAUNCH(true, 5); else HB_UP_LAUNCH(false, 5); }
+    } else {
+        // (the other methods walk their staged columns in a loop that is not unrolled: MC only bounds it)
+        if (aligned) HB_UP_LAUNCH(true, 5); else HB_UP_LAUNCH(false, 5);
+    }
+#undef HB_UP_LAUNCH
+    HB_LAUNCH_OK("upsample_kernel");
+    return 0;
+}
+
 template <typename T, int NB, bool APPLY>
 int launch_upsample(const void *src, NoData nd, const float *coarse, long hs, long ws, long hp, long wp, double sx,
                     double ox, double sy, double oy, const uint8_t *cover, float *out, cudaStream_t stream,
-                    OutSpec ospec = hb_make_outspec(HB_F32, 0, 0.0))
+                    OutSpec ospec, int method)
 {
     HB_REQUIRE(sx > 0 && sy > 0 && sx <= 1.0 + 1e-9 && sy <= 1.0 + 1e-9,
-               "cubic-spline up-sampling needs a destination grid at least as fine as the source (scale %.4f, %.4f)",
-               sx, sy);
+               "up-sampling needs a destination grid at least as fine as the source (scale %.4f, %.4f)", sx, sy);
     HB_REQUIRE(hp < 2147483000L && wp < 2147483000L, "coarse raster too large");
     UpGeom g;
     g.hs = hs; g.ws = ws; g.hp = hp; g.wp = wp; g.sx = sx; g.ox = ox; g.sy = sy; g.oy = oy;
     g.ospec = ospec;
-    g.ncols = (int)ceil((double)kWarpW * sx) + 5;
+    // coarse columns under a warp's 128 destination columns: the cells they span + the taps' reach on either side
+    g.ncols = (int)ceil((double)kWarpW * sx) + up_taps(method) + 1;
     // rows per CTA: a couple of coarse rows' worth, so that the per-cell-row work is amortised
     long rpc = (long)ceil(2.0 / sy);
     rpc = ((rpc + kRb - 1) / kRb) * kRb;
@@ -1670,7 +1863,8 @@ int launch_upsample(const void *src, NoData nd, const float *coarse, long hs, lo
     if (rpc > kUpMaxRows) rpc = kUpMaxRows;
     g.rows_per_cta = (int)rpc;
     const size_t ring = APPLY ? (size_t)kStages * kRb * 32 * kPpt * sizeof(T) : 0;
-    const size_t per_warp = ((size_t)g.ncols * (2 * sizeof(Pair) + 1) + 15) / 16 * 16 + ring;
+    const size_t pairs = (method == HB_UP_CUBIC) ? 3 : 2;    // (must match the kernel's kPairs)
+    const size_t per_warp = ((size_t)g.ncols * (pairs * sizeof(Pair) + 1) + 15) / 16 * 16 + ring;
     const size_t smem = kUpMaxRows * sizeof(RowInfo) + per_warp * kWarps;
     const long cta_w = (long)kWarpW * kWarps;
     dim3 grid((unsigned)((ws + cta_w - 1) / cta_w), (unsigned)((hs + rpc - 1) / rpc));
@@ -1680,27 +1874,31 @@ int launch_upsample(const void *src, NoData nd, const float *coarse, long hs, lo
                          (ws % 4 == 0) && (((uintptr_t)out) % (4 * hb_out_size(ospec.dtype)) == 0);
     NoData ndk = nd;
     if (!ndk.int_ok) ndk.ivalue = -1;                       // integer sources: no pixel can equal it
-    // ---- fast paths: aligned rasters, no coverage mask, >= ~1.6 destination pixels per coarse pixel (a lane's 4 pixels
-    //      must span at most 3 coarse cells: 3 * sx < 2, with margin; the row direction only needs sy <= 1)
-    if (aligned && cover == nullptr && sx <= 0.62 && sy <= 1.0 + 1e-9 && ws % kPpt == 0) {
+    // ---- cubic-spline fast paths: aligned rasters, no coverage mask, >= ~1.6 destination pixels per coarse pixel (a
+    //      lane's 4 pixels must span at most 3 coarse cells: 3 * sx < 2, with margin; the row direction only needs
+    //      sy <= 1).  The other methods always take the general kernel.
+    if (method == HB_UP_CUBIC_SPLINE && aligned && cover == nullptr && sx <= 0.62 && sy <= 1.0 + 1e-9 &&
+        ws % kPpt == 0) {
         const UpPolyGeom pg = {hs, ws, hp, wp, sx, ox, sy, oy, ospec};
         if constexpr (APPLY) return launch_poly<T>((const T *)src, ndk, coarse, pg, out, stream);
         // plain up-sampling: one band in double precision (it feeds a fit); two bands stay on the general kernel
         if constexpr (NB == 1) return launch_yfirst_f64(coarse, pg, out, stream);
     }
-#define HB_UP_LAUNCH(AL_, MC_)                                                                                        \
-    do {                                                                                                              \
-        auto kern = upsample_kernel<T, NB, APPLY, AL_, MC_>;                                                          \
-        if (smem > 48 * 1024)                                                                                         \
-            HB_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));          \
-        kern<<<grid, kThreads, smem, stream>>>((const T *)src, ndk, coarse, g, cover, out);                          \
-    } while (0)
-    if (g.ncols <= 32) { if (aligned) HB_UP_LAUNCH(true, 1); else HB_UP_LAUNCH(false, 1); }
-    else if (g.ncols <= 96) { if (aligned) HB_UP_LAUNCH(true, 3); else HB_UP_LAUNCH(false, 3); }
-    else { if (aligned) HB_UP_LAUNCH(true, 5); else HB_UP_LAUNCH(false, 5); }
-#undef HB_UP_LAUNCH
-    HB_LAUNCH_OK("upsample_kernel");
-    return 0;
+    switch (method) {
+        case HB_UP_CUBIC_SPLINE:
+            return launch_general<T, NB, APPLY, HB_UP_CUBIC_SPLINE>(src, ndk, coarse, g, aligned, grid, smem, cover, out,
+                                                                    stream);
+        case HB_UP_BILINEAR:
+            return launch_general<T, NB, APPLY, HB_UP_BILINEAR>(src, ndk, coarse, g, aligned, grid, smem, cover, out,
+                                                                stream);
+        case HB_UP_CUBIC:
+            return launch_general<T, NB, APPLY, HB_UP_CUBIC>(src, ndk, coarse, g, aligned, grid, smem, cover, out,
+                                                             stream);
+        case HB_UP_LANCZOS:
+            return launch_general<T, NB, APPLY, HB_UP_LANCZOS>(src, ndk, coarse, g, aligned, grid, smem, cover, out,
+                                                               stream);
+    }
+    HB_REQUIRE(false, "up-sampling: unknown method %d", method);
 }
 
 }  // namespace
@@ -1711,10 +1909,14 @@ int launch_upsample(const void *src, NoData nd, const float *coarse, long hs, lo
 extern "C" int hb_upsample_apply(const void *src_dev, int src_dtype, long hs, long ws, int has_nodata, double nodata,
                                  const float *params_dev, long hp, long wp, double sx, double ox, double sy, double oy,
                                  const uint8_t *cover_dev, int out_dtype, int out_has_nodata, double out_nodata,
-                                 void *corr_dev, void *stream)
+                                 void *corr_dev, int method, void *stream)
 {
     HB_REQUIRE(src_dev && params_dev && corr_dev && hs > 0 && ws > 0 && hp > 0 && wp > 0,
                "hb_upsample_apply: bad arguments");
+    HB_REQUIRE(method != HB_UP_NEAREST,
+               "hb_upsample_apply: nearest has no fused form (up-sample with hb_resample_up, then hb_apply_same_grid)");
+    HB_REQUIRE(method == HB_UP_CUBIC_SPLINE || method == HB_UP_BILINEAR || method == HB_UP_CUBIC ||
+               method == HB_UP_LANCZOS, "hb_upsample_apply: unknown method %d", method);
     HB_REQUIRE(hb_outspec_error(out_dtype, out_has_nodata, out_nodata) == nullptr, "hb_upsample_apply: %s",
                hb_outspec_error(out_dtype, out_has_nodata, out_nodata));
     const NoData nd = hb_make_nodata(has_nodata, nodata);
@@ -1724,13 +1926,13 @@ extern "C" int hb_upsample_apply(const void *src_dev, int src_dtype, long hs, lo
     switch (src_dtype) {
         case HB_U8:
             return launch_upsample<uint8_t, 2, true>(src_dev, nd, params_dev, hs, ws, hp, wp, sx, ox, sy, oy, cover_dev,
-                                                     out, st, os);
+                                                     out, st, os, method);
         case HB_U16:
             return launch_upsample<uint16_t, 2, true>(src_dev, nd, params_dev, hs, ws, hp, wp, sx, ox, sy, oy,
-                                                      cover_dev, out, st, os);
+                                                      cover_dev, out, st, os, method);
         case HB_F32:
             return launch_upsample<float, 2, true>(src_dev, nd, params_dev, hs, ws, hp, wp, sx, ox, sy, oy, cover_dev,
-                                                   out, st, os);
+                                                   out, st, os, method);
     }
     HB_REQUIRE(false, "hb_upsample_apply: unknown dtype %d", src_dtype);
 }
@@ -1748,13 +1950,17 @@ extern "C" int hb_resample_up(const float *src_dev, long nb, long hs, long ws, i
         HB_LAUNCH_OK("nearest_kernel");
         return 0;
     }
-    HB_REQUIRE(method == HB_UP_CUBIC_SPLINE, "hb_resample_up: unknown method %d", method);
-    HB_REQUIRE(has_nodata && isnan(nodata), "hb_resample_up: cubic-spline input must use NaN as nodata");
-    HB_REQUIRE(nb <= 2, "hb_resample_up: cubic-spline supports 1 or 2 bands per call (got %ld)", nb);
+    HB_REQUIRE(method == HB_UP_CUBIC_SPLINE || method == HB_UP_BILINEAR || method == HB_UP_CUBIC ||
+               method == HB_UP_LANCZOS, "hb_resample_up: unknown method %d", method);
+    HB_REQUIRE(has_nodata && isnan(nodata), "hb_resample_up: cubic-spline, bilinear, cubic and lanczos input must use "
+               "NaN as nodata");
+    HB_REQUIRE(nb <= 2, "hb_resample_up: cubic-spline, bilinear, cubic and lanczos support 1 or 2 bands per call "
+               "(got %ld)", nb);
     const NoData none = hb_make_nodata(0, 0.0);
+    const OutSpec f32 = hb_make_outspec(HB_F32, 0, 0.0);
     if (nb == 1)
         return launch_upsample<float, 1, false>(nullptr, none, src_dev, hd, wd, hs, ws, sx, ox, sy, oy, nullptr,
-                                                dst_dev, st);
+                                                dst_dev, st, f32, method);
     return launch_upsample<float, 2, false>(nullptr, none, src_dev, hd, wd, hs, ws, sx, ox, sy, oy, nullptr, dst_dev,
-                                            st);
+                                            st, f32, method);
 }

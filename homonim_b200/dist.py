@@ -11,9 +11,9 @@ pixels (utils.py:136-153).  Two regimes follow (SURVEY.md 8e):
   of source rows whose edges coincide with proc-grid (reference) pixel rows.  Two things cross the interconnect:
 
   - **halo rows** (`exchange_halos`, `exchange_halos_inplace`): ``kh // 2`` proc-grid rows from each neighbour for the
-    window sums (+ 2 for the cubic-spline taps when proc_crs = ref, + 100 with R2 in-painting: `halo_rows`), sent point
-    to point between row-band neighbours (NCCL P2P over NVLink on GPUs, gloo in the CPU tests).  Rows beyond the
-    raster stay absent, which is the reference's zero padding (cv BORDER_CONSTANT).  proc_crs = ref exchanges rows of
+    window sums (+ 2 for the up-sampler's taps when proc_crs = ref, 3 for lanczos; + 100 with R2 in-painting:
+    `halo_rows`), sent point to point between row-band neighbours (NCCL P2P over NVLink on GPUs, gloo in the CPU
+    tests).  Rows beyond the raster stay absent, which is the reference's zero padding (cv BORDER_CONSTANT).  proc_crs = ref exchanges rows of
     the DOWN-SAMPLED source (9 x 3000 float32 = 108 KB per neighbour and band for the 60k x 60k configuration); the
     same-grid path exchanges ``kh // 2`` rows of source and reference, received straight into the halo rows of
     pre-allocated planes (no copy of the band itself).
@@ -110,14 +110,21 @@ class RowBands(NamedTuple):
         return max(a - halo, 0), min(b + halo, self.starts[-1])
 
 
-def halo_rows(kernel_shape: Sequence[int], proc_crs_ref: bool, inpaint: bool) -> int:
+def up_reach(upsampling) -> int:
+    """ Parameter rows beyond a source row's cell that the up-sampler reads: 3 for lanczos' 6 taps, 2 for the 4-tap
+    methods (cubic_spline, cubic, bilinear) -- and for nearest, which needs fewer. """
+    from homonim_b200.enums import Resampling
+    return 3 if Resampling.coerce(upsampling) == Resampling.lanczos else 2
+
+
+def halo_rows(kernel_shape: Sequence[int], proc_crs_ref: bool, inpaint: bool, reach: int = 2) -> int:
     """
     Rows of proc-grid halo a row band needs on each side for its results to equal the whole-raster results:
     ``kh // 2`` for the window sums (the reference's block overlap uses the safe ``ceil(kh / 2)``, utils.py:136-153),
-    + 2 for the cubic-spline taps of the first / last up-sampled rows (proc_crs = ref), + 100 when in-painting is on
-    (fillnodata's search radius, kernel_model.py:366).
+    + ``reach`` for the up-sampler's taps of the first / last up-sampled rows (proc_crs = ref; 2 for the 4-tap methods,
+    3 for lanczos: `up_reach`), + 100 when in-painting is on (fillnodata's search radius, kernel_model.py:366).
     """
-    return int(kernel_shape[0]) // 2 + (2 if proc_crs_ref else 0) + (100 if inpaint else 0)
+    return int(kernel_shape[0]) // 2 + (int(reach) if proc_crs_ref else 0) + (100 if inpaint else 0)
 
 
 def _halo_peers(bands: RowBands, rank: int, halo: int) -> List[int]:
@@ -204,18 +211,19 @@ def source_band_for_proc_rows(src_ra_shape: Tuple[int, int], src_transform: Affi
     return r0, max(r1, r0)
 
 
-def fit_row_window(bands: RowBands, rank: int, halo: int) -> Tuple[int, int, int, int]:
+def fit_row_window(bands: RowBands, rank: int, halo: int, reach: int = 2) -> Tuple[int, int, int, int]:
     """
     Proc-grid rows of the sharded proc_crs = ref path for ``rank``: ``(lo, hi, plo, phi)``.  ``[lo, hi)`` are the rows the
     rank holds for the fit (its band extended by ``halo`` rows, clipped to the raster); ``[plo, phi)`` are the rows whose
-    parameters it needs for the up-sampler (its band plus the 2 rows of cubic-spline support on either side, clipped).
-    Every kept row is at least ``halo - 2`` rows away from a cut edge of the held window -- the distance over which
-    window sums (and the in-painting search) are affected by the cut -- unless that edge is the raster's own.
+    parameters it needs for the up-sampler (its band plus the ``reach`` rows of tap support on either side, clipped:
+    2 for the 4-tap methods, 3 for lanczos).  Every kept row is at least ``halo - reach`` rows away from a cut edge of
+    the held window -- the distance over which window sums (and the in-painting search) are affected by the cut --
+    unless that edge is the raster's own.
     """
     a, b = bands.band(rank)
     hp = bands.starts[-1]
     lo, hi = max(a - halo, 0), min(b + halo, hp)
-    plo, phi = max(a - 2, 0), min(b + 2, hp)
+    plo, phi = max(a - reach, 0), min(b + reach, hp)
     return lo, hi, plo, phi
 
 
@@ -419,8 +427,9 @@ def fuse_refspace_sharded_end(shard: _RefspaceShard, out=None, apply_stream=None
                                   n_total=ref_ra.height * ref_ra.width)
     # halo rows of the down-sampled plane, point to point
     inpaint = model.model == Model.gain_offset and model._r2_inpaint_thresh is not None
-    halo = halo_rows(model.kernel_shape, proc_crs_ref=True, inpaint=inpaint)
-    lo, hi, plo, phi = fit_row_window(bands, rank, halo)
+    reach = up_reach(model._upsampling)
+    halo = halo_rows(model.kernel_shape, proc_crs_ref=True, inpaint=inpaint, reach=reach)
+    lo, hi, plo, phi = fit_row_window(bands, rank, halo, reach)
     src_ds, _ = exchange_halos(src_ds_local, bands, halo, group)
     # fit the rows my source rows' spline taps touch, inside the held window
     params = model._fit_planes(src_ds, nan, ref_t[lo:hi], ref_ra.nodata, norm=norm, rows=(plo - lo, phi - plo))
@@ -447,7 +456,7 @@ def fuse_refspace_sharded(model, src_local: RasterArray, ref_ra: RasterArray, ba
     ``src_local`` holds this rank's source rows (its transform already points at its first row); ``ref_ra`` is the
     whole (replicated: it is 1 / ratio^2 of the source) reference band on the proc grid; ``bands`` partitions the
     proc-grid rows.  Returns ``(corr_local, param_ra)``: the corrected rows of this rank and the parameters of the
-    proc-grid rows they depend on (this rank's band plus the 2 rows of cubic-spline support on either side;
+    proc-grid rows they depend on (this rank's band plus the 2 rows of tap support on either side, 3 for lanczos;
     ``param_ra.transform`` points at them).  ``out`` (optional): float32 CUDA tensor to receive the corrected rows.
 
     Per rank: down-sample own rows (`fuse_refspace_sharded_begin`) -> block statistics over own proc rows, merged by

@@ -13,8 +13,12 @@ Differences from the reference, all deliberate:
     uint8 / uint16 sources may be passed in their stored dtype.
   * ``RefSpaceModel.apply`` never materialises the up-sampled parameters: up-sampling and gain*src+offset are one
     kernel.
-  * only the default resampling pair (average down / cubic_spline up) plus nearest are implemented natively; other
-    ``downsampling`` / ``upsampling`` choices raise NotImplementedError rather than silently using something else.
+  * down-sampling is ``average`` only; up-sampling is ``cubic_spline`` (the default), ``bilinear``, ``cubic``,
+    ``lanczos`` or ``nearest``, each as GDAL computes it when the destination is at least as fine as the source (spec:
+    oracle/gdal_restate.c, oracle/interp_up_restate.c).  Other ``downsampling`` / ``upsampling`` choices, and the
+    up-sampling methods on a down-sampling geometry, raise NotImplementedError rather than silently using something else.
+  * ``RefSpaceModel.apply`` fuses up-sampling and apply for every up-sampling method but ``nearest``; the one-call
+    ``RefSpaceModel.fuse`` (``can_fuse``) is the default resampling pair only.
 """
 import functools
 import warnings
@@ -445,13 +449,25 @@ def _downsample_average(src_t, src_transform, src_nodata, dst_shape, dst_transfo
     return dst
 
 
+# up-sampling methods with an sm_100a kernel, and their C-ABI codes
+_UP_METHODS = {
+    Resampling.cubic_spline: _native.HB_UP_CUBIC_SPLINE,
+    Resampling.bilinear: _native.HB_UP_BILINEAR,
+    Resampling.cubic: _native.HB_UP_CUBIC,
+    Resampling.lanczos: _native.HB_UP_LANCZOS,
+    Resampling.nearest: _native.HB_UP_NEAREST,
+}
+# the ones that up-sample with GDAL's tap rules (NaN nodata, 1 or 2 bands per native call) and have a fused apply
+_UP_INTERP = (Resampling.cubic_spline, Resampling.bilinear, Resampling.cubic, Resampling.lanczos)
+
+
 def _resample_up(src_t, src_transform, src_nodata, dst_shape, dst_transform, method=_native.HB_UP_CUBIC_SPLINE):
     """ float32 [nb, hd, wd] (NaN nodata) up-sampling of 1 or 2 float32 bands. """
     lib = _native.lib()
     gm = grid_map(src_transform, dst_transform)
     squeeze = src_t.ndim == 2
     src3 = src_t[None] if squeeze else src_t
-    if method == _native.HB_UP_CUBIC_SPLINE:
+    if method != _native.HB_UP_NEAREST:
         src3 = _as_nan_nodata_f32(src3, src_nodata).contiguous()
         has, nd = 1, NAN
     else:
@@ -471,12 +487,18 @@ def _resample_plane(t, transform, nodata, dst_shape, dst_transform, resampling: 
     """ Resample one plane to a float32, NaN-nodata plane on the destination grid. """
     if resampling == Resampling.average:
         return _downsample_average(t, transform, nodata, dst_shape, dst_transform)
-    if resampling == Resampling.cubic_spline:
-        return _resample_up(t, transform, nodata, dst_shape, dst_transform, _native.HB_UP_CUBIC_SPLINE)
-    if resampling == Resampling.nearest:
-        return _resample_up(t, transform, nodata, dst_shape, dst_transform, _native.HB_UP_NEAREST)
+    if resampling in _UP_METHODS:
+        if resampling in (Resampling.bilinear, Resampling.cubic, Resampling.lanczos):
+            gm = grid_map(transform, dst_transform)
+            if gm.sx > 1.0 + 1e-9 or gm.sy > 1.0 + 1e-9:
+                raise NotImplementedError(
+                    f'resampling {resampling.value!r} is only implemented for up-sampling (a destination grid at least '
+                    f'as fine as the source); down-sampling is implemented for average only'
+                )
+        return _resample_up(t, transform, nodata, dst_shape, dst_transform, _UP_METHODS[resampling])
     raise NotImplementedError(
-        f'resampling {resampling.value!r} has no sm_100a kernel yet (available: average, cubic_spline, nearest)'
+        f'resampling {resampling.value!r} has no sm_100a kernel yet (available: average for down-sampling; '
+        f'cubic_spline, bilinear, cubic, lanczos and nearest for up-sampling)'
     )
 
 
@@ -584,7 +606,7 @@ class RefSpaceModel(KernelModel):
         if self._mask_partial:
             src_mask = self._valid_mask_u8(src_t, src_ra.nodata)
             cover = self._full_coverage_mask(src_mask, src_ra.transform, par2, param_ra.transform)   # :495
-        if resampling == Resampling.cubic_spline:
+        if resampling in _UP_INTERP:
             # fused up-sample + apply (:491, :497-503): the up-sampled parameters never reach memory
             gm = grid_map(param_ra.transform, src_ra.transform)       # source grid -> param grid
             hp, wp = int(par2.shape[-2]), int(par2.shape[-1])
@@ -593,7 +615,8 @@ class RefSpaceModel(KernelModel):
             _call('hb_upsample_apply', src_t.data_ptr(), _plane_code(src_t), hs, ws, has, nd,
                                                 par2.data_ptr(), hp, wp, gm.sx, gm.ox, gm.sy, gm.oy,
                                                 cover.data_ptr() if cover is not None else None,
-                                                *_out_args(corr, out_nodata), corr.data_ptr(), _stream())
+                                                *_out_args(corr, out_nodata), corr.data_ptr(),
+                                                _UP_METHODS[resampling], _stream())
         else:
             # parameters finer than (or as fine as) the source: resample them, then the same-grid apply
             par_us = torch.stack([_resample_plane(par2[b], param_ra.transform, NAN, (hs, ws), src_ra.transform,

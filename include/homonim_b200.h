@@ -35,15 +35,16 @@
 extern "C" {
 #endif
 
-#define HB_ABI_VERSION 8
+#define HB_ABI_VERSION 9
 
 /* storage dtype of a source raster plane */
 enum { HB_U8 = 0, HB_U16 = 1, HB_F32 = 2, HB_I16 = 3 };   /* HB_I16: output dtypes only (out_dtype, hb_convert_dtype,
                                                              hb_build_overviews) */
 /* homonim.enums.Model (homonim/enums.py:22-42) */
 enum { HB_MODEL_GAIN = 0, HB_MODEL_GAIN_BLK_OFFSET = 1, HB_MODEL_GAIN_OFFSET = 2 };
-/* up-sampling methods of hb_resample_up */
-enum { HB_UP_CUBIC_SPLINE = 0, HB_UP_NEAREST = 1 };
+/* up-sampling methods of hb_resample_up and hb_upsample_apply (GDAL GRA_CubicSpline, GRA_NearestNeighbour,
+ * GRA_Bilinear, GRA_Cubic, GRA_Lanczos; spec: oracle/gdal_restate.c, oracle/interp_up_restate.c) */
+enum { HB_UP_CUBIC_SPLINE = 0, HB_UP_NEAREST = 1, HB_UP_BILINEAR = 2, HB_UP_CUBIC = 3, HB_UP_LANCZOS = 4 };
 
 int hb_abi_version(void);
 const char *hb_last_error(void);
@@ -163,18 +164,23 @@ int hb_apply_same_grid(const void *src_dev, int src_dtype, int has_nodata, doubl
  *   cover_dev  optional uint8 [hp][wp] full-coverage mask (mask_partial=True, kernel_model.py:493-498), looked up
  *              with nearest resampling; NULL = mask with the source nodata mask (kernel_model.py:500).
  *   corr       [hs][ws] of the output dtype = up(gain) * src + up(offset) (two float32 roundings, as numpy), nodata where
- *              masked.  The up-sampled parameters are never written to memory.  Up-sampling is GDAL GRA_CubicSpline (4x4 cubic B-spline taps, invalid taps
- *              skipped and the rest renormalised).
+ *              masked.  The up-sampled parameters are never written to memory.
+ *   method     HB_UP_CUBIC_SPLINE (GDAL GRA_CubicSpline: 4x4 cubic B-spline taps, invalid taps skipped and the rest
+ *              renormalised), HB_UP_BILINEAR, HB_UP_CUBIC or HB_UP_LANCZOS.  HB_UP_NEAREST is rejected: nearest
+ *              parameters are up-sampled with hb_resample_up and applied with hb_apply_same_grid.
  * --------------------------------------------------------------------------------------------------------------- */
 int hb_upsample_apply(const void *src_dev, int src_dtype, long hs, long ws, int has_nodata, double nodata,
                       const float *params_dev, long hp, long wp, double sx, double ox, double sy, double oy,
                       const uint8_t *cover_dev, int out_dtype, int out_has_nodata, double out_nodata, void *corr_dev,
-                      void *stream);
+                      int method, void *stream);
 
 /* ---------------------------------------------------------------------------------------------------------------
  * Plain up-sampling of nb float32 bands (NaN nodata in, NaN nodata out): RasterArray.reproject(...,
- * resampling=cubic_spline | nearest), used by SrcSpaceModel.fit (kernel_model.py:520) and RefSpaceModel.apply when
- * the up-sampled parameters themselves are wanted.  (sx, ox, sy, oy) maps destination to source coordinates.
+ * resampling=cubic_spline | nearest | bilinear | cubic | lanczos), used by SrcSpaceModel.fit (kernel_model.py:520)
+ * and RefSpaceModel.apply when the up-sampled parameters themselves are wanted.  (sx, ox, sy, oy) maps destination to
+ * source coordinates; the destination must be at least as fine as the source.  Every method but nearest needs NaN
+ * nodata and 1 or 2 bands per call (2 bands: a tap counts where its own band is valid, the centre pixel where any
+ * band is).
  * --------------------------------------------------------------------------------------------------------------- */
 int hb_resample_up(const float *src_dev, long nb, long hs, long ws, int has_nodata, double nodata, float *dst_dev,
                    long hd, long wd, double sx, double ox, double sy, double oy, int method, void *stream);
