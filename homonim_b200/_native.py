@@ -18,7 +18,8 @@ from homonim_b200.errors import NativeLibraryError
 HB_U8, HB_U16, HB_F32, HB_I16 = 0, 1, 2, 3
 HB_MODEL_GAIN, HB_MODEL_GAIN_BLK_OFFSET, HB_MODEL_GAIN_OFFSET = 0, 1, 2
 HB_UP_CUBIC_SPLINE, HB_UP_NEAREST, HB_UP_BILINEAR, HB_UP_CUBIC, HB_UP_LANCZOS = 0, 1, 2, 3, 4
-ABI_VERSION = 9
+HB_STAT_MIN, HB_STAT_MAX, HB_STAT_MED, HB_STAT_Q1, HB_STAT_Q3, HB_STAT_MODE = 0, 1, 2, 3, 4, 5
+ABI_VERSION = 10
 
 _PKG_DIR = pathlib.Path(__file__).resolve().parent
 LIB_PATH = _PKG_DIR / 'libhomonim_b200.so'
@@ -35,6 +36,8 @@ SIGNATURES = {
     'hb_reset_launch_count': (None, []),
     'hb_downsample_average': (c_int, [c_void_p, c_int, c_long, c_long, c_int, c_double, c_void_p, c_long, c_long,
                                       c_double, c_double, c_double, c_double, c_void_p]),
+    'hb_resample_stat': (c_int, [c_void_p, c_int, c_long, c_long, c_int, c_double, c_void_p, c_long, c_long, c_double,
+                                 c_double, c_double, c_double, c_int, c_void_p]),
     'hb_block_norm_workspace_bytes': (c_size_t, [c_long]),
     'hb_block_norm': (c_int, [c_void_p, c_int, c_double, c_void_p, c_int, c_double, c_long, c_void_p, c_void_p,
                               c_size_t, c_void_p]),

@@ -385,12 +385,21 @@ def fuse_refspace_sharded_begin(model, src_local: RasterArray, ref_ra: RasterArr
     and exchanges of the second stages (with a slab of a few thousand rows per rank those are host-paced, not GPU-paced).
     """
     from homonim_b200 import kernel_model as km
+    from homonim_b200.enums import Resampling
     rank = _rank(group)
     a, b = bands.band(rank)
     src_t = km._to_device(src_local.array)
     ref_t = km._as_f32_plane(km._to_device(ref_ra.array), ref_ra.nodata).contiguous()
     local_tf = ref_ra.transform * Affine.translation(0, a)
-    src_ds_local = km._downsample_average(src_t, src_local.transform, src_local.nodata, (b - a, ref_ra.width), local_tf)
+    # (a footprint statistic is exact here for the reason `average` is: every processing row's footprint lies inside
+    # the source rows `source_band_for_proc_rows` gives this rank)
+    stat = km._STAT_METHODS.get(Resampling.coerce(model._downsampling))
+    if stat is not None:
+        src_ds_local = km._resample_stat(src_t, src_local.transform, src_local.nodata, (b - a, ref_ra.width), local_tf,
+                                         stat)
+    else:
+        src_ds_local = km._downsample_average(src_t, src_local.transform, src_local.nodata, (b - a, ref_ra.width),
+                                              local_tf)
     ds_done = None
     if src_ds_local.is_cuda:
         ds_done = torch.cuda.Event()

@@ -40,6 +40,11 @@ class Resampling(str, Enum):
     lanczos = 'lanczos'
     average = 'average'
     mode = 'mode'
+    max = 'max'
+    min = 'min'
+    med = 'med'
+    q1 = 'q1'
+    q3 = 'q3'
 
     @classmethod
     def coerce(cls, value) -> 'Resampling':

@@ -13,10 +13,12 @@ Differences from the reference, all deliberate:
     uint8 / uint16 sources may be passed in their stored dtype.
   * ``RefSpaceModel.apply`` never materialises the up-sampled parameters: up-sampling and gain*src+offset are one
     kernel.
-  * down-sampling is ``average`` only; up-sampling is ``cubic_spline`` (the default), ``bilinear``, ``cubic``,
+  * down-sampling is ``average``; up-sampling is ``cubic_spline`` (the default), ``bilinear``, ``cubic``,
     ``lanczos`` or ``nearest``, each as GDAL computes it when the destination is at least as fine as the source (spec:
-    oracle/gdal_restate.c, oracle/interp_up_restate.c).  Other ``downsampling`` / ``upsampling`` choices, and the
-    up-sampling methods on a down-sampling geometry, raise NotImplementedError rather than silently using something else.
+    oracle/gdal_restate.c, oracle/interp_up_restate.c).  The footprint statistics ``min``, ``max``, ``med``, ``q1``,
+    ``q3`` and ``mode`` take any geometry and serve either key (spec: oracle/footprint_stats_restate.c).  Other
+    ``downsampling`` / ``upsampling`` choices, and the interpolating up-sampling methods on a down-sampling geometry,
+    raise NotImplementedError rather than silently using something else.
   * ``RefSpaceModel.apply`` fuses up-sampling and apply for every up-sampling method but ``nearest``; the one-call
     ``RefSpaceModel.fuse`` (``can_fuse``) is the default resampling pair only.
 """
@@ -449,6 +451,30 @@ def _downsample_average(src_t, src_transform, src_nodata, dst_shape, dst_transfo
     return dst
 
 
+# footprint statistics (any geometry) and their C-ABI codes
+_STAT_METHODS = {
+    Resampling.min: _native.HB_STAT_MIN,
+    Resampling.max: _native.HB_STAT_MAX,
+    Resampling.med: _native.HB_STAT_MED,
+    Resampling.q1: _native.HB_STAT_Q1,
+    Resampling.q3: _native.HB_STAT_Q3,
+    Resampling.mode: _native.HB_STAT_MODE,
+}
+
+
+def _resample_stat(src_t, src_transform, src_nodata, dst_shape, dst_transform, method):
+    """ float32 [hd, wd] (NaN nodata) footprint statistic ``method`` (an ``HB_STAT_*`` code) of a uint8 / uint16 /
+    float32 plane. """
+    gm = grid_map(src_transform, dst_transform)
+    hs, ws = int(src_t.shape[-2]), int(src_t.shape[-1])
+    hd, wd = int(dst_shape[0]), int(dst_shape[1])
+    dst = torch.empty((hd, wd), dtype=torch.float32, device=src_t.device)
+    has, nd = _nodata_args(src_nodata)
+    _call('hb_resample_stat', src_t.data_ptr(), _plane_code(src_t), hs, ws, has, nd, dst.data_ptr(), hd, wd, gm.sx,
+          gm.ox, gm.sy, gm.oy, method, _stream())
+    return dst
+
+
 # up-sampling methods with an sm_100a kernel, and their C-ABI codes
 _UP_METHODS = {
     Resampling.cubic_spline: _native.HB_UP_CUBIC_SPLINE,
@@ -496,6 +522,8 @@ def _resample_plane(t, transform, nodata, dst_shape, dst_transform, resampling: 
                     f'as fine as the source); down-sampling is implemented for average only'
                 )
         return _resample_up(t, transform, nodata, dst_shape, dst_transform, _UP_METHODS[resampling])
+    if resampling in _STAT_METHODS:
+        return _resample_stat(t, transform, nodata, dst_shape, dst_transform, _STAT_METHODS[resampling])
     raise NotImplementedError(
         f'resampling {resampling.value!r} has no sm_100a kernel yet (available: average for down-sampling; '
         f'cubic_spline, bilinear, cubic, lanczos and nearest for up-sampling)'

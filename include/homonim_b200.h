@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define HB_ABI_VERSION 9
+#define HB_ABI_VERSION 10
 
 /* storage dtype of a source raster plane */
 enum { HB_U8 = 0, HB_U16 = 1, HB_F32 = 2, HB_I16 = 3 };   /* HB_I16: output dtypes only (out_dtype, hb_convert_dtype,
@@ -45,6 +45,9 @@ enum { HB_MODEL_GAIN = 0, HB_MODEL_GAIN_BLK_OFFSET = 1, HB_MODEL_GAIN_OFFSET = 2
 /* up-sampling methods of hb_resample_up and hb_upsample_apply (GDAL GRA_CubicSpline, GRA_NearestNeighbour,
  * GRA_Bilinear, GRA_Cubic, GRA_Lanczos; spec: oracle/gdal_restate.c, oracle/interp_up_restate.c) */
 enum { HB_UP_CUBIC_SPLINE = 0, HB_UP_NEAREST = 1, HB_UP_BILINEAR = 2, HB_UP_CUBIC = 3, HB_UP_LANCZOS = 4 };
+/* footprint statistics of hb_resample_stat (rasterio Resampling min, max, med, q1, q3, mode; spec:
+ * oracle/footprint_stats_restate.c) */
+enum { HB_STAT_MIN = 0, HB_STAT_MAX = 1, HB_STAT_MED = 2, HB_STAT_Q1 = 3, HB_STAT_Q3 = 4, HB_STAT_MODE = 5 };
 
 int hb_abi_version(void);
 const char *hb_last_error(void);
@@ -62,6 +65,21 @@ void hb_reset_launch_count(void);
 int hb_downsample_average(const void *src_dev, int src_dtype, long hs, long ws, int has_nodata, double nodata,
                           float *dst_dev, long hd, long wd, double sx, double ox, double sy, double oy,
                           void *stream);
+
+/* ---------------------------------------------------------------------------------------------------------------
+ * Footprint statistics: RasterArray.reproject(..., resampling=min | max | med | q1 | q3 | mode) on any geometry
+ * (down-sampling, up-sampling or mixed axes).  dst[hd][wd] float32, nodata = NaN.  Each destination pixel takes one of
+ * the valid source values under its footprint -- the window of hb_downsample_average, unweighted: a partly covered
+ * pixel counts as one value.  Valid = passes the nodata test and is not NaN; values compare as float32, -0.0 == +0.0,
+ * a zero result is +0.0.  With v[0..n) the n valid values sorted ascending: HB_STAT_MIN v[0], HB_STAT_MAX v[n-1],
+ * HB_STAT_MED / Q1 / Q3 v[ceil(q n - 1)] with q = 0.5 / 0.25 / 0.75 in double; HB_STAT_MODE the most frequent value,
+ * ties going to the value whose last occurrence comes first in row-major scan order.  NaN where no value is valid.
+ * Exact and deterministic.  At most 128 source pixels per destination pixel on each axis (sx, sy <= 128); beyond that
+ * the call fails.
+ * --------------------------------------------------------------------------------------------------------------- */
+int hb_resample_stat(const void *src_dev, int src_dtype, long hs, long ws, int has_nodata, double nodata,
+                     float *dst_dev, long hd, long wd, double sx, double ox, double sy, double oy, int method,
+                     void *stream);
 
 /* ---------------------------------------------------------------------------------------------------------------
  * Block normalisation statistics: KernelModel._fit_block_norm (kernel_model.py:216-229).
