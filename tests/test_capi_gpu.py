@@ -137,8 +137,9 @@ def test_block_norm():
     _, kmnp = _oracle()
     lib = _native.lib()
     rng = np.random.default_rng(5)
+    # 2**22: the largest block of the single cooperative launch; 2**22 + 1: the smallest of the multi-kernel path
     for n, nodata in ((1, NAN), (7, NAN), (9, NAN), (129, NAN), (1000, NAN), (4097, 0.0), (250_000, 0.0), (1_000_003, NAN),
-                      (9_000_000, NAN)):
+                      (2**22, NAN), (2**22 + 1, 0.0), (9_000_000, NAN)):
         src = rng.normal(3000, 900, n).astype('float32')
         ref = (0.7 * src + 100 + rng.normal(0, 30, n)).astype('float32')
         bad = rng.random(n) < 0.05
