@@ -62,17 +62,13 @@ template <> struct StatKey<float> {
     }
 };
 
-// Footprint of destination index i on one axis: downsample_average_kernel's window (unclamped bounds, a footprint inside
-// one source pixel takes that pixel, then clipped to [0, n)), capped at wmax pixels -- the most the geometry allows, so
-// the cap never binds; it only bounds the shared-memory writes.
+// Footprint of destination index i on one axis: GDAL's window (hb_footprint) clipped to [0, n), capped at wmax pixels --
+// the most the geometry allows, so the cap never binds; it only bounds the shared-memory writes.
 __device__ __forceinline__ void stat_axis(double s, double o, long i, long n, long wmax, long &a, long &b)
 {
-    const double lo = s * (double)i + o, hi = s * (double)(i + 1) + o;
-    const long a0 = (long)floor(lo + 1e-10);
-    long b0 = (long)ceil(hi - 1e-10);
-    if (a0 == b0) b0++;
-    a = max(a0, 0L);
-    b = min(min(b0, n), a + wmax);
+    const HbFootprint f = hb_footprint(s, o, i);
+    a = max(f.a0, 0L);
+    b = min(min(f.b0, n), a + wmax);
 }
 
 // 0-based rank of min / max / med / q1 / q3 among n >= 1 sorted values: v[ceil(q n - 1)], in double

@@ -73,6 +73,22 @@ __device__ __forceinline__ bool hb_valid(float v, const NoData &nd)
 // integer storage: compare as integers (exact; a uint8 / uint16 pixel can only equal an in-range integer nodata)
 __device__ __forceinline__ bool hb_valid_int(uint32_t v, const NoData &nd) { return !(nd.int_ok && (int)v == nd.ivalue); }
 
+// ---- GDAL's down-sampling footprint (GWKAverageOrModeThread) ------------------------------------------------------
+// Destination index i on one axis covers source coordinates [lo, hi) = [s i + o, s (i + 1) + o); its source window is
+// [a0, b0) = [floor(lo + 1e-10), ceil(hi - 1e-10)), and a footprint inside one source pixel takes that pixel.  The window
+// is NOT clamped to the raster: clamping, edge weights and what a window leaving the raster means are the caller's.
+struct HbFootprint { double lo, hi; long a0, b0; };
+__device__ __forceinline__ HbFootprint hb_footprint(double s, double o, long i)
+{
+    HbFootprint f;
+    f.lo = s * (double)i + o;
+    f.hi = s * (double)(i + 1) + o;
+    f.a0 = (long)floor(f.lo + 1e-10);
+    f.b0 = (long)ceil(f.hi - 1e-10);
+    if (f.a0 == f.b0) f.b0++;
+    return f;
+}
+
 // ---- storage dtype -> float32 (what the reference's reader does with out_dtype='float32') -------------------------
 template <typename T> __device__ __forceinline__ float hb_to_f32(T v) { return (float)v; }
 // exact small-integer -> float without the (slow) I2F pipe: 2^23 + v has v in its mantissa

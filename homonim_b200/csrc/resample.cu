@@ -105,24 +105,20 @@ downsample_average_kernel(const T *__restrict__ src, long hs, long ws, NoData nd
     // Footprint rows.  Weights follow GDAL's COMPUTE_WEIGHT_Y on the UNCLAMPED footprint and rows outside the raster
     // are skipped -- i.e. the result equals GDAL's on a source padded with nodata, which is how the reference reads
     // its source blocks (boundless windows, raster_array.py:175-199).
-    const double y_min = sy * (double)i + oy, y_max = sy * (double)(i + 1) + oy;
-    const long iy0u = (long)floor(y_min + 1e-10);
-    long iy1u = (long)ceil(y_max - 1e-10);
-    if (iy0u == iy1u) iy1u++;                                   // footprint inside one source row
+    const HbFootprint fy = hb_footprint(sy, oy, i);
+    const long iy0u = fy.a0, iy1u = fy.b0;
     const long iy0 = max(iy0u, 0L), iy1 = min(iy1u, hs);
     if (iy0 >= iy1) {
         for (long j = j0 + t; j < j1; j += kDsThreads) dst[i * wd + j] = qnan;
         return;
     }
-    const double wy_first = (iy0u + 1 == iy1u) ? 1.0 : 1.0 - (y_min - (double)iy0u);
-    const double wy_last = 1.0 - ((double)iy1u - y_max);
+    const double wy_first = (iy0u + 1 == iy1u) ? 1.0 : 1.0 - (fy.lo - (double)iy0u);
+    const double wy_last = 1.0 - ((double)iy1u - fy.hi);
     const bool first_frac = (iy0u >= 0) && (wy_first != 1.0);
     const bool last_frac = (iy1u <= hs) && (iy0u + 1 < iy1u) && (wy_last != 1.0);
     const long ya = iy0 + (first_frac ? 1 : 0), yb = iy1 - (last_frac ? 1 : 0);   // interior rows [ya, yb)
 
-    const double xs_min = sx * (double)j0 + ox;
-    long c_lo = (long)floor(xs_min + 1e-10);
-    if (c_lo < 0) c_lo = 0;
+    const long c_lo = max(hb_footprint(sx, ox, j0).a0, 0L);
     const long c_base = (c_lo / kDsVec) * kDsVec;
     const long c = c_base + (long)t * kDsVec;
 
@@ -292,10 +288,8 @@ downsample_average_kernel(const T *__restrict__ src, long hs, long ws, NoData nd
 
     // ---- phase 2: one thread per destination pixel ----------------------------------------------------------------
     for (long j = j0 + t; j < j1; j += kDsThreads) {
-        const double x_min = sx * (double)j + ox, x_max = sx * (double)(j + 1) + ox;
-        const long ix0u = (long)floor(x_min + 1e-10);
-        long ix1u = (long)ceil(x_max - 1e-10);
-        if (ix0u == ix1u) ix1u++;
+        const HbFootprint fx = hb_footprint(sx, ox, j);
+        const long ix0u = fx.a0, ix1u = fx.b0;
         const long ix0 = max(ix0u, 0L), ix1 = min(ix1u, ws);
         float out = qnan;
         double total = 0.0, total_w = 0.0;
@@ -305,8 +299,8 @@ downsample_average_kernel(const T *__restrict__ src, long hs, long ws, NoData nd
         long x = ix0 + ((ncol > 0) ? (long)(t % (int)ncol) : 0);
         for (long it = 0; it < ncol; it++) {
             double wx = 1.0;
-            if (x == ix0u) wx = (ix0u + 1 == ix1u) ? 1.0 : 1.0 - (x_min - (double)ix0u);
-            else if (x + 1 == ix1u) wx = 1.0 - ((double)ix1u - x_max);
+            if (x == ix0u) wx = (ix0u + 1 == ix1u) ? 1.0 : 1.0 - (fx.lo - (double)ix0u);
+            else if (x + 1 == ix1u) wx = 1.0 - ((double)ix1u - fx.hi);
             const int s = (int)(x - c_base);
             total += wx * s_sum[s];
             total_w += wx * s_w[s];
@@ -557,12 +551,8 @@ __global__ void coverage_kernel(const uint8_t *__restrict__ in_mask, long hi, lo
         const long i = idx / wp, j = idx - i * wp;
         bool ok = !(isnan(params[idx]) && isnan(params[n + idx]));
         if (ok) {
-            const double y_min = sy * (double)i + oy, y_max = sy * (double)(i + 1) + oy;
-            const double x_min = sx * (double)j + ox, x_max = sx * (double)(j + 1) + ox;
-            long iy0 = (long)floor(y_min + 1e-10), iy1 = (long)ceil(y_max - 1e-10);
-            long ix0 = (long)floor(x_min + 1e-10), ix1 = (long)ceil(x_max - 1e-10);
-            if (iy0 == iy1) iy1++;
-            if (ix0 == ix1) ix1++;
+            const HbFootprint fy = hb_footprint(sy, oy, i), fx = hb_footprint(sx, ox, j);
+            const long iy0 = fy.a0, iy1 = fy.b0, ix0 = fx.a0, ix1 = fx.b0;
             // a footprint that leaves the other image's raster is covered by nodata there (boundless read)
             if (iy0 < 0 || ix0 < 0 || iy1 > hi || ix1 > wi) ok = false;
             for (long y = iy0; ok && y < iy1; y++)

@@ -8,8 +8,12 @@
 //   upsample_poly_kernel        fused up-sample + apply, >= ~3.4 destination pixels per coarse pixel (packed float32)
 //   upsample_yfirst_kernel      fused up-sample + apply at smaller ratios (packed float32)
 //   upsample_yfirst_f64_kernel  plain one-band up-sampling in double (SrcSpaceModel's reference up-sampling)
-// Everything else -- small ratios, unaligned rasters, the coverage mask, plain two-band up-sampling -- runs on the
-// general upsample_kernel.
+// Everything else -- small ratios, unaligned rasters, the coverage mask, plain two-band up-sampling, and the bilinear,
+// cubic and lanczos methods -- runs on the general upsample_kernel.
+//
+// GDAL's rules are each written once and every kernel takes them from there: up_tap (a destination index's taps,
+// fractional position and centre pixel), up_weights<METHOD> (the taps' weights) and gwk_normalise (GWKResample's
+// weight-sum rule; up_normalise<METHOD> picks each method's rule).
 //
 // Replaces, for RefSpaceModel.apply (reference kernel_model.py:484-503): the GDAL GRA_CubicSpline warp of the gain and
 // offset planes onto the source grid, the two float32 planes it writes, and numpy's gain*src + offset pass (:461).
@@ -147,24 +151,40 @@ __device__ __forceinline__ long up_first_index(double scale, double off, long k,
     return i;
 }
 
-__device__ __forceinline__ void bspline_weights(double d, double (&w)[4])   // taps -1, 0, 1, 2: B(tap - d)
+// GDAL's tap / centre geometry of destination index i along one axis of a coarse grid of n pixels: source coordinate
+// c = s (i + 0.5) + o, first tap k - 1 with k = floor(c - 0.5), fractional position d = c - 0.5 - k in [0, 1); the
+// centre pixel is floor(c + 1e-10), moved back to n - 1 when it is n, and `ok` says it exists (c >= 0, centre in
+// [0, n)).  Every kernel takes its tap and centre indices from here, so that all of them agree on every pixel.
+struct UpTap { double c, d; long k, centre; bool ok; };
+__device__ __forceinline__ UpTap up_tap(double scale, double off, long i, long n)
 {
-    const double u = 1.0 - d, d2 = d * d, u2 = u * u;
-    w[0] = u2 * u * (1.0 / 6.0);
-    w[1] = (4.0 + d2 * (3.0 * d - 6.0)) * (1.0 / 6.0);
-    w[2] = (4.0 + u2 * (3.0 * u - 6.0)) * (1.0 / 6.0);
-    w[3] = d2 * d * (1.0 / 6.0);
+    UpTap t;
+    t.c = up_src_coord(scale, off, i);
+    const double kd = floor(t.c - 0.5);
+    t.k = (long)kd;
+    t.d = t.c - 0.5 - kd;
+    t.centre = (long)floor(t.c + 1e-10);
+    if (t.centre == n) t.centre--;
+    t.ok = (t.c >= 0.0) && t.centre >= 0 && t.centre < n;
+    return t;
 }
 
-// ---- the other up-sampling methods of the general kernel (spec: oracle/interp_up_restate.c) ----------------------
+// ---- the up-sampling methods (spec: oracle/gdal_restate.c, oracle/interp_up_restate.c) ----------------------------
 // Taps per axis: 6 for lanczos (k-2 .. k+3), 4 otherwise (k-1 .. k+2; bilinear uses the inner two).
 __host__ __device__ constexpr int up_taps(int method) { return method == HB_UP_LANCZOS ? 6 : 4; }
 
-// Weights of the up_taps(METHOD) taps at fractional position d in [0, 1): bilinear (0, 1-d, d, 0); cubic: Keys, a = -0.5;
-// lanczos: L(i - d), i = -2 .. 3, L(t) = sin(pi t) sin(pi t / 3) / (pi^2 t^2 / 3), L(0) = 1.
+// Weights of the up_taps(METHOD) taps at fractional position d in [0, 1): cubic spline: B(tap - d), the cubic B-spline;
+// bilinear (0, 1-d, d, 0); cubic: Keys, a = -0.5; lanczos: L(i - d), i = -2 .. 3,
+// L(t) = sin(pi t) sin(pi t / 3) / (pi^2 t^2 / 3), L(0) = 1.
 template <int METHOD> __device__ __forceinline__ void up_weights(double d, double (&w)[up_taps(METHOD)])
 {
-    if constexpr (METHOD == HB_UP_BILINEAR) {
+    if constexpr (METHOD == HB_UP_CUBIC_SPLINE) {
+        const double u = 1.0 - d, d2 = d * d, u2 = u * u;
+        w[0] = u2 * u * (1.0 / 6.0);
+        w[1] = (4.0 + d2 * (3.0 * d - 6.0)) * (1.0 / 6.0);
+        w[2] = (4.0 + u2 * (3.0 * u - 6.0)) * (1.0 / 6.0);
+        w[3] = d2 * d * (1.0 / 6.0);
+    } else if constexpr (METHOD == HB_UP_BILINEAR) {
         w[0] = 0.0; w[1] = 1.0 - d; w[2] = d; w[3] = 0.0;
     } else if constexpr (METHOD == HB_UP_CUBIC) {
         w[0] = 0.5 * d * (-1.0 + d * (2.0 - d));
@@ -186,70 +206,62 @@ template <int METHOD> __device__ __forceinline__ void up_weights(double d, doubl
     }
 }
 
-// GDAL's normalisation of a weighted sum `v` by its weight sum `w`; false: the pixel is nodata.  Bilinear / cubic's
-// bilinear fallback (GWKBilinearResample4Sample): nodata below 1e-5, divide unless exactly 1.  Lanczos (GWKResample):
-// nodata below 1e-6, divide unless within 1e-5 of 1.
-template <int METHOD> __device__ __forceinline__ bool up_normalise(double &v, double w)
+// GWKResample's normalisation of a weighted sum `v` by its weight sum `w` (cubic spline, lanczos): false, the pixel is
+// nodata, below 1e-6; divide unless within 1e-5 of 1.
+__device__ __forceinline__ bool gwk_normalise(double &v, double w)
 {
-    if constexpr (METHOD == HB_UP_LANCZOS) {
-        if (w < 0.000001) return false;
-        if (w < 0.99999 || w > 1.00001) v /= w;
-    } else {
-        if (w < 0.00001) return false;
-        if (w != 1.0) v /= w;
-    }
+    if (w < 0.000001) return false;
+    if (w < 0.99999 || w > 1.00001) v /= w;
     return true;
 }
 
-// B-spline weights of one destination index along one axis with GDAL's edge rules folded in: taps outside [0, n) get
-// weight 0 and the remaining weights are divided by their sum unless it is within 1e-5 of 1 (GWKResample's rule,
-// applied per axis -- GDAL applies it to the product of the two axis sums; the two differ by <= 2e-5 relative, and
-// only where taps are dropped on both axes); all weights are NaN when the pixel's centre coarse pixel is out of
-// range (GDAL skips such pixels).  `k` returns the first tap index + 1.
-__device__ __forceinline__ void up_axis_weights(double scale, double off, long i, long n, double (&w)[4], long &k)
+// GDAL's normalisation of a weighted sum `v` by its weight sum `w`; false: the pixel is nodata.  Bilinear / cubic's
+// bilinear fallback (GWKBilinearResample4Sample): nodata below 1e-5, divide unless exactly 1.  Cubic spline and
+// lanczos: GWKResample's rule.
+template <int METHOD> __device__ __forceinline__ bool up_normalise(double &v, double w)
 {
-    const double c = up_src_coord(scale, off, i);
-    const double kd = floor(c - 0.5);
-    k = (long)kd;
-    bspline_weights(c - 0.5 - kd, w);
-    long centre = (long)floor(c + 1e-10);
-    if (centre == n) centre--;
-    const bool ok = (c >= 0.0) && centre >= 0 && centre < n;
-    double sum = 0.0;
-#pragma unroll
-    for (int t = 0; t < 4; t++) {
-        const long tap = k - 1 + t;
-        if (tap < 0 || tap >= n) w[t] = 0.0;
-        sum += w[t];
-    }
-    if (!ok || sum < 0.99999 || sum > 1.00001) {            // (rare: only next to the raster's edges)
-        const double norm = ok ? 1.0 / sum : __longlong_as_double(0x7ff8000000000000LL);
-#pragma unroll
-        for (int t = 0; t < 4; t++) w[t] *= norm;
+    if constexpr (METHOD == HB_UP_CUBIC_SPLINE || METHOD == HB_UP_LANCZOS) {
+        return gwk_normalise(v, w);
+    } else {
+        if (w < 0.00001) return false;
+        if (w != 1.0) v /= w;
+        return true;
     }
 }
 
-// The same without the normalisation: raw B-spline weights with out-of-range taps zeroed, their sum, and whether the
-// pixel's centre coarse pixel is in range (for GDAL's exact rule on the PRODUCT of the two axis sums).
-__device__ __forceinline__ void up_axis_weights_raw(double scale, double off, long i, long n, double (&w)[4], long &k,
-                                                    double &sum, bool &ok)
+// B-spline weights of one destination index along one axis with out-of-range taps zeroed, their sum, and whether no
+// tap was dropped (for GDAL's exact rule on the PRODUCT of the two axis sums).  Returns the tap / centre geometry.
+__device__ __forceinline__ UpTap up_axis_weights_raw(double scale, double off, long i, long n, double (&w)[4], double &sum,
+                                                     bool &all_in)
 {
-    const double c = up_src_coord(scale, off, i);
-    const double kd = floor(c - 0.5);
-    k = (long)kd;
-    bspline_weights(c - 0.5 - kd, w);
-    long centre = (long)floor(c + 1e-10);
-    if (centre == n) centre--;
-    ok = (c >= 0.0) && centre >= 0 && centre < n;
+    const UpTap tp = up_tap(scale, off, i, n);
+    up_weights<HB_UP_CUBIC_SPLINE>(tp.d, w);
     sum = 0.0;
-    bool all_in = true;
+    all_in = true;
 #pragma unroll
     for (int t = 0; t < 4; t++) {
-        const long tap = k - 1 + t;
+        const long tap = tp.k - 1 + t;
         if (tap < 0 || tap >= n) { w[t] = 0.0; all_in = false; }
         sum += w[t];
     }
-    if (all_in) sum = 1.0;                                  // (the four weights sum to 1 up to rounding)
+    return tp;
+}
+
+// The same with GDAL's edge rules folded in: the remaining weights are divided by their sum unless it is within 1e-5 of
+// 1 (GWKResample's rule, applied per axis -- GDAL applies it to the product of the two axis sums; the two differ by
+// <= 2e-5 relative, and only where taps are dropped on both axes); all weights are NaN when the pixel's centre coarse
+// pixel is out of range (GDAL skips such pixels).  `k` returns the first tap index + 1.
+__device__ __forceinline__ void up_axis_weights(double scale, double off, long i, long n, double (&w)[4], long &k)
+{
+    double sum;
+    bool all_in;
+    const UpTap tp = up_axis_weights_raw(scale, off, i, n, w, sum, all_in);
+    k = tp.k;
+    if (!tp.ok || sum < 0.99999 || sum > 1.00001) {         // (rare: only next to the raster's edges)
+        const double norm = tp.ok ? 1.0 / sum : __longlong_as_double(0x7ff8000000000000LL);
+#pragma unroll
+        for (int t = 0; t < 4; t++) w[t] *= norm;
+    }
 }
 
 // ---- cp.async (LDGSTS) ---------------------------------------------------------------------------------------------
@@ -906,17 +918,14 @@ upsample_yfirst_f64_kernel(const float *__restrict__ coarse, UpPolyGeom g, int r
     int *s_ky = reinterpret_cast<int *>(smem_raw + kMaxRows * sizeof(RowEntryD));
     if ((int)threadIdx.x < nrows) {
         RowEntryD e;
-        long ky;
-        bool ok;
-        up_axis_weights_raw(g.sy, g.oy, Y0 + threadIdx.x, g.hp, e.wy, ky, e.sum, ok);
-        if (!ok) e.sum = dnan;
-        const double srcy = up_src_coord(g.sy, g.oy, Y0 + threadIdx.x);
-        long cy = (long)floor(srcy + 1e-10);
-        if (cy == g.hp) cy--;
-        const long jc = cy - (ky - 1);
-        e.jc = (ok && jc >= 0 && jc <= 3) ? (double)jc : -1.0;
+        bool all_in;
+        const UpTap ty = up_axis_weights_raw(g.sy, g.oy, Y0 + threadIdx.x, g.hp, e.wy, e.sum, all_in);
+        if (all_in) e.sum = 1.0;                            // (the four weights sum to 1 up to rounding)
+        if (!ty.ok) e.sum = dnan;
+        const long jc = ty.centre - (ty.k - 1);
+        e.jc = (ty.ok && jc >= 0 && jc <= 3) ? (double)jc : -1.0;
         s_rows[threadIdx.x] = e;
-        s_ky[threadIdx.x] = (int)min(max(ky, -4L), g.hp + 4);
+        s_ky[threadIdx.x] = (int)min(max(ty.k, -4L), g.hp + 4);
     }
     __syncthreads();
 
@@ -934,10 +943,11 @@ upsample_yfirst_f64_kernel(const float *__restrict__ coarse, UpPolyGeom g, int r
 #pragma unroll
         for (int k = 0; k < kPpt; k++) {
             double wx[4];
-            long kx;
-            bool ok;
-            up_axis_weights_raw(g.sx, g.ox, X0 + k, g.wp, wx, kx, xsum[k], ok);
-            if (!ok) xsum[k] = dnan;
+            bool all_in;
+            const UpTap tx = up_axis_weights_raw(g.sx, g.ox, X0 + k, g.wp, wx, xsum[k], all_in);
+            if (all_in) xsum[k] = 1.0;
+            if (!tx.ok) xsum[k] = dnan;
+            const long kx = tx.k;
             if (k == 0) kx0 = kx;
             kx3 = kx;
             const long sh = kx - kx0;                       // 0 .. 2 (>= 1.6 destination pixels per coarse pixel)
@@ -946,11 +956,8 @@ upsample_yfirst_f64_kernel(const float *__restrict__ coarse, UpPolyGeom g, int r
                 const long i = c - sh;
                 w6[k][c] = (i >= 0 && i < 4) ? wx[i < 0 ? 0 : (i > 3 ? 3 : i)] : 0.0;
             }
-            const double srcx = up_src_coord(g.sx, g.ox, X0 + k);
-            long cx = (long)floor(srcx + 1e-10);
-            if (cx == g.wp) cx--;
-            const long ci = cx - (kx0 - 1);
-            cc[k] = (ok && ci >= 0 && ci < kYfCols) ? (int)ci : -1;
+            const long ci = tx.centre - (kx0 - 1);
+            cc[k] = (tx.ok && ci >= 0 && ci < kYfCols) ? (int)ci : -1;
         }
         col0 = (int)min(max(kx0 - 1, -8L), g.wp + 8);
         ncell = (int)min(max(kx3 - kx0, 0L), 2L) + 1;
@@ -1040,11 +1047,7 @@ upsample_yfirst_f64_kernel(const float *__restrict__ coarse, UpPolyGeom g, int r
                     acc = fma(ri.wy[j], a, acc);
                     acc_w = fma(ri.wy[j], m, acc_w);
                 }
-                double res = dnan;
-                if (jc >= 0 && cc[k] >= 0 && centre == centre && !(acc_w < 0.000001)) {
-                    res = (acc_w < 0.99999 || acc_w > 1.00001) ? acc / acc_w : acc;
-                }
-                o[k] = res;
+                o[k] = (jc >= 0 && cc[k] >= 0 && centre == centre && gwk_normalise(acc, acc_w)) ? acc : dnan;
             }
         }
         hb_stg_stream16(orow, make_float4((float)o[0], (float)o[1], (float)o[2], (float)o[3]));
@@ -1104,28 +1107,25 @@ upsample_fixup_kernel(const T *__restrict__ src, NoData nd, const float *__restr
         // the rows' y-weights and centre rows are the same for every column: lane r prepares row ya + r once
         const bool cached = (yb - ya) <= 32;
         __syncwarp();
+        // (every row of the cell has k == ky: its d and centre row are relative to the cell's tap rows)
         if (cached && ya + lane < yb) {
-            const double srcy = up_src_coord(g.sy, g.oy, ya + lane);
-            long cy = (long)floor(srcy + 1e-10);
-            if (cy == g.hp) cy--;
-            const long jc = cy - (ky - 1);
+            const UpTap ty = up_tap(g.sy, g.oy, ya + lane, g.hp);
+            const long jc = ty.centre - (ky - 1);
             double wy[4];
-            bspline_weights(srcy - 0.5 - (double)ky, wy);
+            up_weights<HB_UP_CUBIC_SPLINE>(ty.d, wy);
 #pragma unroll
             for (int j = 0; j < 4; j++) s_wy[threadIdx.x >> 5][lane][j] = wy[j];
-            s_jc[threadIdx.x >> 5][lane] = (srcy >= 0.0 && jc >= 0 && jc <= 2) ? (int)jc : -1;
+            s_jc[threadIdx.x >> 5][lane] = (ty.ok && jc >= 0 && jc <= 2) ? (int)jc : -1;
         }
         __syncwarp();
         // every 4-pixel group (= lane of the fast kernel) that touches the cell was skipped there: do whole groups
         const long ga = (xa / kPpt) * kPpt, gb = min(((xb - 1) / kPpt + 1) * kPpt, g.ws);
         for (long X = ga + lane; X < gb; X += 32) {
-            const double srcx = up_src_coord(g.sx, g.ox, X);
-            long cx = (long)floor(srcx + 1e-10);
-            if (cx == g.wp) cx--;
-            const bool cx_ok = (srcx >= 0.0) && cx >= 0 && cx < g.wp;
-            const long kxx = (long)floor(srcx - 0.5);
+            const UpTap tx = up_tap(g.sx, g.ox, X, g.wp);
+            const long cx = tx.centre, kxx = tx.k;
+            const bool cx_ok = tx.ok;
             double wx[4];
-            bspline_weights(srcx - 0.5 - (double)kxx, wx);
+            up_weights<HB_UP_CUBIC_SPLINE>(tx.d, wx);
             // x-combination of the 4 tap rows ky-1 .. ky+2 (every row of the cell has the same tap rows)
             double A[2][4], M[2][4];                       // [band: gain, offset][tap row]
 #pragma unroll
@@ -1183,12 +1183,10 @@ upsample_fixup_kernel(const T *__restrict__ src, NoData nd, const float *__restr
 #pragma unroll
                         for (int j = 0; j < 4; j++) wy[j] = s_wy[threadIdx.x >> 5][ri][j];
                     } else {
-                        const double srcy = up_src_coord(g.sy, g.oy, Y);
-                        long cy = (long)floor(srcy + 1e-10);
-                        if (cy == g.hp) cy--;
-                        const long j0 = cy - (ky - 1);
-                        jc = (srcy >= 0.0 && j0 >= 0 && j0 <= 2) ? (int)j0 : -1;
-                        bspline_weights(srcy - 0.5 - (double)ky, wy);
+                        const UpTap ty = up_tap(g.sy, g.oy, Y, g.hp);
+                        const long j0 = ty.centre - (ky - 1);
+                        jc = (ty.ok && j0 >= 0 && j0 <= 2) ? (int)j0 : -1;
+                        up_weights<HB_UP_CUBIC_SPLINE>(ty.d, wy);
                     }
                     bool c_ok = (jc == 0 ? cen[0] : (jc == 1 ? cen[1] : (jc == 2 ? cen[2] : false)));
                     const float s = sv[u];
@@ -1203,9 +1201,7 @@ upsample_fixup_kernel(const T *__restrict__ src, NoData nd, const float *__restr
                                 acc = fma(wy[j], A[b][j], acc);
                                 acc_w = fma(wy[j], M[b][j], acc_w);
                             }
-                            if (acc_w < 0.000001) continue;
-                            if (acc_w < 0.99999 || acc_w > 1.00001) acc /= acc_w;
-                            r[b] = (float)acc;
+                            if (gwk_normalise(acc, acc_w)) r[b] = (float)acc;
                         }
                     }
                     hb_store1_out(out, Y * g.ws + X, __fadd_rn(__fmul_rn(r[0], s), r[1]), g.ospec);   // two roundings, as numpy
@@ -1293,10 +1289,11 @@ struct UpGeom {
 // T: storage type of the source plane (APPLY); NB: coarse bands (1 or 2); APPLY: fuse gain*src+offset;
 // MC: coarse columns per lane (ncols <= 32 * MC); METHOD: HB_UP_CUBIC_SPLINE, HB_UP_BILINEAR, HB_UP_CUBIC or
 // HB_UP_LANCZOS.
-//   The other methods share the geometry, the centre / cover rules and the stores.  They differ in phase A: no tap-row
-//   register cache (the taps are re-read through L1 every row: nothing persists across rows, so even MC = 5 stays
-//   clear of spills with 6 taps), per-band "tap missing" flags (bit0 gain, bit2 offset), and for cubic a second
-//   column combination of the two inner taps with its own weight sum (its bilinear fallback, s_val2 / s_wgt).
+//   All methods share the geometry, the centre / cover rules, phase C and the stores; every column stores per-band
+//   "tap missing" flags (bit0 gain, bit2 offset) and "centre usable" (bit1).  Phase A has two forms: cubic spline keeps
+//   its tap rows in a register cache (MC = 1 / 3 / 5); the other methods re-read the taps through L1 every row (nothing
+//   persists across rows, so even MC = 5 stays clear of spills with 6 taps), and cubic stores a second column
+//   combination of the two inner taps with its own weight sum (its bilinear fallback, s_val2 / s_wgt).
 template <typename T, int NB, bool APPLY, bool ALIGNED, int MC, int METHOD>
 __global__ void __launch_bounds__(kThreads, kMinCtas)
 upsample_kernel(const T *__restrict__ src, NoData nd, const float *__restrict__ coarse, UpGeom g,
@@ -1310,23 +1307,18 @@ upsample_kernel(const T *__restrict__ src, NoData nd, const float *__restrict__ 
     constexpr int kLaneBytes = APPLY ? Src4<T>::kBytes : 0;
     constexpr int kRowBytes = 32 * kLaneBytes;                            // one staged source row of the warp
     constexpr int kRingBytes = kStages * kRb * kRowBytes;
-    constexpr unsigned kFullMask = (NB == 2) ? 0xFFu : 0x0Fu;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int ncols = g.ncols;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const float qnan = __int_as_float(0x7fc00000);
 
     auto row_info = [&](long Y) {
-        const double srcy = g.sy * ((double)Y + 0.5) + g.oy;
-        const long ky = (long)floor(srcy - 0.5);
-        long cy = (long)floor(srcy + 1e-10);
-        if (cy == g.hp) cy--;
-        const bool cy_ok = (srcy >= 0.0) && cy >= 0 && cy < g.hp;
+        const UpTap ty = up_tap(g.sy, g.oy, Y, g.hp);
         RowInfo ri;
-        ri.dy = srcy - 0.5 - (double)ky;
-        ri.ky = (int)ky;
-        ri.jc = cy_ok ? (int)(cy - (ky - kLo)) : -1;        // kLo or kLo + 1 (kLo - 1 when clamped at the bottom edge)
-        ri.cy = (int)cy;
+        ri.dy = ty.d;
+        ri.ky = (int)ty.k;
+        ri.jc = ty.ok ? (int)(ty.centre - (ty.k - kLo)) : -1;   // kLo or kLo + 1 (kLo - 1 when clamped at the bottom edge)
+        ri.cy = (int)ty.centre;
         ri.pad = 0;
         return ri;
     };
@@ -1355,21 +1347,16 @@ upsample_kernel(const T *__restrict__ src, NoData nd, const float *__restrict__ 
     const long plane = g.hp * g.wp;
 
     // coarse column window of the warp: the taps of its first pixel start at column kx - 1
-    const double srcx_w0 = g.sx * ((double)Xw0 + 0.5) + g.ox;
-    const long col_base = (long)floor(srcx_w0 - 0.5) - kLo;
+    const long col_base = up_tap(g.sx, g.ox, Xw0, g.wp).k - kLo;
 
     // ---- per-pixel, row-invariant geometry (recomputed on demand: keeps it out of the hot loop's registers) ------------
     auto px_geom = [&](int k, double &dxk, int &clk, int &ctk) {
-        const double srcx = g.sx * ((double)(X0 + k) + 0.5) + g.ox;
-        const long kx = (long)floor(srcx - 0.5);
-        dxk = srcx - 0.5 - (double)kx;                      // fractional column position inside the cell
-        long c = kx - kLo - col_base;                       // first tap column, relative to col_base
-        long cx = (long)floor(srcx + 1e-10);
-        if (cx == g.wp) cx--;
-        const bool okx = (srcx >= 0.0) && (cx >= 0) && (cx < g.wp);
+        const UpTap tx = up_tap(g.sx, g.ox, X0 + k, g.wp);
+        dxk = tx.d;                                         // fractional column position inside the cell
+        long c = tx.k - kLo - col_base;                     // first tap column, relative to col_base
         int ct = -1;                                        // tap column hosting the centre (0..NT-1), -1: none usable
         if (c < 0 || c + (NT - 1) >= ncols) c = 0;          // only for X >= ws (never stored)
-        else if (okx) ct = (int)(cx - (kx - kLo));          // kLo or kLo + 1 (kLo - 1 when clamped at the right edge)
+        else if (tx.ok) ct = (int)(tx.centre - (tx.k - kLo));   // kLo or kLo + 1 (kLo - 1 when clamped at the right edge)
         clk = (int)c;
         ctk = (ct >= 0 && ct < NT) ? ct : -1;
     };
@@ -1380,14 +1367,8 @@ upsample_kernel(const T *__restrict__ src, NoData nd, const float *__restrict__ 
     int clr[kPpt], ctr[kPpt];
 #pragma unroll
     for (int k = 0; k < kPpt; k++) {
-        double dxk;
-        px_geom(k, dxk, clr[k], ctr[k]);
-        if constexpr (kSpline) {
-            bspline_weights(dxk, wxr[k]);
-        } else {
-            up_weights<METHOD>(dxk, wxr[k]);
-            dxr[k] = dxk;
-        }
+        px_geom(k, dxr[k], clr[k], ctr[k]);
+        up_weights<METHOD>(dxr[k], wxr[k]);
     }
 
     // ---- tap rows cached per lane column ---------------------------------------------------------------------------
@@ -1468,118 +1449,116 @@ upsample_kernel(const T *__restrict__ src, NoData nd, const float *__restrict__ 
             float res[NOUT][kPpt];
 
             // ---- GENERAL row, phase A: column combinations ------------------------------------------------------------
-            if constexpr (kSpline) {
-            double wy[4];
-            bspline_weights(ri.dy, wy);
-            if (ri.ky != a_ky) {                            // (warp-uniform) fetch / shift the tap rows
-                const bool shift1 = (ri.ky - a_ky) == 1;
-#pragma unroll
-                for (int m = 0; m < MC; m++) {
-                    const long col = col_base + lane + 32 * m;
-                    const bool col_in = (lane + 32 * m < ncols) && col >= 0 && col < g.wp;
-                    unsigned mask = shift1 ? ((tmask[m] >> 1) & 0x77u) : 0u;
-#pragma unroll
-                    for (int j = 0; j < 4; j++) {
-                        const long row = (long)ri.ky - 1 + j;
-                        const bool inside = col_in && row >= 0 && row < g.hp;
-#pragma unroll
-                        for (int b = 0; b < NB; b++) {
-                            if (shift1 && j < 3) {
-                                tv[m][b][j] = tv[m][b][j + 1];
-                            } else {
-                                const float v = inside ? __ldg(coarse + b * plane + row * g.wp + col) : qnan;
-                                const bool okv = !isnan(v);
-                                tv[m][b][j] = okv ? v : 0.f;
-                                if (okv) mask |= 1u << (b * 4 + j);
-                            }
-                        }
-                    }
-                    tmask[m] = mask;
-                }
-                a_ky = ri.ky;
-            }
-#pragma unroll
-            for (int m = 0; m < MC; m++) {
-                const int c = lane + 32 * m;
-                if (c < ncols) {
-                    Pair val;                               // invalid taps are stored as 0: no predication needed
-                    val.g = fma(wy[3], (double)tv[m][0][3], fma(wy[2], (double)tv[m][0][2],
-                            fma(wy[1], (double)tv[m][0][1], wy[0] * (double)tv[m][0][0])));
-                    val.o = 0.0;
-                    if (NB > 1)
-                        val.o = fma(wy[3], (double)tv[m][1][3], fma(wy[2], (double)tv[m][1][2],
-                                fma(wy[1], (double)tv[m][1][1], wy[0] * (double)tv[m][1][0])));
-                    s_val[c] = val;
-                    const unsigned mask = tmask[m];
-                    const bool all_ok = (mask == kFullMask);
-                    // centre pixel: its coarse pixel must be in range and valid in any band (+ the coverage mask)
-                    bool c_ok = (ri.jc >= 0) && (((mask | (mask >> 4)) >> ri.jc) & 1u);
-                    if (c_ok && cover != nullptr) c_ok = cover[(long)ri.cy * g.wp + col_base + c] != 0;
-                    // a band's tap counts iff that band is valid there (band-valid implies "any band" validity)
-                    Pair wgt = {0.0, 0.0};
-#pragma unroll
-                    for (int j = 0; j < 4; j++) {
-                        if ((mask >> j) & 1u) wgt.g += wy[j];
-                        if (NB > 1 && ((mask >> (4 + j)) & 1u)) wgt.o += wy[j];
-                    }
-                    s_wgt[c] = wgt;
-                    s_colf[c] = (uint8_t)((all_ok ? 0 : 1) | (c_ok ? 2 : 0));
-                }
-            }
-            } else {
             double wy[NT];
             up_weights<METHOD>(ri.dy, wy);
-            const double by[2] = {1.0 - ri.dy, ri.dy};      // (cubic: the bilinear fallback's y-weights)
-#pragma unroll 1
-            for (int m = 0; m < MC; m++) {
-                const int c = lane + 32 * m;
-                if (c < ncols) {
-                    const long col = col_base + c;
-                    const bool col_in = col >= 0 && col < g.wp;
-                    double acc[NB], wsum[NB], acc2[NB], wsum2[NB];
+            if constexpr (kSpline) {
+                if (ri.ky != a_ky) {                            // (warp-uniform) fetch / shift the tap rows
+                    const bool shift1 = (ri.ky - a_ky) == 1;
 #pragma unroll
-                    for (int b = 0; b < NB; b++) acc[b] = wsum[b] = acc2[b] = wsum2[b] = 0.0;
-                    unsigned miss = 0;
-                    bool c_any = false;
+                    for (int m = 0; m < MC; m++) {
+                        const long col = col_base + lane + 32 * m;
+                        const bool col_in = (lane + 32 * m < ncols) && col >= 0 && col < g.wp;
+                        unsigned mask = shift1 ? ((tmask[m] >> 1) & 0x77u) : 0u;
 #pragma unroll
-                    for (int j = 0; j < NT; j++) {
-                        // bilinear weighs only the inner two rows; an outer row is read only when it hosts the centre
-                        const bool weighed = METHOD != HB_UP_BILINEAR || (j == 1 || j == 2);
-                        const long row = (long)ri.ky - kLo + j;
-                        const bool inside = (weighed || j == ri.jc) && col_in && row >= 0 && row < g.hp;
-                        bool any = false;
+                        for (int j = 0; j < 4; j++) {
+                            const long row = (long)ri.ky - 1 + j;
+                            const bool inside = col_in && row >= 0 && row < g.hp;
 #pragma unroll
-                        for (int b = 0; b < NB; b++) {
-                            const float v = inside ? __ldg(coarse + b * plane + row * g.wp + col) : qnan;
-                            const bool okv = !isnan(v);
-                            any |= okv;
-                            if (!weighed) continue;
-                            if (okv) {
-                                acc[b] = fma(wy[j], (double)v, acc[b]);
-                                wsum[b] += wy[j];
-                                if (METHOD == HB_UP_CUBIC && (j == 1 || j == 2)) {
-                                    acc2[b] = fma(by[j - 1], (double)v, acc2[b]);
-                                    wsum2[b] += by[j - 1];
+                            for (int b = 0; b < NB; b++) {
+                                if (shift1 && j < 3) {
+                                    tv[m][b][j] = tv[m][b][j + 1];
+                                } else {
+                                    const float v = inside ? __ldg(coarse + b * plane + row * g.wp + col) : qnan;
+                                    const bool okv = !isnan(v);
+                                    tv[m][b][j] = okv ? v : 0.f;
+                                    if (okv) mask |= 1u << (b * 4 + j);
                                 }
-                            } else {
-                                miss |= 1u << (2 * b);
                             }
                         }
-                        if (j == ri.jc) c_any = any;
+                        tmask[m] = mask;
                     }
-                    // centre pixel: its coarse pixel must be in range and valid in any band (+ the coverage mask)
-                    bool c_ok = (ri.jc >= 0) && c_any;
-                    if (c_ok && cover != nullptr) c_ok = cover[(long)ri.cy * g.wp + col] != 0;
-                    s_val[c] = Pair{acc[0], NB > 1 ? acc[NB - 1] : 0.0};
-                    if constexpr (METHOD == HB_UP_CUBIC) {
-                        s_val2[c] = Pair{acc2[0], NB > 1 ? acc2[NB - 1] : 0.0};
-                        s_wgt[c] = Pair{wsum2[0], NB > 1 ? wsum2[NB - 1] : 0.0};
-                    } else {
-                        s_wgt[c] = Pair{wsum[0], NB > 1 ? wsum[NB - 1] : 0.0};
-                    }
-                    s_colf[c] = (uint8_t)(miss | (c_ok ? 2u : 0u));
+                    a_ky = ri.ky;
                 }
-            }
+#pragma unroll
+                for (int m = 0; m < MC; m++) {
+                    const int c = lane + 32 * m;
+                    if (c < ncols) {
+                        Pair val;                               // invalid taps are stored as 0: no predication needed
+                        val.g = fma(wy[3], (double)tv[m][0][3], fma(wy[2], (double)tv[m][0][2],
+                                fma(wy[1], (double)tv[m][0][1], wy[0] * (double)tv[m][0][0])));
+                        val.o = 0.0;
+                        if (NB > 1)
+                            val.o = fma(wy[3], (double)tv[m][1][3], fma(wy[2], (double)tv[m][1][2],
+                                    fma(wy[1], (double)tv[m][1][1], wy[0] * (double)tv[m][1][0])));
+                        s_val[c] = val;
+                        const unsigned mask = tmask[m];
+                        const unsigned miss = ((mask & 0xFu) != 0xFu ? 1u : 0u) | ((NB > 1 && (mask >> 4) != 0xFu) ? 4u : 0u);
+                        // centre pixel: its coarse pixel must be in range and valid in any band (+ the coverage mask)
+                        bool c_ok = (ri.jc >= 0) && (((mask | (mask >> 4)) >> ri.jc) & 1u);
+                        if (c_ok && cover != nullptr) c_ok = cover[(long)ri.cy * g.wp + col_base + c] != 0;
+                        // a band's tap counts iff that band is valid there (band-valid implies "any band" validity)
+                        Pair wgt = {0.0, 0.0};
+#pragma unroll
+                        for (int j = 0; j < 4; j++) {
+                            if ((mask >> j) & 1u) wgt.g += wy[j];
+                            if (NB > 1 && ((mask >> (4 + j)) & 1u)) wgt.o += wy[j];
+                        }
+                        s_wgt[c] = wgt;
+                        s_colf[c] = (uint8_t)(miss | (c_ok ? 2u : 0u));
+                    }
+                }
+            } else {
+                const double by[2] = {1.0 - ri.dy, ri.dy};      // (cubic: the bilinear fallback's y-weights)
+#pragma unroll 1
+                for (int m = 0; m < MC; m++) {
+                    const int c = lane + 32 * m;
+                    if (c < ncols) {
+                        const long col = col_base + c;
+                        const bool col_in = col >= 0 && col < g.wp;
+                        double acc[NB], wsum[NB], acc2[NB], wsum2[NB];
+#pragma unroll
+                        for (int b = 0; b < NB; b++) acc[b] = wsum[b] = acc2[b] = wsum2[b] = 0.0;
+                        unsigned miss = 0;
+                        bool c_any = false;
+#pragma unroll
+                        for (int j = 0; j < NT; j++) {
+                            // bilinear weighs only the inner two rows; an outer row is read only when it hosts the centre
+                            const bool weighed = METHOD != HB_UP_BILINEAR || (j == 1 || j == 2);
+                            const long row = (long)ri.ky - kLo + j;
+                            const bool inside = (weighed || j == ri.jc) && col_in && row >= 0 && row < g.hp;
+                            bool any = false;
+#pragma unroll
+                            for (int b = 0; b < NB; b++) {
+                                const float v = inside ? __ldg(coarse + b * plane + row * g.wp + col) : qnan;
+                                const bool okv = !isnan(v);
+                                any |= okv;
+                                if (!weighed) continue;
+                                if (okv) {
+                                    acc[b] = fma(wy[j], (double)v, acc[b]);
+                                    wsum[b] += wy[j];
+                                    if (METHOD == HB_UP_CUBIC && (j == 1 || j == 2)) {
+                                        acc2[b] = fma(by[j - 1], (double)v, acc2[b]);
+                                        wsum2[b] += by[j - 1];
+                                    }
+                                } else {
+                                    miss |= 1u << (2 * b);
+                                }
+                            }
+                            if (j == ri.jc) c_any = any;
+                        }
+                        // centre pixel: its coarse pixel must be in range and valid in any band (+ the coverage mask)
+                        bool c_ok = (ri.jc >= 0) && c_any;
+                        if (c_ok && cover != nullptr) c_ok = cover[(long)ri.cy * g.wp + col] != 0;
+                        s_val[c] = Pair{acc[0], NB > 1 ? acc[NB - 1] : 0.0};
+                        if constexpr (METHOD == HB_UP_CUBIC) {
+                            s_val2[c] = Pair{acc2[0], NB > 1 ? acc2[NB - 1] : 0.0};
+                            s_wgt[c] = Pair{wsum2[0], NB > 1 ? wsum2[NB - 1] : 0.0};
+                        } else {
+                            s_wgt[c] = Pair{wsum[0], NB > 1 ? wsum[NB - 1] : 0.0};
+                        }
+                        s_colf[c] = (uint8_t)(miss | (c_ok ? 2u : 0u));
+                    }
+                }
             }
             __syncwarp();
 
@@ -1588,11 +1567,12 @@ upsample_kernel(const T *__restrict__ src, NoData nd, const float *__restrict__ 
                 load_src(Y, ring_b + rr * kRowBytes, s, ok);
 #pragma unroll
                 for (int k = 0; k < kPpt; k++) {
-                    if constexpr (!kSpline) {
                     const double (&wx)[NT] = wxr[k];
                     const int clk = clr[k], ctk = ctr[k];
                     const Pair *v = s_val + clk;
-                    double gv = 0.0, ov = 0.0;
+                    // (cubic spline starts from -0.0, and fma(w, a, -0.0) == w * a: its sum starts with a product, as
+                    //  in its phase A and its fast paths, so that a sum of negative zeros stays -0.0 on every path)
+                    double gv = kSpline ? -0.0 : 0.0, ov = gv;
                     unsigned fm = 0;                        // per-band "tap missing" over the footprint's columns
 #pragma unroll
                     for (int i = 0; i < NT; i++) {
@@ -1637,39 +1617,6 @@ upsample_kernel(const T *__restrict__ src, NoData nd, const float *__restrict__ 
                         res[0][k] = gf;
                         if constexpr (NOUT == 2) res[1][k] = of;
                     }
-                    } else {
-                    const double (&wx)[4] = wxr[k];
-                    const int clk = clr[k], ctk = ctr[k];
-                    const Pair *v = s_val + clk;
-                    const Pair a0 = v[0], a1 = v[1], a2 = v[2], a3 = v[3];
-                    double gv = fma(wx[3], a3.g, fma(wx[2], a2.g, fma(wx[1], a1.g, wx[0] * a0.g)));
-                    double ov = 0.0;
-                    if (NB > 1) ov = fma(wx[3], a3.o, fma(wx[2], a2.o, fma(wx[1], a1.o, wx[0] * a0.o)));
-                    const unsigned f0 = s_colf[clk], f1 = s_colf[clk + 1], f2 = s_colf[clk + 2], f3 = s_colf[clk + 3];
-                    const unsigned fc = (ctk == 0) ? f0 : (ctk == 1) ? f1 : (ctk == 2) ? f2 : (ctk == 3) ? f3 : 0u;
-                    bool g_ok = ok[k] && (fc & 2u), o_ok = g_ok;
-                    if ((f0 | f1 | f2 | f3) & 1u) {
-                        // GDAL GWKResample: drop if sum(w) < 1e-6, divide unless sum(w) is within 1e-5 of 1
-                        const Pair *w = s_wgt + clk;
-                        const Pair m0 = w[0], m1 = w[1], m2 = w[2], m3 = w[3];
-                        const double wg = fma(wx[3], m3.g, fma(wx[2], m2.g, fma(wx[1], m1.g, wx[0] * m0.g)));
-                        if (wg < 0.000001) g_ok = false;
-                        else if (wg < 0.99999 || wg > 1.00001) gv /= wg;
-                        if (NB > 1) {
-                            const double wo = fma(wx[3], m3.o, fma(wx[2], m2.o, fma(wx[1], m1.o, wx[0] * m0.o)));
-                            if (wo < 0.000001) o_ok = false;
-                            else if (wo < 0.99999 || wo > 1.00001) ov /= wo;
-                        }
-                    }
-                    const float gf = g_ok ? (float)gv : qnan;
-                    const float of = o_ok ? (float)ov : qnan;
-                    if (APPLY) {
-                        res[0][k] = __fadd_rn(__fmul_rn(gf, s[k]), of);
-                    } else {
-                        res[0][k] = gf;
-                        if constexpr (NOUT == 2) res[1][k] = of;
-                    }
-                    }
                 }
                 store_row(orow, res);
             }
@@ -1686,15 +1633,11 @@ __global__ void nearest_kernel(const float *__restrict__ src, long nb, long hs, 
     const float qnan = __int_as_float(0x7fc00000);
     for (long idx = (long)blockIdx.x * blockDim.x + threadIdx.x; idx < n; idx += (long)gridDim.x * blockDim.x) {
         const long i = idx / wd, j = idx - i * wd;
-        const double srcy = sy * ((double)i + 0.5) + oy, srcx = sx * ((double)j + 0.5) + ox;
-        long cy = (long)floor(srcy + 1e-10), cx = (long)floor(srcx + 1e-10);
-        if (cy == hs) cy--;
-        if (cx == ws) cx--;
-        const bool ok = srcy >= 0.0 && srcx >= 0.0 && cy >= 0 && cy < hs && cx >= 0 && cx < ws;
+        const UpTap ty = up_tap(sy, oy, i, hs), tx = up_tap(sx, ox, j, ws);
         for (long b = 0; b < nb; b++) {
             float v = qnan;
-            if (ok) {
-                const float s = src[b * hs * ws + cy * ws + cx];
+            if (ty.ok && tx.ok) {
+                const float s = src[b * hs * ws + ty.centre * ws + tx.centre];
                 if (hb_valid(s, nd)) v = s;
             }
             dst[b * n + idx] = v;
