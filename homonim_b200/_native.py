@@ -19,7 +19,7 @@ HB_U8, HB_U16, HB_F32, HB_I16 = 0, 1, 2, 3
 HB_MODEL_GAIN, HB_MODEL_GAIN_BLK_OFFSET, HB_MODEL_GAIN_OFFSET = 0, 1, 2
 HB_UP_CUBIC_SPLINE, HB_UP_NEAREST, HB_UP_BILINEAR, HB_UP_CUBIC, HB_UP_LANCZOS = 0, 1, 2, 3, 4
 HB_STAT_MIN, HB_STAT_MAX, HB_STAT_MED, HB_STAT_Q1, HB_STAT_Q3, HB_STAT_MODE = 0, 1, 2, 3, 4, 5
-ABI_VERSION = 10
+ABI_VERSION = 11
 
 _PKG_DIR = pathlib.Path(__file__).resolve().parent
 LIB_PATH = _PKG_DIR / 'libhomonim_b200.so'

@@ -58,7 +58,8 @@ static int fuse_refspace_direct(const void *src_dev, int src_dtype, long hs, lon
                                 double out_nodata, void *corr_dev, float *params_dev, void *stream)
 {
     HB_REQUIRE(src_dev && ref_dev && corr_dev && hs > 0 && ws > 0 && hr > 0 && wr > 0, "hb_fuse_refspace: bad arguments");
-    HB_REQUIRE(src_dtype == HB_U8 || src_dtype == HB_U16 || src_dtype == HB_F32, "hb_fuse_refspace: bad dtype");
+    HB_REQUIRE(src_dtype == HB_U8 || src_dtype == HB_U16 || src_dtype == HB_I16 || src_dtype == HB_F32,
+               "hb_fuse_refspace: bad dtype");
     cudaStream_t st = (cudaStream_t)stream;
     const bool inpaint = (model == HB_MODEL_GAIN_OFFSET) && do_inpaint;
     const int r2 = (want_r2 || inpaint) ? 1 : 0;
@@ -128,7 +129,8 @@ extern "C" int hb_fuse_refspace_host(const void *src_host, int src_dtype, long h
 {
     HB_REQUIRE(src_host && ref_host && corr_host && hs > 0 && ws > 0 && hr > 0 && wr > 0,
                "hb_fuse_refspace_host: bad arguments");
-    HB_REQUIRE(src_dtype == HB_U8 || src_dtype == HB_U16 || src_dtype == HB_F32, "hb_fuse_refspace_host: bad dtype");
+    HB_REQUIRE(src_dtype == HB_U8 || src_dtype == HB_U16 || src_dtype == HB_I16 || src_dtype == HB_F32,
+               "hb_fuse_refspace_host: bad dtype");
     cudaStream_t st = (cudaStream_t)stream;
     const bool inpaint = (model == HB_MODEL_GAIN_OFFSET) && do_inpaint;
     const int r2 = (want_r2 || inpaint) ? 1 : 0;

@@ -5,15 +5,15 @@
 // result is exact and does not depend on launch or scheduling order.  The rules (footprint window, validity, quantile
 // index, mode tie-break) are specified in oracle/footprint_stats_restate.c.
 //
-// Values are compared through order-preserving 32-bit keys: the value itself for uint8 / uint16, the float_key map of
-// block_norm.cu for float32 (after -0.0 -> +0.0).  Two paths, chosen at launch from the largest footprint the geometry
-// allows:
+// Values are compared through order-preserving 32-bit keys: the value itself for uint8 / uint16, v + 32768 for int16,
+// the float_key map of block_norm.cu for float32 (after -0.0 -> +0.0).  Two paths, chosen at launch from the largest
+// footprint the geometry allows:
 //   * stat_thread_kernel  (<= kStatSmallMax pixels: up-sampling and ratios up to ~5)  one thread per destination pixel;
 //     the thread's valid keys sit in a shared-memory column and a rank / count double loop over them selects the value.
 //   * stat_warp_kernel    (larger footprints)  one warp per destination pixel; the warp stages the footprint's valid keys
 //     in scan order into its shared-memory slice, then: min / max by a warp reduction; med / q1 / q3 by radix select
-//     (8-bit digits, one level for uint8, two for uint16, four for float32, shared-memory histograms); mode by a bitonic
-//     sort of (key, scan index) pairs, whose runs give each value's count and last occurrence.
+//     (8-bit digits, one level for uint8, two for uint16 / int16, four for float32, shared-memory histograms); mode by a
+//     bitonic sort of (key, scan index) pairs, whose runs give each value's count and last occurrence.
 #include "hb_common.cuh"
 
 namespace {
@@ -44,6 +44,17 @@ template <> struct StatKey<uint16_t> {
         return hb_valid_int(k, nd);
     }
     static __device__ __forceinline__ float value(uint32_t k) { return (float)k; }
+};
+template <> struct StatKey<int16_t> {
+    static constexpr int kTopShift = 8;       // keys < 2^16: two digits
+    // v ^ 0x8000 on the 16-bit pattern is v + 32768: order-preserving
+    static __device__ __forceinline__ bool load(const int16_t *p, const NoData &nd, uint32_t &k)
+    {
+        const int16_t v = __ldg(p);
+        k = (uint32_t)(uint16_t)v ^ 0x8000u;
+        return hb_valid_int((uint32_t)(int)v, nd);
+    }
+    static __device__ __forceinline__ float value(uint32_t k) { return __uint_as_float(0x4B000000u | k) - 8421376.0f; }
 };
 template <> struct StatKey<float> {
     static constexpr int kTopShift = 24;      // four digits
@@ -350,11 +361,12 @@ extern "C" int hb_resample_stat(const void *src_dev, int src_dtype, long hs, lon
                "hb_resample_stat: %.4g x %.4g source pixels per destination pixel exceed the maximum of %d on each axis",
                sx, sy, kStatMaxRatio);
     HB_REQUIRE(method >= HB_STAT_MIN && method <= HB_STAT_MODE, "hb_resample_stat: unknown method %d", method);
-    const NoData nd = hb_make_nodata(has_nodata, nodata);
+    const NoData nd = hb_make_nodata(has_nodata, nodata, src_dtype);
     cudaStream_t st = (cudaStream_t)stream;
     switch (src_dtype) {
         case HB_U8: return launch_stat<uint8_t>(src_dev, hs, ws, nd, dst_dev, hd, wd, sx, ox, sy, oy, method, st);
         case HB_U16: return launch_stat<uint16_t>(src_dev, hs, ws, nd, dst_dev, hd, wd, sx, ox, sy, oy, method, st);
+        case HB_I16: return launch_stat<int16_t>(src_dev, hs, ws, nd, dst_dev, hd, wd, sx, ox, sy, oy, method, st);
         case HB_F32: return launch_stat<float>(src_dev, hs, ws, nd, dst_dev, hd, wd, sx, ox, sy, oy, method, st);
     }
     HB_REQUIRE(false, "hb_resample_stat: unknown dtype %d", src_dtype);

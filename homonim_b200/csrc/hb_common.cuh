@@ -2,6 +2,7 @@
 #pragma once
 
 #include <cuda_runtime.h>
+#include <limits.h>
 #include <math.h>
 #include <mutex>
 #include <stdint.h>
@@ -41,7 +42,7 @@ void hb_count_launch(int n = 1);
         }                                                                                                    \
     } while (0)
 
-static inline size_t hb_dtype_size(int dtype) { return dtype == HB_U8 ? 1 : (dtype == HB_U16 ? 2 : 4); }
+static inline size_t hb_dtype_size(int dtype) { return dtype == HB_U8 ? 1 : ((dtype == HB_U16 || dtype == HB_I16) ? 2 : 4); }
 
 // ---- nodata ---------------------------------------------------------------------------------------------------------
 // A pixel is invalid iff it equals the nodata value, or both are NaN (homonim/utils.py:54-56).  The comparison is
@@ -50,18 +51,23 @@ struct NoData {
     int has;       // 0: every pixel valid
     int is_nan;    // nodata is NaN
     float value;   // nodata as float32
-    int int_ok;    // nodata is an integer in [0, 65535]: only then can a uint8 / uint16 pixel equal it
-    int ivalue;    // nodata as integer (when int_ok)
+    int int_ok;    // nodata is an integer in the range of the plane's storage type: only then can an integer pixel equal
+                   // it ([0, 65535] for uint8 / uint16 -- the uint8 kernels also check <= 255 -- [-32768, 32767] for int16)
+    int ivalue;    // nodata as integer when int_ok, otherwise kHbNoIntNodata
 };
+// ivalue when there is no integer nodata: no uint8, uint16 or int16 pixel, zero- or sign-extended, can equal it
+constexpr int kHbNoIntNodata = INT_MIN;
 
-static inline NoData hb_make_nodata(int has, double nodata)
+// `dtype`: storage type of the plane the nodata value belongs to (HB_U8 / HB_U16 / HB_I16 / HB_F32)
+static inline NoData hb_make_nodata(int has, double nodata, int dtype = HB_F32)
 {
+    const double lo = (dtype == HB_I16) ? -32768.0 : 0.0, hi = (dtype == HB_I16) ? 32767.0 : 65535.0;
     NoData nd;
     nd.has = has ? 1 : 0;
     nd.is_nan = (has && isnan(nodata)) ? 1 : 0;
     nd.value = (float)nodata;
-    nd.int_ok = (has && !nd.is_nan && nodata >= 0.0 && nodata <= 65535.0 && nodata == floor(nodata)) ? 1 : 0;
-    nd.ivalue = nd.int_ok ? (int)nodata : -1;
+    nd.int_ok = (has && !nd.is_nan && nodata >= lo && nodata <= hi && nodata == floor(nodata)) ? 1 : 0;
+    nd.ivalue = nd.int_ok ? (int)nodata : kHbNoIntNodata;
     return nd;
 }
 
@@ -70,8 +76,11 @@ __device__ __forceinline__ bool hb_valid(float v, const NoData &nd)
     if (!nd.has) return true;
     return nd.is_nan ? !isnan(v) : (v != nd.value);
 }
-// integer storage: compare as integers (exact; a uint8 / uint16 pixel can only equal an in-range integer nodata)
+// integer storage: compare as integers (exact; `v` is the pixel zero-extended -- uint8 / uint16 -- or sign-extended --
+// int16 -- so a pixel can only equal an in-range integer nodata)
 __device__ __forceinline__ bool hb_valid_int(uint32_t v, const NoData &nd) { return !(nd.int_ok && (int)v == nd.ivalue); }
+// the stored 16-bit pattern of an int16 nodata value (two's complement), for packed comparisons with raw words
+__device__ __forceinline__ uint32_t hb_nd_bits16(const NoData &nd) { return (uint32_t)nd.ivalue & 0xFFFFu; }
 
 // ---- GDAL's down-sampling footprint (GWKAverageOrModeThread) ------------------------------------------------------
 // Destination index i on one axis covers source coordinates [lo, hi) = [s i + o, s (i + 1) + o); its source window is
@@ -99,6 +108,11 @@ template <> __device__ __forceinline__ float hb_to_f32<uint8_t>(uint8_t v)
 template <> __device__ __forceinline__ float hb_to_f32<uint16_t>(uint16_t v)
 {
     return __uint_as_float(0x4B000000u | (uint32_t)v) - 8388608.0f;
+}
+// int16: v ^ 0x8000 is the 16-bit pattern of v + 32768, so the float is 2^23 + 32768 + v
+template <> __device__ __forceinline__ float hb_to_f32<int16_t>(int16_t v)
+{
+    return __uint_as_float(0x4B000000u | ((uint32_t)(uint16_t)v ^ 0x8000u)) - 8421376.0f;
 }
 
 // ---- streaming loads / stores (read-once data: keep it out of L1) -------------------------------------------------

@@ -36,6 +36,16 @@ template <> struct Raw8<uint16_t> {
         v[6] = (uint16_t)(w.w & 0xFFFFu); v[7] = (uint16_t)(w.w >> 16);
     }
 };
+template <> struct Raw8<int16_t> {
+    static __device__ __forceinline__ void load(const int16_t *p, int16_t (&v)[8])
+    {
+        const uint4 w = hb_ldg_stream16(p);
+        v[0] = (int16_t)(w.x & 0xFFFFu); v[1] = (int16_t)(w.x >> 16);
+        v[2] = (int16_t)(w.y & 0xFFFFu); v[3] = (int16_t)(w.y >> 16);
+        v[4] = (int16_t)(w.z & 0xFFFFu); v[5] = (int16_t)(w.z >> 16);
+        v[6] = (int16_t)(w.w & 0xFFFFu); v[7] = (int16_t)(w.w >> 16);
+    }
+};
 template <> struct Raw8<uint8_t> {
     static __device__ __forceinline__ void load(const uint8_t *p, uint8_t (&v)[8])
     {
@@ -62,8 +72,25 @@ template <> struct IsInt<float> { static constexpr bool value = false; };
 
 template <typename T> __device__ __forceinline__ bool ds_valid(T v, const NoData &nd)
 {
-    if (IsInt<T>::value) return hb_valid_int((uint32_t)v, nd);
+    if (IsInt<T>::value) return hb_valid_int((uint32_t)v, nd);         // (int16: sign-extended)
     return hb_valid((float)v, nd);
+}
+
+// The integer paths sum raw 32-bit words of packed pixels.  int16 words hold two's-complement fields: they are summed by
+// the signed form of dp2a, their nodata pattern is the value's 16-bit two's complement, and the 32-bit sums (exact: at
+// most 65025 * 32768 < 2^31 in magnitude) are read back as signed.
+template <typename T> __device__ __forceinline__ uint32_t ds_nd_field(const NoData &nd)
+{
+    return std::is_same<T, int16_t>::value ? hb_nd_bits16(nd) : (uint32_t)nd.ivalue;
+}
+template <typename T> __device__ __forceinline__ uint32_t ds_dp2a_lo(uint32_t w, uint32_t b, uint32_t acc)
+{
+    if constexpr (std::is_same<T, int16_t>::value) return (uint32_t)__dp2a_lo((int)w, (int)b, (int)acc);
+    else return __dp2a_lo(w, b, acc);
+}
+template <typename T> __device__ __forceinline__ double ds_sum(uint32_t s)
+{
+    return std::is_same<T, int16_t>::value ? (double)(int)s : (double)s;
 }
 
 // fetch 8 pixels of row `row` starting at column c (may be partially / wholly outside [0, ws))
@@ -84,8 +111,8 @@ __device__ __forceinline__ void ds_fetch(const T *row, long c, long ws, T (&v)[8
 }
 
 // One CTA: one destination row, `ndc` destination columns.  Phase 1: every thread owns 8 source columns and sums them
-// down the footprint rows (interior rows have weight 1: exact integer sums for uint8/uint16, double for float32; the
-// <= 2 fractionally covered rows are added in double).  Phase 2: one thread per destination pixel combines its
+// down the footprint rows (interior rows have weight 1: exact integer sums for uint8/uint16/int16, double for float32;
+// the <= 2 fractionally covered rows are added in double).  Phase 2: one thread per destination pixel combines its
 // footprint columns from shared memory with the fractional edge weights.
 template <typename T, bool ALIGNED>
 __global__ void __launch_bounds__(kDsThreads, (sizeof(T) == 4) ? HB_DS_MIN_CTAS - 1 : HB_DS_MIN_CTAS)
@@ -140,7 +167,7 @@ downsample_average_kernel(const T *__restrict__ src, long hs, long ws, NoData nd
             constexpr uint32_t kOnes = (sizeof(T) == 2) ? 0x00010001u : 0x01010101u;
             constexpr uint32_t kHigh = (sizeof(T) == 2) ? 0x80008000u : 0x80808080u;
             const bool scan_nd = ndk.int_ok && (sizeof(T) == 2 || ndk.ivalue <= 255);
-            const uint32_t ndpat = scan_nd ? (uint32_t)ndk.ivalue * kOnes : 0u;
+            const uint32_t ndpat = scan_nd ? ds_nd_field<T>(ndk) * kOnes : 0u;
             uint32_t ndc[8];
 #pragma unroll
             for (int k = 0; k < 8; k++) ndc[k] = 0;
@@ -175,8 +202,8 @@ downsample_average_kernel(const T *__restrict__ src, long hs, long ws, NoData nd
 #pragma unroll
                 for (int i = 0; i < NW; i++) {
                     if (sizeof(T) == 2) {
-                        isum[2 * i] = __dp2a_lo(w[i], 0x0001u, isum[2 * i]);
-                        isum[2 * i + 1] = __dp2a_lo(w[i], 0x0100u, isum[2 * i + 1]);
+                        isum[2 * i] = ds_dp2a_lo<T>(w[i], 0x0001u, isum[2 * i]);
+                        isum[2 * i + 1] = ds_dp2a_lo<T>(w[i], 0x0100u, isum[2 * i + 1]);
                     } else {
                         isum[4 * i] = __dp4a(w[i], 0x00000001u, isum[4 * i]);
                         isum[4 * i + 1] = __dp4a(w[i], 0x00000100u, isum[4 * i + 1]);
@@ -192,7 +219,7 @@ downsample_average_kernel(const T *__restrict__ src, long hs, long ws, NoData nd
                         const uint32_t word = (sizeof(T) == 2) ? w[k >> 1] : w[k >> 2];
                         const uint32_t v = (sizeof(T) == 2) ? ((word >> (16 * (k & 1))) & 0xFFFFu)
                                                             : ((word >> (8 * (k & 3))) & 0xFFu);
-                        ndc[k] += (v == (uint32_t)ndk.ivalue) ? 1u : 0u;
+                        ndc[k] += (v == ds_nd_field<T>(ndk)) ? 1u : 0u;
                     }
                 }
             }
@@ -200,7 +227,7 @@ downsample_average_kernel(const T *__restrict__ src, long hs, long ws, NoData nd
             const uint32_t nrows = (uint32_t)(yb > ya ? yb - ya : 0);
 #pragma unroll
             for (int k = 0; k < 8; k++) {
-                colsum[k] = (double)(isum[k] - (scan_nd ? (uint32_t)ndk.ivalue * ndc[k] : 0u));
+                colsum[k] = ds_sum<T>(isum[k] - (scan_nd ? (uint32_t)ndk.ivalue * ndc[k] : 0u));
                 colw[k] = (double)(nrows - ndc[k]);
             }
         } else {
@@ -216,7 +243,7 @@ downsample_average_kernel(const T *__restrict__ src, long hs, long ws, NoData nd
                 }
             }
 #pragma unroll
-            for (int k = 0; k < 8; k++) { colsum[k] = (double)isum[k]; colw[k] = (double)icnt[k]; }
+            for (int k = 0; k < 8; k++) { colsum[k] = ds_sum<T>(isum[k]); colw[k] = (double)icnt[k]; }
         }
     } else {
         uint32_t icnt[8];
@@ -314,8 +341,8 @@ downsample_average_kernel(const T *__restrict__ src, long hs, long ws, NoData nd
 // ---- integer sources on aligned grids with an integer ratio (the benchmark configurations; any "aerial image against a
 //      coarser, snapped reference" case) ------------------------------------------------------------------------------------
 // Every destination pixel is then the exact box of ry x rx source pixels (all GDAL weights are 1), and with rx a multiple
-// of the G = 2 (uint16) / 4 (uint8) pixels of a 32-bit word no word straddles two destination pixels.  The kernel is
-// instruction-issue bound, not DRAM bound, in its general form (ncu: 9.6 lane-instructions per pixel, issue-active ~45 %),
+// of the G = 2 (uint16 / int16) / 4 (uint8) pixels of a 32-bit word no word straddles two destination pixels.  The kernel
+// is instruction-issue bound, not DRAM bound, in its general form (ncu: 9.6 lane-instructions per pixel, issue-active ~45 %),
 // so this variant spends as few instructions per WORD as it can:
 //   * one integer dot-product per word sums its G pixels at once (dp2a / dp4a against all-ones);
 //   * nodata is not counted per pixel: a packed running minimum of (word ^ nodata pattern) -- one min.u16x2 per word --
@@ -348,7 +375,7 @@ downsample_int_aligned_kernel(const T *__restrict__ src, long ws, NoData nd, flo
     const long c_base = (c_first / kDsVec) * kDsVec;                       // 16-byte aligned start of the staged span
     const long c = c_base + (long)t * kDsVec;                              // this thread's 8 columns
     const long c_end = c_first + (long)nj * rx;                            // one past the footprint's last column
-    const uint32_t ndpat = NDSCAN ? (uint32_t)nd.ivalue * kOnes : 0u;
+    const uint32_t ndpat = NDSCAN ? ds_nd_field<T>(nd) * kOnes : 0u;
     if (c + kDsVec > c_first && c < c_end) {                               // (threads wholly outside the footprint idle)
         uint32_t acc[NW], mn[NW];
 #pragma unroll
@@ -358,7 +385,7 @@ downsample_int_aligned_kernel(const T *__restrict__ src, long ws, NoData nd, flo
 #pragma unroll
             for (int k = 0; k < NW; k++) {
                 // (dp2a.lo multiplies the two 16-bit halves of the word by the two LOW BYTES of its second operand)
-                if (sizeof(T) == 2) acc[k] = __dp2a_lo(w[k], 0x0101u, acc[k]);
+                if (sizeof(T) == 2) acc[k] = ds_dp2a_lo<T>(w[k], 0x0101u, acc[k]);
                 else acc[k] = __dp4a(w[k], 0x01010101u, acc[k]);
                 if (NDSCAN) {
                     const uint32_t x = w[k] ^ ndpat;
@@ -401,7 +428,7 @@ downsample_int_aligned_kernel(const T *__restrict__ src, long ws, NoData nd, flo
 #pragma unroll
                         for (int f = 0; f < G; f++) {
                             const uint32_t v = (w1[k] >> (f * 8 * (int)sizeof(T))) & ((sizeof(T) == 2) ? 0xFFFFu : 0xFFu);
-                            ndcnt[k] += (v == (uint32_t)nd.ivalue) ? 1u : 0u;
+                            ndcnt[k] += (v == ds_nd_field<T>(nd)) ? 1u : 0u;
                         }
                     }
                 }
@@ -430,7 +457,7 @@ downsample_int_aligned_kernel(const T *__restrict__ src, long ws, NoData nd, flo
     const float qnan = __int_as_float(0x7fc00000);
     for (int k = t; k < nj; k += kDsThreads) {
         const uint32_t n = s_cnt[k];
-        dst[i * wd + j0 + k] = n ? (float)((double)s_sum[k] / (double)n) : qnan;
+        dst[i * wd + j0 + k] = n ? (float)(ds_sum<T>(s_sum[k]) / (double)n) : qnan;
     }
 }
 
@@ -589,11 +616,12 @@ extern "C" int hb_downsample_average(const void *src_dev, int src_dtype, long hs
 {
     HB_REQUIRE(src_dev && dst_dev && hs > 0 && ws > 0 && hd > 0 && wd > 0, "hb_downsample_average: bad arguments");
     HB_REQUIRE(sx > 0 && sy > 0, "hb_downsample_average: grids must have the same orientation");
-    const NoData nd = hb_make_nodata(has_nodata, nodata);
+    const NoData nd = hb_make_nodata(has_nodata, nodata, src_dtype);
     cudaStream_t st = (cudaStream_t)stream;
     switch (src_dtype) {
         case HB_U8: return launch_downsample<uint8_t>(src_dev, hs, ws, nd, dst_dev, hd, wd, sx, ox, sy, oy, st);
         case HB_U16: return launch_downsample<uint16_t>(src_dev, hs, ws, nd, dst_dev, hd, wd, sx, ox, sy, oy, st);
+        case HB_I16: return launch_downsample<int16_t>(src_dev, hs, ws, nd, dst_dev, hd, wd, sx, ox, sy, oy, st);
         case HB_F32: return launch_downsample<float>(src_dev, hs, ws, nd, dst_dev, hd, wd, sx, ox, sy, oy, st);
     }
     HB_REQUIRE(false, "hb_downsample_average: unknown dtype %d", src_dtype);
@@ -606,7 +634,7 @@ extern "C" int hb_apply_same_grid(const void *src_dev, int src_dtype, int has_no
     HB_REQUIRE(src_dev && params_dev && corr_dev && h > 0 && w > 0, "hb_apply_same_grid: bad arguments");
     HB_REQUIRE(hb_outspec_error(out_dtype, out_has_nodata, out_nodata) == nullptr, "hb_apply_same_grid: %s",
                hb_outspec_error(out_dtype, out_has_nodata, out_nodata));
-    const NoData nd = hb_make_nodata(has_nodata, nodata);
+    const NoData nd = hb_make_nodata(has_nodata, nodata, src_dtype);
     const OutSpec os = hb_make_outspec(out_dtype, out_has_nodata, out_nodata);
     cudaStream_t st = (cudaStream_t)stream;
     const long n = h * w;
@@ -619,6 +647,10 @@ extern "C" int hb_apply_same_grid(const void *src_dev, int src_dtype, int has_no
         case HB_U16:
             apply_same_grid_kernel<uint16_t><<<grid, 256, 0, st>>>((const uint16_t *)src_dev, nd, mask_src, params_dev,
                                                                    n, corr_dev, os);
+            break;
+        case HB_I16:
+            apply_same_grid_kernel<int16_t><<<grid, 256, 0, st>>>((const int16_t *)src_dev, nd, mask_src, params_dev,
+                                                                  n, corr_dev, os);
             break;
         case HB_F32:
             apply_same_grid_kernel<float><<<grid, 256, 0, st>>>((const float *)src_dev, nd, mask_src, params_dev, n,
@@ -667,13 +699,16 @@ extern "C" int hb_valid_mask(const void *src_dev, int src_dtype, long n, int has
                              uint8_t *mask_dev, void *stream)
 {
     HB_REQUIRE(src_dev && mask_dev && n > 0, "hb_valid_mask: bad arguments");
-    const NoData nd = hb_make_nodata(has_nodata, nodata);
+    const NoData nd = hb_make_nodata(has_nodata, nodata, src_dtype);
     cudaStream_t st = (cudaStream_t)stream;
     const unsigned grid = hb_grid_for(n, 256, 16);
     switch (src_dtype) {
         case HB_U8: valid_mask_kernel<uint8_t><<<grid, 256, 0, st>>>((const uint8_t *)src_dev, n, nd, mask_dev); break;
         case HB_U16:
             valid_mask_kernel<uint16_t><<<grid, 256, 0, st>>>((const uint16_t *)src_dev, n, nd, mask_dev);
+            break;
+        case HB_I16:
+            valid_mask_kernel<int16_t><<<grid, 256, 0, st>>>((const int16_t *)src_dev, n, nd, mask_dev);
             break;
         case HB_F32: valid_mask_kernel<float><<<grid, 256, 0, st>>>((const float *)src_dev, n, nd, mask_dev); break;
         default: HB_REQUIRE(false, "hb_valid_mask: unknown dtype %d", src_dtype);

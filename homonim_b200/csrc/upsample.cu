@@ -301,6 +301,33 @@ template <> struct SrcQuad<uint16_t> {
         ok[3] = __float_as_uint(m1.y) != magic;
     }
 };
+template <> struct SrcQuad<int16_t> {
+    static constexpr int kBytes = 8;
+    typedef uint32_t Key;
+    static __device__ __forceinline__ Key key(const NoData &nd)
+    {
+        return nd.int_ok ? (0x4B000000u | (hb_nd_bits16(nd) ^ 0x8000u)) : 0xFFFFFFFFu;
+    }
+    static __device__ __forceinline__ void get_shared(uint32_t sa, const Key magic, float2 (&s)[2], bool (&ok)[4])
+    {
+        uint2 w;
+        asm volatile("ld.shared.v2.u32 {%0,%1}, [%2];" : "=r"(w.x), "=r"(w.y) : "r"(sa));
+        // flipping the sign bits turns each field into v + 32768 (one LOP per two pixels); then as uint16, with
+        // 2^23 + 32768 subtracted (exact)
+        w.x ^= 0x80008000u;
+        w.y ^= 0x80008000u;
+        const float2 m0 = make_float2(__uint_as_float(__byte_perm(w.x, 0x4B000000u, 0x7410)),
+                                      __uint_as_float(__byte_perm(w.x, 0x4B000000u, 0x7432)));
+        const float2 m1 = make_float2(__uint_as_float(__byte_perm(w.y, 0x4B000000u, 0x7410)),
+                                      __uint_as_float(__byte_perm(w.y, 0x4B000000u, 0x7432)));
+        s[0] = fadd2(m0, splat(-8421376.0f));
+        s[1] = fadd2(m1, splat(-8421376.0f));
+        ok[0] = __float_as_uint(m0.x) != magic;
+        ok[1] = __float_as_uint(m0.y) != magic;
+        ok[2] = __float_as_uint(m1.x) != magic;
+        ok[3] = __float_as_uint(m1.y) != magic;
+    }
+};
 template <> struct SrcQuad<uint8_t> {
     static constexpr int kBytes = 4;
     typedef uint32_t Key;
@@ -1249,7 +1276,22 @@ template <> struct Src4<uint16_t> {
 #pragma unroll
         for (int k = 0; k < 4; k++) {
             v[k] = __uint_as_float(0x4B000000u | r[k]) - 8388608.0f;      // exact, no I2F
-            ok[k] = (int)r[k] != nd.ivalue;                                // ivalue = -1 when no integer nodata
+            ok[k] = (int)r[k] != nd.ivalue;                                // (kHbNoIntNodata when no integer nodata)
+        }
+    }
+};
+template <> struct Src4<int16_t> {
+    static constexpr int kBytes = 8;
+    static __device__ __forceinline__ void get(const void *p, const NoData &nd, float (&v)[4], bool (&ok)[4])
+    {
+        uint2 w = *reinterpret_cast<const uint2 *>(p);
+        w.x ^= 0x80008000u;                                                 // fields: v + 32768
+        w.y ^= 0x80008000u;
+        const uint32_t r[4] = {w.x & 0xFFFFu, w.x >> 16, w.y & 0xFFFFu, w.y >> 16};
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+            v[k] = __uint_as_float(0x4B000000u | r[k]) - 8421376.0f;      // exact, no I2F
+            ok[k] = (int)r[k] - 32768 != nd.ivalue;
         }
     }
 };
@@ -1815,30 +1857,28 @@ int launch_upsample(const void *src, NoData nd, const float *coarse, long hs, lo
     const size_t align = APPLY ? sizeof(T) * kPpt : 16;
     const bool aligned = (!APPLY || (((ws * (long)sizeof(T)) % (long)align == 0) && (((uintptr_t)src) % align == 0))) &&
                          (ws % 4 == 0) && (((uintptr_t)out) % (4 * hb_out_size(ospec.dtype)) == 0);
-    NoData ndk = nd;
-    if (!ndk.int_ok) ndk.ivalue = -1;                       // integer sources: no pixel can equal it
     // ---- cubic-spline fast paths: aligned rasters, no coverage mask, >= ~1.6 destination pixels per coarse pixel (a
     //      lane's 4 pixels must span at most 3 coarse cells: 3 * sx < 2, with margin; the row direction only needs
     //      sy <= 1).  The other methods always take the general kernel.
     if (method == HB_UP_CUBIC_SPLINE && aligned && cover == nullptr && sx <= 0.62 && sy <= 1.0 + 1e-9 &&
         ws % kPpt == 0) {
         const UpPolyGeom pg = {hs, ws, hp, wp, sx, ox, sy, oy, ospec};
-        if constexpr (APPLY) return launch_poly<T>((const T *)src, ndk, coarse, pg, out, stream);
+        if constexpr (APPLY) return launch_poly<T>((const T *)src, nd, coarse, pg, out, stream);
         // plain up-sampling: one band in double precision (it feeds a fit); two bands stay on the general kernel
         if constexpr (NB == 1) return launch_yfirst_f64(coarse, pg, out, stream);
     }
     switch (method) {
         case HB_UP_CUBIC_SPLINE:
-            return launch_general<T, NB, APPLY, HB_UP_CUBIC_SPLINE>(src, ndk, coarse, g, aligned, grid, smem, cover, out,
+            return launch_general<T, NB, APPLY, HB_UP_CUBIC_SPLINE>(src, nd, coarse, g, aligned, grid, smem, cover, out,
                                                                     stream);
         case HB_UP_BILINEAR:
-            return launch_general<T, NB, APPLY, HB_UP_BILINEAR>(src, ndk, coarse, g, aligned, grid, smem, cover, out,
+            return launch_general<T, NB, APPLY, HB_UP_BILINEAR>(src, nd, coarse, g, aligned, grid, smem, cover, out,
                                                                 stream);
         case HB_UP_CUBIC:
-            return launch_general<T, NB, APPLY, HB_UP_CUBIC>(src, ndk, coarse, g, aligned, grid, smem, cover, out,
+            return launch_general<T, NB, APPLY, HB_UP_CUBIC>(src, nd, coarse, g, aligned, grid, smem, cover, out,
                                                              stream);
         case HB_UP_LANCZOS:
-            return launch_general<T, NB, APPLY, HB_UP_LANCZOS>(src, ndk, coarse, g, aligned, grid, smem, cover, out,
+            return launch_general<T, NB, APPLY, HB_UP_LANCZOS>(src, nd, coarse, g, aligned, grid, smem, cover, out,
                                                                stream);
     }
     HB_REQUIRE(false, "up-sampling: unknown method %d", method);
@@ -1862,7 +1902,7 @@ extern "C" int hb_upsample_apply(const void *src_dev, int src_dtype, long hs, lo
                method == HB_UP_LANCZOS, "hb_upsample_apply: unknown method %d", method);
     HB_REQUIRE(hb_outspec_error(out_dtype, out_has_nodata, out_nodata) == nullptr, "hb_upsample_apply: %s",
                hb_outspec_error(out_dtype, out_has_nodata, out_nodata));
-    const NoData nd = hb_make_nodata(has_nodata, nodata);
+    const NoData nd = hb_make_nodata(has_nodata, nodata, src_dtype);
     const OutSpec os = hb_make_outspec(out_dtype, out_has_nodata, out_nodata);
     cudaStream_t st = (cudaStream_t)stream;
     float *out = (float *)corr_dev;                          // (typed by `os`; the kernels index it in pixels)
@@ -1873,6 +1913,9 @@ extern "C" int hb_upsample_apply(const void *src_dev, int src_dtype, long hs, lo
         case HB_U16:
             return launch_upsample<uint16_t, 2, true>(src_dev, nd, params_dev, hs, ws, hp, wp, sx, ox, sy, oy,
                                                       cover_dev, out, st, os, method);
+        case HB_I16:
+            return launch_upsample<int16_t, 2, true>(src_dev, nd, params_dev, hs, ws, hp, wp, sx, ox, sy, oy,
+                                                     cover_dev, out, st, os, method);
         case HB_F32:
             return launch_upsample<float, 2, true>(src_dev, nd, params_dev, hs, ws, hp, wp, sx, ox, sy, oy, cover_dev,
                                                    out, st, os, method);

@@ -25,7 +25,7 @@ except ImportError:  # pragma: no cover
 
 logger = logging.getLogger(__name__)
 
-_NATIVE_DTYPES = ('uint8', 'uint16', 'float32')      # storage dtypes the kernels read directly
+_NATIVE_DTYPES = ('uint8', 'uint16', 'int16', 'float32')      # storage dtypes the kernels read directly
 
 
 def is_path(obj) -> bool:
@@ -83,8 +83,8 @@ class FilePair:
 
     @staticmethod
     def _read(im: GeoTiffReader, bands: Sequence[int], window, pinned: bool) -> RasterArray:
-        """ The chosen bands as a [bands, H, W] RasterArray: uint8 / uint16 / float32 stay as stored (the kernels read
-        them directly), other sample types are widened to float32 as the reference's reader does for every type
+        """ The chosen bands as a [bands, H, W] RasterArray: uint8 / uint16 / int16 / float32 stay as stored (the kernels
+        read them directly), other sample types are widened to float32 as the reference's reader does for every type
         (raster_array.py:178-188).  A file without a nodata value gets the default NaN nodata, as in the reference. """
         array = im.read(list(bands), window=window, pinned=pinned and im.dtype.name in _NATIVE_DTYPES)
         nodata = im.nodata

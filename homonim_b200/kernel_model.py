@@ -10,7 +10,7 @@ CPU implementation here and none is fallen back to.
 Differences from the reference, all deliberate:
   * ``fit`` does not mutate its inputs (the reference zeroes invalid pixels in place, kernel_model.py:246-247).
   * rasters may be host numpy arrays (copied to the device and back) or torch CUDA tensors (stay on the device);
-    uint8 / uint16 sources may be passed in their stored dtype.
+    uint8 / uint16 / int16 sources may be passed in their stored dtype.
   * ``RefSpaceModel.apply`` never materialises the up-sampled parameters: up-sampling and gain*src+offset are one
     kernel.
   * down-sampling is ``average``; up-sampling is ``cubic_spline`` (the default), ``bilinear``, ``cubic``,
@@ -40,7 +40,7 @@ except ImportError:  # pragma: no cover
     torch = None
 
 NAN = float('nan')
-_DTYPE_CODES = {'uint8': _native.HB_U8, 'uint16': _native.HB_U16, 'float32': _native.HB_F32}
+_DTYPE_CODES = {'uint8': _native.HB_U8, 'uint16': _native.HB_U16, 'int16': _native.HB_I16, 'float32': _native.HB_F32}
 _OUT_DTYPE_CODES = {'uint8': _native.HB_U8, 'uint16': _native.HB_U16, 'int16': _native.HB_I16, 'float32': _native.HB_F32}
 _MODEL_CODES = {
     Model.gain: _native.HB_MODEL_GAIN,
@@ -201,7 +201,7 @@ def _to_device(array, device=None):
 def _plane_code(t) -> int:
     name = str(t.dtype).replace('torch.', '')
     if name not in _DTYPE_CODES:
-        raise TypeError(f'unsupported raster dtype {name!r}: expected uint8, uint16 or float32')
+        raise TypeError(f'unsupported raster dtype {name!r}: expected uint8, uint16, int16 or float32')
     return _DTYPE_CODES[name]
 
 
@@ -439,7 +439,7 @@ class KernelModel:
 # resampling between grids (reference RasterArray.reproject, raster_array.py:526-578)
 # ---------------------------------------------------------------------------------------------------------------------
 def _downsample_average(src_t, src_transform, src_nodata, dst_shape, dst_transform):
-    """ float32 [hd, wd] (NaN nodata) average of a uint8 / uint16 / float32 plane. """
+    """ float32 [hd, wd] (NaN nodata) average of a uint8 / uint16 / int16 / float32 plane. """
     lib = _native.lib()
     gm = grid_map(src_transform, dst_transform)
     hs, ws = int(src_t.shape[-2]), int(src_t.shape[-1])
@@ -464,7 +464,7 @@ _STAT_METHODS = {
 
 def _resample_stat(src_t, src_transform, src_nodata, dst_shape, dst_transform, method):
     """ float32 [hd, wd] (NaN nodata) footprint statistic ``method`` (an ``HB_STAT_*`` code) of a uint8 / uint16 /
-    float32 plane. """
+    int16 / float32 plane. """
     gm = grid_map(src_transform, dst_transform)
     hs, ws = int(src_t.shape[-2]), int(src_t.shape[-1])
     hd, wd = int(dst_shape[0]), int(dst_shape[1])

@@ -8,7 +8,7 @@ constructor, ``from_profile``, ``array`` / ``mask`` / ``nodata`` / ``profile`` /
 
   * ``array`` may be a numpy array (host) OR a torch CUDA tensor (device-resident raster).  Results of
     ``KernelModel.fit/apply`` live where their inputs live.
-  * integer rasters (uint8 / uint16) may be kept in their stored dtype: the CUDA kernels convert on load, which is
+  * integer rasters (uint8 / uint16 / int16) may be kept in their stored dtype: the CUDA kernels convert on load, which is
     what the reference's reader does on the host with ``out_dtype='float32'`` (raster_array.py:178-188).
   * no rasterio dependency: ``crs`` is an opaque comparable label, ``transform`` any 6-coefficient affine.
   * file I/O methods (``from_rio_dataset`` / ``to_rio_dataset`` / ``to_file``) are out of scope (SURVEY.md 8, 2).

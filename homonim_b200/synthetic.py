@@ -26,7 +26,7 @@ from homonim_b200.geometry import Affine, CRS
 from homonim_b200.raster_array import RasterArray
 
 _DTYPES = {'uint8': (torch.uint8, 1.0, 255.0), 'uint16': (torch.uint16, 1.0, 65535.0),
-           'float32': (torch.float32, -3.0e38, 3.0e38)}
+           'int16': (torch.int16, -32768.0, 32767.0), 'float32': (torch.float32, -3.0e38, 3.0e38)}
 
 
 def _gauss_kernel(sigma: float, device) -> torch.Tensor:
@@ -53,7 +53,9 @@ def make_pair(hp: int, wp: int, ratio: int, bands: int = 1, dtype: str = 'uint16
 
     hp, wp:      proc (reference) grid size covered by the source.
     ratio:       integer source pixels per reference pixel (aligned grids).
-    dtype:       source storage dtype: 'uint8', 'uint16' or 'float32'.
+    dtype:       source storage dtype: 'uint8', 'uint16', 'int16' or 'float32'.  int16 sources are shifted down by
+                 mu / 2 per band (before the reference is derived), so that a few percent of their values are negative,
+                 as in surface-reflectance products stored as int16.
     src_nodata:  source nodata value (use float('nan') for float32 sources).
     Returns (src_ra [bands, hs, ws], ref_ra [bands, hp + 2*ref_pad, wp + 2*ref_pad] float32, fully valid, nodata nan).
     """
@@ -75,6 +77,8 @@ def make_pair(hp: int, wp: int, ratio: int, bands: int = 1, dtype: str = 'uint16
             hi_res = hi_res + 0.02 * mu_b * torch.randn((hs, ws), generator=gen, device=device)
         else:
             hi_res = lo_res + 0.02 * mu_b * torch.randn((hs, ws), generator=gen, device=device)
+        if dtype == 'int16':
+            hi_res = hi_res - 0.5 * mu_b
         hi_res = hi_res.clamp(lo, hi)
         if dtype != 'float32':
             hi_res = hi_res.round()

@@ -35,11 +35,13 @@
 extern "C" {
 #endif
 
-#define HB_ABI_VERSION 10
+#define HB_ABI_VERSION 11
 
-/* storage dtype of a source raster plane */
-enum { HB_U8 = 0, HB_U16 = 1, HB_F32 = 2, HB_I16 = 3 };   /* HB_I16: output dtypes only (out_dtype, hb_convert_dtype,
-                                                             hb_build_overviews) */
+/* storage dtype of a raster plane.  Every dtype is a source dtype of the entry points that read a stored source plane
+ * (hb_downsample_average, hb_resample_stat, hb_apply_same_grid, hb_upsample_apply, hb_valid_mask, hb_fuse_refspace,
+ * hb_fuse_refspace_host) and an output dtype.  A stored pixel v reads as the float32 value (float)v; an integer pixel
+ * equals the nodata value only when that is an integer in the dtype's range. */
+enum { HB_U8 = 0, HB_U16 = 1, HB_F32 = 2, HB_I16 = 3 };
 /* homonim.enums.Model (homonim/enums.py:22-42) */
 enum { HB_MODEL_GAIN = 0, HB_MODEL_GAIN_BLK_OFFSET = 1, HB_MODEL_GAIN_OFFSET = 2 };
 /* up-sampling methods of hb_resample_up and hb_upsample_apply (GDAL GRA_CubicSpline, GRA_NearestNeighbour,
